@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MuDPT ViT-B/16 train step throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" = one MuDPT train step of BASELINE config 2: forward + mean cross-entropy + dgrad-only
@@ -332,10 +332,13 @@ def run_ours(args):
         trainer = build_trainer(device, truncate)
         model = trainer.model
         eng = model._clip_ref[0].engine(device)
+        last = {}
 
         def step_resident(i):
             trainer.optim.zero_grad()
-            model.forward_backward(imgs_dev[i % NBUF], labs_dev[i % NBUF])
+            out = model.forward_backward(imgs_dev[i % NBUF], labs_dev[i % NBUF])
+            if args.dump_outputs:
+                last["loss"], last["logits"] = out
             trainer.optim.step()
 
         def step_e2e(i):
@@ -353,6 +356,8 @@ def run_ours(args):
         ms, t0, t1 = timed_loop(step_resident, K, W, device, world)
         if variant == "full":
             clocks = sampler.stop(t0, t1)
+            if args.dump_outputs and rank == 0:  # before any further step overwrites them
+                dump_outputs(args.dump_outputs, model, last["loss"], last["logits"])
         launches = (eng.launch_count() - l0) // (K + W)
         ms_e2e, _, _ = timed_loop(step_e2e, K, W, device, world)
         # instrumented pass of the same step: per-kernel-class CUDA-event times
@@ -479,6 +484,21 @@ def run_ours(args):
         dist.barrier()
         dist.destroy_process_group()
 
+
+
+def dump_outputs(out_dir, model, loss, logits):
+    """--dump-outputs: what the last timed step of the headline hands its caller, one float32 .npy per array: the loss,
+    rank 0's logits, and for each of the 10 trainable prompt tensors its gradient (grad.<name>) and its value after the
+    SGD update (param.<name>).  About 10 MB at ViT-B/16 and 19 MB at ViT-L/14.  The inputs are seeded, so two builds
+    run with the same arguments can be compared array by array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "logits": logits}
+    for n, p in model.named_parameters():
+        if p.requires_grad:
+            arrays["grad." + n], arrays["param." + n] = p.grad, p
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def reference_step_flops(batch, classes, text_len):
@@ -727,7 +747,10 @@ def run_config4(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps: exactly K for the train steps of --config 2, 4 and 5; --config 3 times at least 5 "
+                         "batches, and --impl reference at most 2 full-size (or 40 sampled) CPU steps so that it ends within "
+                         "minutes; the JSON line reports the count used")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="profiling aid: resident loop of the full-length variant only")
@@ -736,7 +759,12 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5],
                     help="BASELINE.json configs (1-based): 2 = the headline (default), 3 = inference with cached text features, "
                          "4 = CoCoOp-shaped step, 5 = ViT-L/14 prompt depth 12")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, logits, prompt gradients and updated prompt parameters of the last timed train "
+                         "step (full-length text tower) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.quick or args.config in (3, 4)):
+        ap.error("--dump-outputs applies to the native train step of --config 2 or 5")
     if args.config == 5:
         global ARCH, DEPTH
         ARCH, DEPTH = "ViT-L/14", 12

@@ -5,7 +5,7 @@ Only tests/, __graft_entry__.smoke() and bench.py's CPU leg may import this file
 (mudpt_b200/) never does.  Pinned against the reference itself: tests/golden/cocoop_*.npz are
 produced by oracle/make_golden.py from the unmodified trainers/cocoop.py, and
 tests/test_oracle.py checks this restatement against them (and against the live reference when
-/root/reference exists).
+MUDPT_REFERENCE_ROOT names a checkout of it).
 
   PromptLearner.forward ... trainers/cocoop.py:149-163     (ctx + meta_net(im_features), per image)
   TextEncoder.forward ..... trainers/cocoop.py:52-64       (plain blocks, clip/model.py:178-199)

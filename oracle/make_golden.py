@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/*.npz from the REFERENCE itself.
 
-Runs in the build container only (needs /root/reference, imported read-only under
+Needs the reference (MUDPT_REFERENCE_ROOT, imported read-only under
 oracle/ref_shims.py).  For each case it
 
   1. builds the reference `CLIP(...)` + `trainers.mudpt.CustomCLIP` (unmodified reference
@@ -28,6 +28,7 @@ sys.path.insert(0, ROOT)
 
 from oracle import ref_shims  # noqa: E402
 from mudpt_b200 import synthetic as syn  # noqa: E402
+from tests import golden_util as gu  # noqa: E402
 
 CASES = {
     # name: arch, n_ctx, depth, ctx_init, classnames, batch, image kind
@@ -111,7 +112,7 @@ def run_case(name: str, spec: dict, out_dir: str) -> None:
             out["grad/" + n] = (p.grad if p.grad is not None else torch.zeros_like(p)).numpy()
     assert len(trainable) == 10, trainable
     path = os.path.join(out_dir, name + ".npz")
-    np.savez_compressed(path, **out)
+    gu.save(path, out)
     print(f"{name}: loss={float(loss.detach()):.6f} logits{tuple(logits.shape)} -> {path} "
           f"({os.path.getsize(path)/1e6:.2f} MB, {time.time()-t0:.1f}s)")
 
@@ -176,7 +177,7 @@ def run_cocoop_case(name: str, spec: dict, out_dir: str) -> None:
         if p.requires_grad:
             out["grad/" + n] = p.grad.numpy()
     path = os.path.join(out_dir, name + ".npz")
-    np.savez_compressed(path, **out)
+    gu.save(path, out)
     print(f"{name}: loss={float(loss.detach()):.6f} logits{tuple(logits.shape)} -> {path} "
           f"({os.path.getsize(path)/1e6:.2f} MB, {time.time()-t0:.1f}s)")
 
@@ -230,7 +231,7 @@ def run_variant_case(name: str, spec: dict, out_dir: str) -> None:
         if p.requires_grad:
             out["grad/" + n] = p.grad.numpy()
     path = os.path.join(out_dir, name + ".npz")
-    np.savez_compressed(path, **out)
+    gu.save(path, out)
     print(f"{name}: loss={float(loss.detach()):.6f} logits{tuple(logits.shape)} trainable={sum(1 for k in out if k.startswith('grad/'))} "
           f"-> {path} ({os.path.getsize(path)/1e6:.2f} MB, {time.time()-t0:.1f}s)")
 

@@ -16,7 +16,7 @@ math of the reference:
 The arithmetic of the reference lives in third-party PyTorch (unpinned by the reference;
 torch 2.11.0 CPU here).  Parity pinning: `tests/test_oracle.py` runs the
 *reference itself* (imported read-only under oracle/ref_shims.py) against this file when
-/root/reference is present, and `tests/golden/*.npz` (made by oracle/make_golden.py from the
+MUDPT_REFERENCE_ROOT names a checkout of it, and `tests/golden/*.npz` (made by oracle/make_golden.py from the
 reference) pins it everywhere else.  The reference has no tests / golden vectors of its own
 (SURVEY.md section 4).
 

@@ -1,17 +1,17 @@
 """TEST INFRASTRUCTURE ONLY -- import the read-only reference under import shims.
 
-The reference (/root/reference) needs `yacs`, `dassl` and `ftfy`, none of which exist in
-this image (SURVEY.md section 8c).  This module registers minimal stand-ins *before*
+The reference (a checkout of the original MuDPT Python project, not part of this repository,
+located by the environment variable MUDPT_REFERENCE_ROOT) needs `yacs`, `dassl` and `ftfy`
+(SURVEY.md section 8c).  This module registers minimal stand-ins *before*
 importing the reference packages so that the reference's own `clip/model.py` and
 `trainers/mudpt.py` run unmodified on CPU fp32.  It is used only
 
-  * by `oracle/make_golden.py` (in the build container, where /root/reference exists) to
-    generate the golden fixtures committed under tests/golden/, and
+  * by `oracle/make_golden.py` to generate the golden fixtures committed under tests/golden/, and
   * by tests marked `needs_reference` that pin the restatement in `oracle/mudpt_oracle.py`
     against the reference itself.
 
-Nothing under mudpt_b200/ imports this file.  /root/reference does not exist on the GPU
-box; `reference_available()` is the gate.
+Nothing under mudpt_b200/ imports this file.  `reference_available()` is the gate: without
+MUDPT_REFERENCE_ROOT the golden fixtures stand in for the reference.
 """
 from __future__ import annotations
 
@@ -19,11 +19,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("MUDPT_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("MUDPT_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "trainers", "mudpt.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "trainers", "mudpt.py"))
 
 
 class CfgNode(dict):
@@ -100,7 +100,7 @@ def _install_shims() -> None:
 def import_reference():
     """Returns (clip_pkg, clip.model module, trainers.mudpt module) of the reference."""
     if not reference_available():
-        raise RuntimeError(f"reference not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference not found: set MUDPT_REFERENCE_ROOT to a MuDPT checkout (now {REFERENCE_ROOT!r})")
     _install_shims()
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)

@@ -9,15 +9,42 @@ from mudpt_b200 import synthetic as syn
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 TINY = ["tiny_a", "tiny_b", "tiny_c", "tiny_d"]
+LOWRANK = "lowrank/"  # lowrank/<key>/a and lowrank/<key>/b stand for the array <key> = a @ b
 
 _cache = {}
+
+
+def save(path, arrays):
+    """np.savez_compressed, except that a large 2-D gradient of low numerical rank r (the weight gradient of a
+    projection applied to a few prompt rows) is stored as two rank-r factors when they take less than half its
+    space, which keeps the ViT-B/16 fixture small.  Their product equals the gradient to fp32 rounding."""
+    out = {}
+    for k, v in arrays.items():
+        if k.startswith("grad/") and v.ndim == 2 and v.dtype == np.float32 and v.size >= 4096:
+            u, s, vt = np.linalg.svd(v.astype(np.float64), full_matrices=False)
+            r = int((s > 1e-6 * s[0]).sum())
+            if 2 * r * sum(v.shape) < v.size:
+                a, b = (u[:, :r] * s[:r]).astype(np.float32), vt[:r].astype(np.float32)
+                if np.abs(a.astype(np.float64) @ b - v).max() <= 1e-6 * np.abs(v).max():
+                    out[LOWRANK + k + "/a"], out[LOWRANK + k + "/b"] = a, b
+                    continue
+        out[k] = v
+    np.savez_compressed(path, **out)
+
+
+def _read(name):
+    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False)
+    g = {k: z[k] for k in z.files if not k.startswith(LOWRANK)}
+    for k in z.files:
+        if k.startswith(LOWRANK) and k.endswith("/a"):
+            g[k[len(LOWRANK):-2]] = (z[k].astype(np.float64) @ z[k[:-1] + "b"]).astype(np.float32)
+    return g
 
 
 def load(name):
     if name in _cache:
         return _cache[name]
-    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False)
-    g = {k: z[k] for k in z.files}
+    g = _read(name)
     arch = syn.ARCHS[str(g["arch"])]
     n_ctx, depth, batch = int(g["n_ctx"]), int(g["depth"]), int(g["batch"])
     tok = torch.from_numpy(g["tokenized_prompts"])
@@ -62,8 +89,7 @@ def load_cocoop(name):
     """CoCoOp fixture (BASELINE config 4) made from the reference's trainers/cocoop.py."""
     if name in _cache:
         return _cache[name]
-    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False)
-    g = {k: z[k] for k in z.files}
+    g = _read(name)
     arch = syn.ARCHS[str(g["arch"])]
     n_ctx, batch = int(g["n_ctx"]), int(g["batch"])
     tok = torch.from_numpy(g["tokenized_prompts"])
@@ -110,8 +136,7 @@ def load_variant(name):
     """UMuDPT / UUMuDPT fixture (SURVEY 8f N4) made from the reference's trainers/{umudpt,uumudpt}.py."""
     if name in _cache:
         return _cache[name]
-    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"), allow_pickle=False)
-    g = {k: z[k] for k in z.files}
+    g = _read(name)
     arch = syn.ARCHS[str(g["arch"])]
     case = dict(trainer=str(g["trainer"]), arch=arch, n_ctx=int(g["n_ctx"]), depth=int(g["depth"]), batch=int(g["batch"]),
                 tokenized=torch.from_numpy(g["tokenized_prompts"]), labels=torch.from_numpy(g["labels"]),

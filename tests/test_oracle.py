@@ -25,6 +25,25 @@ def test_oracle_matches_reference_golden(name):
             assert m["cos"] > 0.99999 and m["rel_l2"] < 2e-3, (k, m)
 
 
+def test_golden_low_rank_storage_round_trip(tmp_path, monkeypatch):
+    """golden_util.save keeps a low-rank weight gradient as two factors and loading multiplies them back; a full-rank
+    gradient and every other array are stored as they are."""
+    rng = np.random.default_rng(0)
+    arrays = {"grad/low": (rng.standard_normal((300, 3)) @ rng.standard_normal((3, 200))).astype(np.float32),
+              "grad/full": rng.standard_normal((100, 100)).astype(np.float32),
+              "logits": rng.standard_normal((4, 7)).astype(np.float32), "arch": np.array("tiny")}
+    monkeypatch.setattr(gu, "GOLDEN_DIR", str(tmp_path))
+    gu.save(str(tmp_path / "case.npz"), arrays)
+    stored = np.load(tmp_path / "case.npz").files
+    assert "grad/low" not in stored and gu.LOWRANK + "grad/low/a" in stored and "grad/full" in stored
+    back = gu._read("case")
+    assert set(back) == set(arrays)
+    low = arrays["grad/low"]
+    assert back["grad/low"].dtype == np.float32 and np.abs(back["grad/low"] - low).max() <= 1e-6 * np.abs(low).max()
+    for k in ("grad/full", "logits", "arch"):
+        assert np.array_equal(back[k], arrays[k]), k
+
+
 def test_post_eot_tokens_are_dead():
     """SURVEY.md 8c(i): tokens after EOT do not influence features or gradients (causal mask),
     so the text tower may be truncated to max(eot)+1 rows exactly."""
