@@ -105,13 +105,22 @@ int mudpt_vision_backward(mudpt_handle* h, const float* d_f_img, float* d_prompt
  * are dropped; with seq_len = max(eot)+1 this is exact under the causal mask (SURVEY.md 8c-i). */
 int mudpt_text_set_classes(mudpt_handle* h, const float* embeddings, int32_t C, int32_t src_len, int32_t seq_len,
                            const int32_t* eot_host, void* stream);
+/* The same class set-up with every class at its own length (ragged tower): class c keeps its first len_host[c] tokens,
+ * 1 + n_ctx <= len_host[c] <= min(src_len, 128) and eot_host[c] < len_host[c]; len_c = max(eot_c + 1, 1 + n_ctx) is exact
+ * under the causal mask.  The classes are packed (class c on rows [off_c, off_c + len_c), off_c = sum of the lengths before
+ * it), so no row runs past its class's EOT.  A ragged tower always uses the stand-alone LayerNorm kernels (option
+ * "ln_fused" does not apply) and the warp-MMA attention kernels.  The next mudpt_text_set_classes call makes the tower
+ * padded again. */
+int mudpt_text_set_classes_ragged(mudpt_handle* h, const float* embeddings, int32_t C, int32_t src_len, const int32_t* len_host,
+                                  const int32_t* eot_host, void* stream);
 /* prompts [depth, n_ctx, width]: prompts[0] = ctx + positional_embedding[1:1+n_ctx],
  *         prompts[i>=1] = deep_prompts[i-1] + v2t_text_prompts[i-1] (trainers/mudpt.py:175)
  * splice_layer0 = 0 keeps rows 1..n_ctx of the embeddings as given (per-class ctx, dense API).
  * f_txt [C, embed_dim] */
 int mudpt_text_forward(mudpt_handle* h, const float* prompts, int32_t splice_layer0, float* f_txt, void* stream);
 /* d_f_txt [C, embed_dim] -> d_prompts [depth, n_ctx, width]; d_x0 (optional, may be NULL)
- * [C, seq_len, width] = gradient of the tower input (dense module-level API). */
+ * [C, seq_len, width] = gradient of the tower input (dense module-level API).  Ragged tower: d_x0 is
+ * [C, max(len_host), width] with zeros at positions >= len_c (exact: those tokens do not reach any output). */
 int mudpt_text_backward(mudpt_handle* h, const float* d_f_txt, float* d_prompts, float* d_x0, void* stream);
 
 /* ---- logits + loss head (trainers/mudpt.py:178-182, :250) ---------------------------------------
@@ -148,6 +157,13 @@ int mudpt_attention_forward(const uint16_t* qkv, uint16_t* o, float* lse2, int32
 int mudpt_attention_backward(const uint16_t* qkv, const uint16_t* o, const uint16_t* d_o, const float* lse2,
                              float* dsum_scratch, uint16_t* dqkv, int32_t S, int32_t L, int32_t H, int32_t causal,
                              void* stream);
+/* Causal attention over packed variable-length sequences: sequence s occupies rows [seq_off[s], seq_off[s+1]) of
+ * qkv [M, 3*width] / o / d_o [M, width] / dqkv (seq_off: device int32 [S+1], lengths 1..128, max_len = the longest);
+ * lse2 [M * H] holds sequence s's [H, len_s] block at seq_off[s] * H. */
+int mudpt_attention_varlen_forward(const uint16_t* qkv, uint16_t* o, float* lse2, const int32_t* seq_off, int32_t S,
+                                   int32_t max_len, int32_t H, void* stream);
+int mudpt_attention_varlen_backward(const uint16_t* qkv, const uint16_t* d_o, const float* lse2, uint16_t* dqkv,
+                                    const int32_t* seq_off, int32_t S, int32_t max_len, int32_t H, void* stream);
 /* C = A[M,K] x B[N,K]^T (bf16, fp32 accumulate on tcgen05) with epilogue `mode`:
  * 0 bf16 = acc+bias | 1 f32 = acc+bias | 2 f32 = acc+bias+resid | 3 out0 = h, out1 = QuickGELU(h)
  * 4 bf16 = acc * QuickGELU'(aux) | 5 patch-embedding scatter (+pos) */

@@ -30,6 +30,7 @@ SIGNATURES = {
     "mudpt_vision_forward": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_vision_backward": (C.c_int, [C.c_void_p, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_text_set_classes": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "mudpt_text_set_classes_ragged": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mudpt_text_forward": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, C.c_void_p]),
     "mudpt_text_backward": (C.c_int, [C.c_void_p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_logits_head": (C.c_int, [C.c_void_p, c_f32p, c_f32p, C.c_void_p, C.c_int32, C.c_int32, C.c_float,
@@ -45,6 +46,10 @@ SIGNATURES = {
     "mudpt_attention_forward": (C.c_int, [C.c_void_p, C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "mudpt_attention_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, c_f32p, c_f32p, C.c_void_p, C.c_int32,
                                            C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "mudpt_attention_varlen_forward": (C.c_int, [C.c_void_p, C.c_void_p, c_f32p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                                 C.c_void_p]),
+    "mudpt_attention_varlen_backward": (C.c_int, [C.c_void_p, C.c_void_p, c_f32p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                                  C.c_int32, C.c_void_p]),
     "mudpt_gemm_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                   C.c_void_p, c_f32p, c_f32p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "mudpt_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32]),

@@ -51,8 +51,19 @@ struct Layer {
 struct Tower {
   int d = 0, H = 0, layers = 0, n_ctx = 0, row0 = 0, depth = 0;
   bool causal = false;
-  int L = 0;        // current tokens per sequence
+  int L = 0;        // current tokens per sequence (ragged: the longest sequence)
   int S = 0;        // current sequences
+  int rows = 0;     // token rows: S * L, or (ragged) the sum of the sequence lengths
+  double attn_sq = 0;  // sum over sequences of length^2 (attention FLOP counts)
+  // Ragged text tower (mudpt_text_set_classes_ragged): sequence s occupies the packed rows [seq_off[s], seq_off[s + 1]),
+  // tok_pos[row] = the row's position in its sequence; sel_rows / p0_rows hold absolute rows (row stride row_L() = 0).
+  // The LayerNorms run stand-alone (the fused GEMM epilogues locate prompt rows with row % L).
+  bool ragged = false;
+  int *seq_off = nullptr, *tok_pos = nullptr;
+  size_t off_cap = 0, pos_cap = 0;
+  int row_L() const { return ragged ? 0 : L; }
+  const int* packed_pos() const { return ragged ? tok_pos : nullptr; }  // (the arrays outlive a switch back to padded)
+  const int* packed_off() const { return ragged ? seq_off : nullptr; }
   size_t cap_rows = 0;
   std::vector<Layer> lw;
   bool fold_dirty = true;  // a tensor that enters the LayerNorm folding changed since the last fold
@@ -202,11 +213,19 @@ bool env_flag(const char* name, bool dflt) {
   return e ? atoi(e) != 0 : dflt;
 }
 
-// (re)allocate the activation workspace of a tower for S sequences of L tokens
-int ensure_tower(mudpt_handle* h, Tower& t, int S, int L) {
-  const size_t rows = static_cast<size_t>(S) * L;
+// (re)allocate the activation workspace of a tower for S sequences of L tokens, or (off != null: host row offsets [S+1])
+// for S packed sequences of at most L tokens
+int ensure_tower(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullptr) {
+  const size_t rows = off ? static_cast<size_t>(off[S]) : static_cast<size_t>(S) * L;
   t.S = S;
   t.L = L;
+  t.rows = static_cast<int>(rows);
+  t.ragged = off != nullptr;
+  t.attn_sq = static_cast<double>(S) * L * L;
+  if (off) {
+    t.attn_sq = 0;
+    for (int q = 0; q < S; ++q) t.attn_sq += static_cast<double>(off[q + 1] - off[q]) * (off[q + 1] - off[q]);
+  }
   const size_t head_need = feature_head_workspace_floats(S, t.d, h->cfg.embed_dim);
   if (head_need > t.head_cap) {  // gathered CLS / EOT rows of the feature head + split-K partials
     CUDA_OK(h, dev_alloc(h, &t.head_ws, head_need));
@@ -256,13 +275,13 @@ int ensure_tower(mudpt_handle* h, Tower& t, int S, int L) {
     t.p0_cap = R0;
     t.p0_S = 0;
   }
-  if (R0 > 0 && (t.p0_S != S || t.p0_L != L)) {
+  if (R0 > 0 && (off || t.p0_S != S || t.p0_L != L)) {
     std::vector<int> r(R0);
     for (int q = 0; q < S; ++q)
-      for (int j = 0; j < t.n_ctx; ++j) r[static_cast<size_t>(q) * t.n_ctx + j] = q * L + t.row0 + j;
+      for (int j = 0; j < t.n_ctx; ++j) r[static_cast<size_t>(q) * t.n_ctx + j] = (off ? off[q] : q * L) + t.row0 + j;
     CUDA_OK(h, cudaMemcpy(t.p0_rows, r.data(), R0 * sizeof(int), cudaMemcpyHostToDevice));  // (set-up: shapes change rarely)
     t.p0_S = S;
-    t.p0_L = L;
+    t.p0_L = off ? -1 : L;  // (packed rows: rebuilt on the next set-up)
   }
   if (rows <= t.cap_rows) return 0;
   // grow: the outgrown buffers are released first (cudaFree waits for the device, so nothing in flight uses them);
@@ -415,14 +434,15 @@ int ensure_folded(mudpt_handle* h, Tower& t, cudaStream_t st) {
 // the normalisation in their epilogue (EPI_LN_*: gamma folded into the weight, mean as a rank-1 correction).
 // Precondition of the fused path: x_in[0], xb_in[0], st_in[0] hold the tower input (layer-0 splice excepted).
 int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_splice_layer, cudaStream_t st) {
-  const int M = t.S * t.L, d = t.d;
+  const int M = t.rows, d = t.d;
   const double Md = static_cast<double>(M), dd = d;
-  const double attn_fl = 4.0 * t.S * t.H * static_cast<double>(t.L) * t.L * 64.0;  // QK^T + PV, dense count
+  const double attn_fl = 4.0 * t.H * t.attn_sq * 64.0;  // QK^T + PV, dense count
   // Measured on B200 (profiles/r02_ln_fusion_ab.txt): folding the LayerNorm into the GEMMs saves its 4 B/element read
   // but makes the four forward epilogues heavier (+2 B/element bf16 copy, statistics, rank-1 correction).  For the
   // large HBM-bound tower (text, 77,000 rows) that is a gain; for ~6,000-row towers, whose 25-40 us GEMMs are
   // launch / epilogue bound, the stand-alone LayerNorm kernels are faster: choose by row count unless told otherwise.
-  const bool fused = h->ln_fused == 1 || (h->ln_fused < 0 && M >= 32768);
+  // (ragged towers: always the stand-alone kernels, which take the packed positions)
+  const bool fused = !t.ragged && (h->ln_fused == 1 || (h->ln_fused < 0 && M >= 32768));
   const bool pruned = h->prune;
   const int parts = d / 64;
   auto spliced = [&](int i) { return i < t.depth && i >= first_splice_layer && t.n_ctx > 0 && i < t.layers; };
@@ -445,17 +465,19 @@ int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_spl
     } else {
       CKP(h, st, PC_LN_FWD, 0, Md * dd * 6,
           layernorm_fwd_splice(t.x_in[i], spliced(i) ? prompts + static_cast<size_t>(i) * t.n_ctx * d : nullptr, t.L, t.row0,
-                               spliced(i) ? t.n_ctx : 0, w.ln1_g, w.ln1_b, t.a_buf, true, M, d, kLnEps, st));
+                               spliced(i) ? t.n_ctx : 0, w.ln1_g, w.ln1_b, t.a_buf, true, M, d, kLnEps, st, t.packed_pos()));
       e1.mode = EPI_BF16; e1.bias = w.b_in;
       CKP(h, st, PC_GEMM_QKV, 2.0 * Md * 3 * dd * dd, 2 * (Md * dd + 3 * dd * dd + Md * 3 * dd),
           gemm_bf16_tn(t.a_buf, d, w.w_in, d, e1, M, 3 * d, d, st, &t.gws));
     }
-    CKP(h, st, PC_ATTN_FWD, attn_fl, Md * dd * 2 * 4, attention_fwd(t.qkv[i], t.o[i], t.lse[i], t.S, t.L, t.H, d, t.causal, st));
+    CKP(h, st, PC_ATTN_FWD, attn_fl, Md * dd * 2 * 4,
+        t.ragged ? attention_varlen_fwd(t.qkv[i], t.o[i], t.lse[i], t.seq_off, t.S, t.L, t.H, d, st)
+                 : attention_fwd(t.qkv[i], t.o[i], t.lse[i], t.S, t.L, t.H, d, t.causal, st));
     if (pruned && i == t.layers - 1) {
       // the block's output is consumed on one row per sequence: out-proj and the MLP on S gathered rows
       const int S = t.S;
       const double Sd = S;
-      CKP(h, st, PC_SPLICE, 0, Sd * dd * 12, gather_rows(t.x_in[i], t.o[i], t.sel_rows, S, t.L, t.pr_x, t.pr_o, d, st));
+      CKP(h, st, PC_SPLICE, 0, Sd * dd * 12, gather_rows(t.x_in[i], t.o[i], t.sel_rows, S, t.row_L(), t.pr_x, t.pr_o, d, st));
       GemmEpilogue p2;
       p2.out0 = t.pr_xm; p2.bias = w.b_out; p2.resid = t.pr_x; p2.ldc = d;
       if (fused) { p2.mode = EPI_RESID_STATS; p2.out2 = t.pr_xmb; p2.stats_out = t.pr_stm; }
@@ -518,7 +540,7 @@ int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_spl
 // x (and the row stride) the feature head reads its one row per sequence from
 const float* tower_head_input(const Tower& t, const int** rows, int* L) {
   if (t.fwd_pruned) { *rows = nullptr; *L = 1; return t.pr_xo; }
-  *rows = t.sel_rows; *L = t.L;
+  *rows = t.sel_rows; *L = t.row_L();
   return t.x_in[t.layers];
 }
 
@@ -529,9 +551,9 @@ const float* tower_head_input(const Tower& t, const int** rows, int* L) {
 //   mean(g) = (1/d) dout . colsum,   mean(g xhat) = (1/d) dout . (y - b')      (dout = the GEMM's A operand, y = the
 // saved output of the forward LN-GEMM), so the PRODUCER of dout (GELU' epilogue, attention backward) emits them.
 int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice_layer, cudaStream_t st, bool need_dx0 = false) {
-  const int M = t.S * t.L, d = t.d;
+  const int M = t.rows, d = t.d;
   const double Md = static_cast<double>(M), dd = d;
-  const double attn_fl = 2.5 * 4.0 * t.S * t.H * static_cast<double>(t.L) * t.L * 64.0;  // SURVEY.md 8d: 2.5x forward
+  const double attn_fl = 2.5 * 4.0 * t.H * t.attn_sq * 64.0;  // SURVEY.md 8d: 2.5x forward
   const bool fused = t.fwd_fused && h->ln_bwd_fused;  // (the fused forward also keeps the fp32 LN inputs the kernel needs)
   // stand-alone LayerNorm backward after a fused forward: the bf16 row + its exact statistics instead of the fp32 row
   // (14 instead of 16 B/element on an HBM-bound kernel; xhat from bf16(x) -- the operand precision of every GEMM here)
@@ -549,7 +571,7 @@ int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice
     const bool rb = has_resid && !f32_whole;
     const void* resid = !has_resid ? nullptr : (rb ? static_cast<const void*>(t.dx_bf16) : static_cast<const void*>(t.dx));
     const char* e = layernorm_bwd_stream(t.a_buf, true, xrow, stats, gamma, resid, rb, t.dx, t.dx_bf16, M, d, kLnEps, t.L, t.row0,
-                                         whole_f32_out ? -1 : t.n_ctx, st);
+                                         whole_f32_out ? -1 : t.n_ctx, st, t.packed_pos());
     f32_whole = whole_f32_out;
     return e;
   };
@@ -581,7 +603,7 @@ int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice
       CKP(h, st, PC_GEMM, 2.0 * Sd * dd * dd, 2 * (2 * Sd * dd + dd * dd), gemm_bf16_tn(t.pr_dxb, d, w.w_out_t, d, p3, S, d, d, st, &t.gws));
       // dO of the whole block: zero but for the S consumed rows
       CUDA_OK(h, cudaMemsetAsync(t.do_buf, 0, static_cast<size_t>(M) * d * sizeof(bf16), st));
-      CKP(h, st, PC_SPLICE, 0, Sd * dd * 4, scatter_rows_bf16(t.pr_do, t.sel_rows, S, t.L, t.do_buf, d, st));
+      CKP(h, st, PC_SPLICE, 0, Sd * dd * 4, scatter_rows_bf16(t.pr_do, t.sel_rows, S, t.row_L(), t.do_buf, d, st));
     } else {
     // MLP branch: dg = dx W_pr ; dh = dg * GELU'(h) ; dm = dh W_fc ; dx += LN2_bwd(dm)
     GemmEpilogue e1;
@@ -610,8 +632,9 @@ int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice
     CKP(h, st, PC_GEMM_DOUT, 2.0 * Md * dd * dd, 2 * (2 * Md * dd + dd * dd), gemm_bf16_tn(t.dx_bf16, d, w.w_out_t, d, e3, M, d, d, st, &t.gws));
     }
     CKP(h, st, PC_ATTN_BWD, attn_fl, Md * dd * 2 * 8,
-        attention_bwd(t.qkv[i], t.o[i], t.do_buf, t.lse[i], t.dsum, t.dqkv_buf, t.S, t.L, t.H, d, t.causal, st,
-                      fused ? w.sb_in : nullptr, fused ? t.dots : nullptr));
+        t.ragged ? attention_varlen_bwd(t.qkv[i], t.do_buf, t.lse[i], t.dqkv_buf, t.seq_off, t.S, t.L, t.H, d, st)
+                 : attention_bwd(t.qkv[i], t.o[i], t.do_buf, t.lse[i], t.dsum, t.dqkv_buf, t.S, t.L, t.H, d, t.causal, st,
+                                 fused ? w.sb_in : nullptr, fused ? t.dots : nullptr));
     // exact work skipping below block 0: only the prompt rows of its input gradient are ever read (by the splice backward)
     const bool head_pruned = i == 0 && h->prune && !fused && !tail_pruned && !need_dx0 && first_splice_layer == 0 && t.depth > 0 &&
                              t.n_ctx > 0 && t.S * t.n_ctx < M;
@@ -627,7 +650,7 @@ int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice
       CKP(h, st, PC_SPLICE, 0, Rd * dd * 8, gather_rows(t.dx, nullptr, t.p0_rows, R, 0, t.p0_dx, nullptr, d, st));
       CKP(h, st, PC_LN_BWD, 0, Rd * dd * 16, layernorm_bwd(t.p0_a, true, t.p0_x, nullptr, w.ln1_g, t.p0_dx, t.p0_dx, t.p0_dxb, R, d, kLnEps, st));
       CKP(h, st, PC_SPLICE, 0, Rd * dd * 8, scatter_rows(t.p0_dx, t.p0_rows, R, 0, t.dx, nullptr, d, false, st));
-      CKP(h, st, PC_SPLICE, 0, t.S * t.n_ctx * dd * 4, splice_bwd(t.dx, t.dx_bf16, d_prompts, t.splice_ws, t.S, t.L, t.row0, t.n_ctx, d, false, st));
+      CKP(h, st, PC_SPLICE, 0, t.S * t.n_ctx * dd * 4, splice_bwd(t.dx, t.dx_bf16, d_prompts, t.splice_ws, t.S, t.L, t.row0, t.n_ctx, d, false, st, t.packed_off()));
       continue;
     }
     GemmEpilogue e4;
@@ -647,12 +670,13 @@ int tower_backward(mudpt_handle* h, Tower& t, float* d_prompts, int first_splice
                       tail_pruned));
     }
     if (tail_pruned)  // the residual path of the S consumed rows (everything else of it is zero)
-      CKP(h, st, PC_SPLICE, 0, t.S * dd * 14, scatter_rows(t.pr_dx, t.sel_rows, t.S, t.L, t.dx, t.dx_bf16, d, true, st));
+      CKP(h, st, PC_SPLICE, 0, t.S * dd * 14, scatter_rows(t.pr_dx, t.sel_rows, t.S, t.row_L(), t.dx, t.dx_bf16, d, true, st));
     // splice backward: the inserted prompt rows collect the batch-summed gradient; the rows
     // they overwrote get none (clip/model.py:281-297, SURVEY.md 3.3)
     if (i < t.depth && i >= first_splice_layer && t.n_ctx > 0)
       CKP(h, st, PC_SPLICE, 0, t.S * t.n_ctx * dd * 4,
-          splice_bwd(t.dx, t.dx_bf16, d_prompts + static_cast<size_t>(i) * t.n_ctx * d, t.splice_ws, t.S, t.L, t.row0, t.n_ctx, d, i > 0, st));
+          splice_bwd(t.dx, t.dx_bf16, d_prompts + static_cast<size_t>(i) * t.n_ctx * d, t.splice_ws, t.S, t.L, t.row0, t.n_ctx, d, i > 0, st,
+                     t.packed_off()));
   }
   return 0;
 }
@@ -665,10 +689,10 @@ int head_backward(mudpt_handle* h, Tower& t, const float* d_f, const float* gamm
     CK(h, feature_head_bwd(d_f, t.pr_xo, nullptr, gamma, proj, t.pr_dx, t.pr_dxb, t.head_ws, t.S, 1, t.d, e, kLnEps, st));
     return 0;
   }
-  const size_t n = static_cast<size_t>(t.S) * t.L * t.d;
+  const size_t n = static_cast<size_t>(t.rows) * t.d;
   CUDA_OK(h, cudaMemsetAsync(t.dx, 0, n * sizeof(float), st));
   CUDA_OK(h, cudaMemsetAsync(t.dx_bf16, 0, n * sizeof(bf16), st));
-  CK(h, feature_head_bwd(d_f, t.x_in[t.layers], t.sel_rows, gamma, proj, t.dx, t.dx_bf16, t.head_ws, t.S, t.L, t.d, e, kLnEps, st));
+  CK(h, feature_head_bwd(d_f, t.x_in[t.layers], t.sel_rows, gamma, proj, t.dx, t.dx_bf16, t.head_ws, t.S, t.row_L(), t.d, e, kLnEps, st));
   return 0;
 }
 
@@ -876,6 +900,57 @@ int mudpt_text_set_classes(mudpt_handle* h, const float* embeddings, int32_t C, 
   return 0;
 }
 
+int mudpt_text_set_classes_ragged(mudpt_handle* h, const float* embeddings, int32_t C, int32_t src_len, const int32_t* len_host,
+                                  const int32_t* eot_host, void* stream) {
+  if (!h || !embeddings || !len_host || !eot_host) return fail(h, "mudpt_text_set_classes_ragged: null argument");
+  const mudpt_config& c = h->cfg;
+  if (C <= 0 || src_len <= 0 || src_len > c.context_length)
+    return fail(h, "mudpt_text_set_classes_ragged: bad lengths (C=%d src_len=%d)", C, src_len);
+  const int max_ok = src_len < attention_varlen_max_len() ? src_len : attention_varlen_max_len();
+  int max_len = 0;
+  for (int i = 0; i < C; ++i) {
+    if (len_host[i] < 1 + c.n_ctx || len_host[i] > max_ok)
+      return fail(h, "mudpt_text_set_classes_ragged: len[%d]=%d outside [%d, %d] (SOT + n_ctx .. src_len, at most %d)", i, len_host[i],
+                  1 + c.n_ctx, max_ok, attention_varlen_max_len());
+    if (eot_host[i] < 0 || eot_host[i] >= len_host[i])
+      return fail(h, "mudpt_text_set_classes_ragged: eot[%d]=%d outside len %d", i, eot_host[i], len_host[i]);
+    max_len = len_host[i] > max_len ? len_host[i] : max_len;
+  }
+  if (!(h->stem_have & SB_POS_T)) return fail(h, "mudpt_text_set_classes_ragged: positional_embedding not set");
+  cudaSetDevice(c.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  Tower& t = h->txt;
+  std::vector<int> off(C + 1, 0), sel(C);
+  for (int i = 0; i < C; ++i) {
+    off[i + 1] = off[i] + len_host[i];
+    sel[i] = off[i] + eot_host[i];  // absolute EOT row
+  }
+  const int M = off[C];
+  std::vector<int> pos(M);
+  for (int i = 0; i < C; ++i)
+    for (int j = 0; j < len_host[i]; ++j) pos[off[i] + j] = j;
+  if (ensure_tower(h, t, C, max_len, off.data())) return -1;
+  if (static_cast<size_t>(C) > h->eot_cap) {
+    CUDA_OK(h, dev_alloc(h, &h->eot, static_cast<size_t>(C)));
+    h->eot_cap = C;
+  }
+  if (static_cast<size_t>(C) + 1 > t.off_cap) {
+    CUDA_OK(h, dev_alloc(h, &t.seq_off, static_cast<size_t>(C) + 1));
+    t.off_cap = static_cast<size_t>(C) + 1;
+  }
+  if (static_cast<size_t>(M) > t.pos_cap) {
+    CUDA_OK(h, dev_alloc(h, &t.tok_pos, static_cast<size_t>(M)));
+    t.pos_cap = M;
+  }
+  CUDA_OK(h, cudaMemcpyAsync(h->eot, sel.data(), C * sizeof(int), cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaMemcpyAsync(t.seq_off, off.data(), (C + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaMemcpyAsync(t.tok_pos, pos.data(), M * sizeof(int), cudaMemcpyHostToDevice, st));
+  CUDA_OK(h, cudaStreamSynchronize(st));  // (the host vectors go out of scope)
+  CK(h, add_positional(t.x_in[0], embeddings, h->pos_t, C, max_len, src_len, t.d, st, t.seq_off));
+  t.fwd_done = false;
+  return 0;
+}
+
 int mudpt_text_forward(mudpt_handle* h, const float* prompts, int32_t splice_layer0, float* f_txt, void* stream) {
   if (!h || !f_txt || (!prompts && h->cfg.n_ctx > 0)) return fail(h, "mudpt_text_forward: null argument");
   if (mudpt_weights_complete(h)) return -1;
@@ -898,10 +973,11 @@ int mudpt_text_backward(mudpt_handle* h, const float* d_f_txt, float* d_prompts,
   if (!t.fwd_done) return fail(h, "mudpt_text_backward: no forward pass to differentiate");
   cudaSetDevice(h->cfg.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t n = static_cast<size_t>(t.S) * t.L * t.d;
+  const size_t n = static_cast<size_t>(t.rows) * t.d;
   if (head_backward(h, t, d_f_txt, h->ln_final_g, h->proj_t, st)) return -1;
   if (tower_backward(h, t, d_prompts, t.first_splice, st, d_x0 != nullptr)) return -1;
-  if (d_x0) CUDA_OK(h, cudaMemcpyAsync(d_x0, t.dx, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  if (d_x0 && t.ragged) CK(h, unpack_rows(t.dx, t.seq_off, t.S, t.L, t.d, d_x0, st));
+  else if (d_x0) CUDA_OK(h, cudaMemcpyAsync(d_x0, t.dx, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 
@@ -985,6 +1061,18 @@ int mudpt_attention_backward(const uint16_t* qkv, const uint16_t* o, const uint1
                              uint16_t* dqkv, int32_t S, int32_t L, int32_t H, int32_t causal, void* stream) {
   CKG(attention_bwd(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<const bf16*>(o), reinterpret_cast<const bf16*>(d_o),
                     lse2, dsum, reinterpret_cast<bf16*>(dqkv), S, L, H, H * 64, causal != 0, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+int mudpt_attention_varlen_forward(const uint16_t* qkv, uint16_t* o, float* lse2, const int32_t* seq_off, int32_t S, int32_t max_len,
+                                   int32_t H, void* stream) {
+  CKG(attention_varlen_fwd(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(o), lse2, seq_off, S, max_len, H, H * 64,
+                           static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+int mudpt_attention_varlen_backward(const uint16_t* qkv, const uint16_t* d_o, const float* lse2, uint16_t* dqkv, const int32_t* seq_off,
+                                    int32_t S, int32_t max_len, int32_t H, void* stream) {
+  CKG(attention_varlen_bwd(reinterpret_cast<const bf16*>(qkv), reinterpret_cast<const bf16*>(d_o), lse2, reinterpret_cast<bf16*>(dqkv),
+                           seq_off, S, max_len, H, H * 64, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 // stream-K scratch of the handle-less GEMM entry points (tests, one stream at a time)
@@ -1120,7 +1208,7 @@ int mudpt_debug_buffer(mudpt_handle* h, int32_t tower, const char* name, int32_t
   if (!h || !name || !ptr || !numel) return fail(h, "mudpt_debug_buffer: null argument");
   Tower& t = tower == MUDPT_TOWER_VISION ? h->vis : h->txt;
   if (t.cap_rows == 0) return fail(h, "mudpt_debug_buffer: tower has no workspace yet");
-  const int64_t rows = static_cast<int64_t>(t.S) * t.L;
+  const int64_t rows = t.rows;
   if (!strcmp(name, "dx")) { *ptr = t.dx; *numel = rows * t.d; return 0; }
   if (!strcmp(name, "x_in")) {
     if (layer < 0 || layer > t.layers) return fail(h, "mudpt_debug_buffer: layer out of range");

@@ -614,36 +614,64 @@ __device__ __forceinline__ void short_fwd_body(uint8_t* smem, uint32_t sQ, uint3
 // 77-token text tower (5 tiles) does not pay for 128-token sequences (8 tiles).
 constexpr int short_min_ctas(int maxt, bool bwd) { return maxt <= 2 ? 8 : maxt <= 5 ? (bwd ? 3 : 5) : (bwd ? 1 : 2); }
 
+// One (sequence, head) problem: the sequence occupies rows [seq_row, seq_row + L) of qkv / o, its lse2 row block starts at
+// lse_base.  The CTA may have more warps than the sequence has 16-row tiles (variable-length launches are sized by the
+// longest sequence): those warps help with the loads and leave after the only block-wide barrier.
 template <bool CAUSAL, int MAXT>
-__global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, false)) attn_short_fwd_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ o,
-                                                                              float* __restrict__ lse2, int L, int H, int d,
-                                                                              float scale_log2e) {
-  extern __shared__ __align__(128) uint8_t smem[];
+__device__ __forceinline__ void short_fwd_cta(uint8_t* smem, const bf16* qkv, bf16* o, float* lse_base, size_t seq_row, int L, int h,
+                                              int d, float scale_log2e) {
   const int nw = blockDim.x >> 5, Lp = nw * 16;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
   const uint32_t sQ = smem_u32(smem), sK = sQ + Lp * ROW_BYTES, sV = sK + Lp * ROW_BYTES;
   const int ld = 3 * d;
-  const bf16* base = qkv + static_cast<size_t>(s) * L * ld + h * DH;
-  pdl_wait();
-  pdl_trigger();
+  const bf16* base = qkv + seq_row * ld + h * DH;
   load_tile(sQ, base, ld, 0, L, Lp);
   load_tile(sK, base + d, ld, 0, L, Lp);
   load_tile(sV, base + 2 * d, ld, 0, L, Lp);
   cp_async_commit();
   cp_async_wait_all();
   __syncthreads();
-  bf16* ob = o + static_cast<size_t>(s) * L * d + h * DH;
-  float* lb = lse2 + (static_cast<size_t>(s) * H + h) * L;
-  const int T = CAUSAL ? warp + 1 : nw;
+  const int nt = (L + 15) >> 4;
+  if (warp >= nt) return;
+  bf16* ob = o + seq_row * d + h * DH;
+  const int T = CAUSAL ? warp + 1 : nt;
 #define MUDPT_FWD_CASE(k) \
-  case k: if constexpr (MAXT >= k) short_fwd_body<CAUSAL, k>(smem, sQ, sK, sV, warp, L, lane, scale_log2e, ob, d, lb); break;
+  case k: if constexpr (MAXT >= k) short_fwd_body<CAUSAL, k>(smem, sQ, sK, sV, warp, L, lane, scale_log2e, ob, d, lse_base); break;
   switch (T) {
     MUDPT_FWD_CASE(1) MUDPT_FWD_CASE(2) MUDPT_FWD_CASE(3) MUDPT_FWD_CASE(4)
     MUDPT_FWD_CASE(5) MUDPT_FWD_CASE(6) MUDPT_FWD_CASE(7) MUDPT_FWD_CASE(8)
     default: break;
   }
 #undef MUDPT_FWD_CASE
+}
+
+template <bool CAUSAL, int MAXT>
+__global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, false)) attn_short_fwd_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ o,
+                                                                              float* __restrict__ lse2, int L, int H, int d,
+                                                                              float scale_log2e) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
+  pdl_wait();
+  pdl_trigger();
+  short_fwd_cta<CAUSAL, MAXT>(smem, qkv, o, lse2 + (static_cast<size_t>(s) * H + h) * L, static_cast<size_t>(s) * L, L, h, d, scale_log2e);
+}
+
+// Packed variable-length causal sequences (the ragged text tower): sequence s occupies rows [seq_off[s], seq_off[s + 1]); its
+// lse2 block is [H, len_s] at seq_off[s] * H (with equal lengths: the layout and the results of attn_short_fwd_kernel).
+// 3 instead of 5 resident CTAs for the 3-5 tile forward: its 16 x 80 score block, P fragments, Q fragments and output
+// accumulator need ~110 registers, and 5 (4) CTAs cap it at 80 (96), where it spills.
+constexpr int varlen_min_ctas(int maxt, bool bwd) { return maxt <= 2 ? 8 : maxt <= 5 ? 3 : (bwd ? 1 : 2); }
+
+template <int MAXT>
+__global__ void __launch_bounds__(MAXT * 32, varlen_min_ctas(MAXT, false)) attn_varlen_fwd_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ o,
+                                                                               float* __restrict__ lse2, const int* __restrict__ seq_off,
+                                                                               int H, int d, float scale_log2e) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
+  pdl_wait();
+  pdl_trigger();
+  const int r0 = seq_off[s], L = seq_off[s + 1] - r0;
+  short_fwd_cta<true, MAXT>(smem, qkv, o, lse2 + static_cast<size_t>(r0) * H + static_cast<size_t>(h) * L, r0, L, h, d, scale_log2e);
 }
 
 // Phase 1 of the fused backward for query tile t: returns dQ in `dq`, P / dS (bf16, accumulator
@@ -733,26 +761,19 @@ __device__ __forceinline__ void short_bwd_phase1(uint32_t sQ, uint32_t sdO, uint
   }
 }
 
+// One (sequence, head) problem of the fused backward (rows [seq_row, seq_row + L), lse2 row block at lse_base).  Warps
+// past the sequence's last 16-row tile (variable-length launches) do no work but reach both block-wide barriers.
 template <bool CAUSAL, int MAXT>
-__global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_short_bwd_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ o,
-                                                                              const bf16* __restrict__ d_o,
-                                                                              const float* __restrict__ lse2,
-                                                                              bf16* __restrict__ dqkv, int L, int H, int d,
-                                                                              float scale, float scale_log2e,
-                                                                              const float2* __restrict__ ln_sb,
-                                                                              float2* __restrict__ ln_dots) {
-  extern __shared__ __align__(128) uint8_t smem[];
+__device__ __forceinline__ void short_bwd_cta(uint8_t* smem, const bf16* qkv, const bf16* d_o, const float* lse_base, bf16* dqkv,
+                                              size_t seq_row, int L, int h, int H, int d, float scale, float scale_log2e,
+                                              const float2* ln_sb, float2* ln_dots) {
   const int nw = blockDim.x >> 5, Lp = nw * 16;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
   // [Q | dO | K | V | pad]; after phase 1 the K / V / pad region is reused for P and dS
   const uint32_t tile_bytes = Lp * ROW_BYTES;
   const uint32_t sQ = smem_u32(smem), sdO = sQ + tile_bytes, sK = sdO + tile_bytes, sV = sK + tile_bytes;
   const int ld = 3 * d;
-  const size_t seq_row = static_cast<size_t>(s) * L;
   const bf16* base = qkv + seq_row * ld + h * DH;
-  pdl_wait();
-  pdl_trigger();
   load_tile(sQ, base, ld, 0, L, Lp);
   load_tile(sdO, d_o + seq_row * d + h * DH, d, 0, L, Lp);
   load_tile(sK, base + d, ld, 0, L, Lp);
@@ -760,16 +781,17 @@ __global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_sh
   cp_async_commit();
   const int row0 = warp * 16;
   const int qr = row0 + (lane >> 2);
-  const size_t stat_base = (static_cast<size_t>(s) * H + h) * L;
   // rows >= L: lse = 0 with zero Q / dO rows gives finite p, dP = 0, hence D = 0 and dS = 0: no contribution to dK / dV
-  const float lse0 = qr < L ? lse2[stat_base + qr] : 0.f;
-  const float lse1 = qr + 8 < L ? lse2[stat_base + qr + 8] : 0.f;
+  const float lse0 = qr < L ? lse_base[qr] : 0.f;
+  const float lse1 = qr + 8 < L ? lse_base[qr + 8] : 0.f;
   cp_async_wait_all();
   __syncthreads();
 
   float dq[8][4];
   uint32_t pp[2 * MAXT][2], ds[2 * MAXT][2];
-  const int T = CAUSAL ? warp + 1 : nw;
+  const int ntiles = (L + 15) >> 4;  // live tiles; warps past them take part in the barriers only
+  const bool live = warp < ntiles;
+  const int T = !live ? 0 : CAUSAL ? warp + 1 : ntiles;
 #define MUDPT_BWD_CASE(k) \
   case k: if constexpr (MAXT >= k) short_bwd_phase1<CAUSAL, k, MAXT>(sQ, sdO, sK, sV, warp, L, lane, scale_log2e, lse0, lse1, dq, pp, ds); break;
   switch (T) {
@@ -782,7 +804,7 @@ __global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_sh
   const uint32_t stride = ps_stride(Lp);
   uint8_t* gP = smem + 2 * tile_bytes;
   uint8_t* gS = gP + Lp * stride;
-  {
+  if (live) {
     // accumulator fragment layout: rows (lane/4, +8), column pair 2*(lane%4) of each 8-column tile
     const uint32_t r_lo = static_cast<uint32_t>(row0 + (lane >> 2)) * stride + (lane & 3) * 4;
     const uint32_t r_hi = r_lo + 8 * stride;
@@ -803,7 +825,7 @@ __global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_sh
   zero_acc(dk);
   zero_acc(dv);
   const uint32_t aP = smem_u32(gP), aS = smem_u32(gS);
-  for (int g = CAUSAL ? warp : 0; g < nw; ++g) {
+  for (int g = CAUSAL ? warp : 0; live && g < ntiles; ++g) {
     // A = (P^T)[keys row0.., queries 16g..]: 8x8 blocks of P (rows = queries) read transposed.
     // a0..a3 = blocks (queries 0-7, keys 0-7), (q 0-7, keys 8-15), (q 8-15, keys 0-7), (q 8-15, keys 8-15):
     // lanes 8i..8i+7 address the 8 query rows of block i
@@ -826,7 +848,7 @@ __global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_sh
   }
   __syncthreads();  // all reads of Q / dO / P / dS are done: the Q and dO tiles become store staging
   bf16* out = dqkv + seq_row * ld + h * DH;
-  if (row0 < L) {
+  if (live) {
     RowDots rq, rk, rv;
     if (ln_dots != nullptr) {
       rq.sb = ln_sb + h * DH; rq.y = base; rq.out = ln_dots + seq_row * 3 * H; rq.parts = 3 * H; rq.part = h;
@@ -838,6 +860,40 @@ __global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_sh
     __syncwarp();
     store_rows_bf16(dv, 1.f, 1.f, smem, 0, row0, out + 2 * d, ld, row0, L, lane, rv);
   }
+}
+
+template <bool CAUSAL, int MAXT>
+__global__ void __launch_bounds__(MAXT * 32, short_min_ctas(MAXT, true)) attn_short_bwd_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ o,
+                                                                              const bf16* __restrict__ d_o,
+                                                                              const float* __restrict__ lse2,
+                                                                              bf16* __restrict__ dqkv, int L, int H, int d,
+                                                                              float scale, float scale_log2e,
+                                                                              const float2* __restrict__ ln_sb,
+                                                                              float2* __restrict__ ln_dots) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
+  pdl_wait();
+  pdl_trigger();
+  short_bwd_cta<CAUSAL, MAXT>(smem, qkv, d_o, lse2 + (static_cast<size_t>(s) * H + h) * L, dqkv, static_cast<size_t>(s) * L, L, h, H, d,
+                              scale, scale_log2e, ln_sb, ln_dots);
+}
+
+// Backward of attn_varlen_fwd_kernel (same packed layout).
+template <int MAXT>
+__global__ void __launch_bounds__(MAXT * 32, varlen_min_ctas(MAXT, true)) attn_varlen_bwd_kernel(const bf16* __restrict__ qkv,
+                                                                               const bf16* __restrict__ d_o,
+                                                                               const float* __restrict__ lse2,
+                                                                               bf16* __restrict__ dqkv, const int* __restrict__ seq_off,
+                                                                               int H, int d, float scale, float scale_log2e,
+                                                                               const float2* __restrict__ ln_sb,
+                                                                               float2* __restrict__ ln_dots) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int sh = blockIdx.x, s = sh / H, h = sh - s * H;
+  pdl_wait();
+  pdl_trigger();
+  const int r0 = seq_off[s], L = seq_off[s + 1] - r0;
+  short_bwd_cta<true, MAXT>(smem, qkv, d_o, lse2 + static_cast<size_t>(r0) * H + static_cast<size_t>(h) * L, dqkv, r0, L, h, H, d,
+                              scale, scale_log2e, ln_sb, ln_dots);
 }
 
 static size_t short_bwd_smem(int Lp) {
@@ -920,6 +976,50 @@ const char* attention_fwd(const bf16* qkv, bf16* o, float* lse2, int S, int L, i
   }
   count_launch(1);
   return launch_status("attention fwd launch failed");
+}
+
+// Varlen launches (causal): one CTA per (sequence, head), sized by the longest sequence (16-row tiles, <= SHORT_MAX_TILES).
+int attention_varlen_max_len() { return 16 * SHORT_MAX_TILES; }
+
+const char* attention_varlen_fwd(const bf16* qkv, bf16* o, float* lse2, const int* seq_off, int S, int max_len, int H, int d,
+                                 cudaStream_t stream) {
+  if (S <= 0) return nullptr;
+  if (d != H * DH) return "attention: head width must be 64";
+  if (max_len <= 0 || max_len > 16 * SHORT_MAX_TILES) return "attention (varlen): sequences must have 1..128 tokens";
+  const float sl2 = 0.125f * 1.4426950408889634f;
+  const int tiles = (max_len + 15) / 16;
+  const size_t sm = 3u * tiles * 16 * ROW_BYTES;
+  const char* es = nullptr;
+#define MUDPT_LAUNCH_VFWD(MT)                                                                                     \
+  do {                                                                                                            \
+    if ((es = set_smem(attn_varlen_fwd_kernel<MT>, sm))) return es;                                               \
+    launch_pdl(attn_varlen_fwd_kernel<MT>, dim3(S * H), dim3(tiles * 32), sm, stream, qkv, o, lse2, seq_off, H, d, sl2); \
+  } while (0)
+  if (tiles <= 2) MUDPT_LAUNCH_VFWD(2); else if (tiles <= 5) MUDPT_LAUNCH_VFWD(5); else MUDPT_LAUNCH_VFWD(8);
+#undef MUDPT_LAUNCH_VFWD
+  count_launch(1);
+  return launch_status("attention fwd (varlen) launch failed");
+}
+
+const char* attention_varlen_bwd(const bf16* qkv, const bf16* d_o, const float* lse2, bf16* dqkv, const int* seq_off, int S, int max_len,
+                                 int H, int d, cudaStream_t stream, const float2* ln_sb, float2* ln_dots) {
+  if (S <= 0) return nullptr;
+  if (d != H * DH) return "attention: head width must be 64";
+  if (max_len <= 0 || max_len > 16 * SHORT_MAX_TILES) return "attention (varlen): sequences must have 1..128 tokens";
+  const int tiles = (max_len + 15) / 16;
+  const size_t sm = short_bwd_smem(tiles * 16);
+  const char* es = nullptr;
+  const float sc = 0.125f, sl2s = 0.125f * 1.4426950408889634f;
+#define MUDPT_LAUNCH_VBWD(MT)                                                                                      \
+  do {                                                                                                             \
+    if ((es = set_smem(attn_varlen_bwd_kernel<MT>, sm))) return es;                                                \
+    launch_pdl(attn_varlen_bwd_kernel<MT>, dim3(S * H), dim3(tiles * 32), sm, stream, qkv, d_o, lse2, dqkv, seq_off, H, d, sc, sl2s, \
+               ln_sb, ln_dots);                                                                                    \
+  } while (0)
+  if (tiles <= 2) MUDPT_LAUNCH_VBWD(2); else if (tiles <= 5) MUDPT_LAUNCH_VBWD(5); else MUDPT_LAUNCH_VBWD(8);
+#undef MUDPT_LAUNCH_VBWD
+  count_launch(1);
+  return launch_status("attention bwd (varlen) launch failed");
 }
 
 const char* attention_bwd(const bf16* qkv, const bf16* o, const bf16* d_o, const float* lse2, float* dsum, bf16* dqkv,

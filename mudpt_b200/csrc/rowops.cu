@@ -21,13 +21,14 @@ static constexpr int LN_MAXV = 8;  // float4 per lane -> width <= 1024
 // do not pay registers for wide ones). OUT_BF16: normalized row as bf16 (GEMM A operand); else fp32
 // (may alias x).
 template <int NV, bool OUT_BF16>
-// sp_prompt != nullptr: the deep-prompt splice of the block is done here too -- rows (row % sp_L) in [sp_row0, sp_row0 + sp_n)
-// take their values from sp_prompt (copied verbatim into x: bit-exact, clip/model.py:281-297) before being normalised.
+// sp_prompt != nullptr: the deep-prompt splice of the block is done here too -- rows whose position (row % sp_L, or sp_pos[row]
+// for packed variable-length sequences) is in [sp_row0, sp_row0 + sp_n) take their values from sp_prompt (copied verbatim into x: bit-exact, clip/model.py:281-297) before being normalised.
 // (x is read through the read-only path; x_w is the same buffer, written for spliced rows only -- rows that are never read)
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, float* __restrict__ x_w,
                                                      const float* __restrict__ gamma, const float* __restrict__ beta,
                                                      void* __restrict__ out, int M, int d, float eps,
-                                                     const float* __restrict__ sp_prompt, int sp_L, int sp_row0, int sp_n) {
+                                                     const float* __restrict__ sp_prompt, int sp_L, int sp_row0, int sp_n,
+                                                     const int* __restrict__ sp_pos) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   pdl_wait();
@@ -37,7 +38,7 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
   const float* src = x + static_cast<size_t>(row) * d;
   bool spliced = false;
   if (sp_prompt != nullptr) {
-    const int pos = row % sp_L - sp_row0;
+    const int pos = (sp_pos != nullptr ? sp_pos[row] : row % sp_L) - sp_row0;
     if (pos >= 0 && pos < sp_n) {
       src = sp_prompt + static_cast<size_t>(pos) * d;
       spliced = true;
@@ -107,37 +108,37 @@ static int ln_warps() {
 
 template <int NV>
 static void launch_ln_fwd(float* x, const float* gamma, const float* beta, void* out, bool out_bf16, int M, int d, float eps,
-                          const float* sp_prompt, int sp_L, int sp_row0, int sp_n, cudaStream_t stream) {
+                          const float* sp_prompt, int sp_L, int sp_row0, int sp_n, const int* sp_pos, cudaStream_t stream) {
   const int wpc = ln_warps();
   const int grid = (M + wpc - 1) / wpc;
   if (out_bf16)
-    launch_pdl(ln_fwd_kernel<NV, true>, dim3(grid), dim3(32 * wpc), 0, stream, x, x, gamma, beta, out, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n);
+    launch_pdl(ln_fwd_kernel<NV, true>, dim3(grid), dim3(32 * wpc), 0, stream, x, x, gamma, beta, out, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos);
   else
-    launch_pdl(ln_fwd_kernel<NV, false>, dim3(grid), dim3(32 * wpc), 0, stream, x, x, gamma, beta, out, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n);
+    launch_pdl(ln_fwd_kernel<NV, false>, dim3(grid), dim3(32 * wpc), 0, stream, x, x, gamma, beta, out, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos);
 }
 
 // (defined with the pipeline kernels below) true when the shared-memory pipeline took the launch; *err is set if it failed
 static bool ln_fwd_pipe_try(float* x, const float* gamma, const float* beta, bf16* out, int M, int d, float eps, const float* sp_prompt,
-                            int sp_L, int sp_row0, int sp_n, cudaStream_t stream, const char** err);
+                            int sp_L, int sp_row0, int sp_n, const int* sp_pos, cudaStream_t stream, const char** err);
 
 static const char* ln_fwd_dispatch(float* x, const float* gamma, const float* beta, void* out, bool out_bf16, int M, int d, float eps,
-                                   const float* sp_prompt, int sp_L, int sp_row0, int sp_n, cudaStream_t stream) {
+                                   const float* sp_prompt, int sp_L, int sp_row0, int sp_n, const int* sp_pos, cudaStream_t stream) {
   if (M <= 0) return nullptr;
   if (d % 4 != 0 || d > LN_MAXV * 128) return "layernorm: width must be a multiple of 4 and <= 1024";
   if (out_bf16) {
     const char* e = nullptr;
-    if (ln_fwd_pipe_try(x, gamma, beta, reinterpret_cast<bf16*>(out), M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream, &e)) {
+    if (ln_fwd_pipe_try(x, gamma, beta, reinterpret_cast<bf16*>(out), M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream, &e)) {
       if (e) return e;
       count_launch(1);
       return launch_status("layernorm fwd (pipeline) launch failed");
     }
   }
   switch (pick_nv(d)) {
-    case 1: launch_ln_fwd<1>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream); break;
-    case 2: launch_ln_fwd<2>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream); break;
-    case 4: launch_ln_fwd<4>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream); break;
-    case 6: launch_ln_fwd<6>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream); break;
-    default: launch_ln_fwd<8>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, stream); break;
+    case 1: launch_ln_fwd<1>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream); break;
+    case 2: launch_ln_fwd<2>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream); break;
+    case 4: launch_ln_fwd<4>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream); break;
+    case 6: launch_ln_fwd<6>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream); break;
+    default: launch_ln_fwd<8>(x, gamma, beta, out, out_bf16, M, d, eps, sp_prompt, sp_L, sp_row0, sp_n, sp_pos, stream); break;
   }
   count_launch(1);
   return launch_status("layernorm fwd launch failed");
@@ -146,14 +147,18 @@ static const char* ln_fwd_dispatch(float* x, const float* gamma, const float* be
 const char* layernorm_fwd(const float* x, const float* gamma, const float* beta, void* out, bool out_bf16, int M, int d,
                           float eps, cudaStream_t stream) {
   // (x is only written for spliced rows: none here)
-  return ln_fwd_dispatch(const_cast<float*>(x), gamma, beta, out, out_bf16, M, d, eps, nullptr, 1, 0, 0, stream);
+  return ln_fwd_dispatch(const_cast<float*>(x), gamma, beta, out, out_bf16, M, d, eps, nullptr, 1, 0, 0, nullptr, stream);
 }
 
 const char* layernorm_fwd_splice(float* x, const float* prompt, int L, int row0, int n, const float* gamma, const float* beta,
-                                 void* out, bool out_bf16, int M, int d, float eps, cudaStream_t stream) {
-  if (n <= 0 || prompt == nullptr) return ln_fwd_dispatch(x, gamma, beta, out, out_bf16, M, d, eps, nullptr, 1, 0, 0, stream);
+                                 void* out, bool out_bf16, int M, int d, float eps, cudaStream_t stream, const int* tok_pos) {
+  if (n <= 0 || prompt == nullptr) return ln_fwd_dispatch(x, gamma, beta, out, out_bf16, M, d, eps, nullptr, 1, 0, 0, nullptr, stream);
+  if (tok_pos != nullptr) {
+    if (row0 < 0) return "layernorm + splice: bad geometry";
+    return ln_fwd_dispatch(x, gamma, beta, out, out_bf16, M, d, eps, prompt, 1, row0, n, tok_pos, stream);
+  }
   if (L <= 0 || row0 < 0 || row0 + n > L || M % L != 0) return "layernorm + splice: bad geometry";
-  return ln_fwd_dispatch(x, gamma, beta, out, out_bf16, M, d, eps, prompt, L, row0, n, stream);
+  return ln_fwd_dispatch(x, gamma, beta, out, out_bf16, M, d, eps, prompt, L, row0, n, nullptr, stream);
 }
 
 // Registers holding the residual-gradient piece of a lane: fp32 (float4) or the packed bf16 form (uint2)
@@ -181,13 +186,14 @@ template <> struct ResidRegs<true> {
 // keeps, rowops.cu "fused-LayerNorm plumbing"): 2 B instead of 4 B per element read, exact fp32 mean / rstd.
 // RESID_BF16: the residual gradient is read from the bf16 copy of the stream (it may alias dx_bf16: every lane reads its
 // own elements before it writes them).  win_n >= 0 restricts the fp32 output to the rows of the deep-prompt window,
-// (row % win_L) in [win_row0, win_row0 + win_n) -- the only fp32 rows anyone reads when the gradient stream is kept in
+// (row % win_L, or win_pos[row] for packed variable-length sequences) in [win_row0, win_row0 + win_n) -- the only fp32 rows anyone reads when the gradient stream is kept in
 // bf16 (the splice backward sums them); win_n < 0: every row.  8 instead of 14 B per element on an HBM-bound kernel.
 template <int NV, bool DY_BF16, bool X_STATS, bool RESID_BF16>
 __global__ void __launch_bounds__(256, NV == 4 ? 4 : 1) ln_bwd_kernel(const void* __restrict__ dy, const void* __restrict__ xv,
                                                      const float2* __restrict__ stats, const float* __restrict__ gamma,
                                                      const void* resid, float* dx, bf16* dx_bf16, int M, int d,
-                                                     float eps, int win_L, int win_row0, int win_n) {
+                                                     float eps, int win_L, int win_row0, int win_n,
+                                                     const int* __restrict__ win_pos) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   pdl_wait();
@@ -197,7 +203,7 @@ __global__ void __launch_bounds__(256, NV == 4 ? 4 : 1) ln_bwd_kernel(const void
   const float* x = reinterpret_cast<const float*>(xv);
   bool write_f32 = dx != nullptr;  // (warp-uniform)
   if (win_n >= 0) {
-    const int pos = row % win_L - win_row0;
+    const int pos = (win_pos != nullptr ? win_pos[row] : row % win_L) - win_row0;
     write_f32 = write_f32 && pos >= 0 && pos < win_n;
   }
   float4 v[NV], g[NV];
@@ -299,32 +305,32 @@ __global__ void __launch_bounds__(256, NV == 4 ? 4 : 1) ln_bwd_kernel(const void
 template <int NV, bool RB>
 static void launch_ln_bwd(const void* dy, bool dy_bf16, const void* x, const float2* stats, const float* gamma, const void* resid,
                           float* dx, bf16* dx_bf16, int M, int d, float eps, int win_L, int win_row0, int win_n,
-                          cudaStream_t stream) {
+                          const int* win_pos, cudaStream_t stream) {
   const int wpc = ln_warps();
   const int grid = (M + wpc - 1) / wpc;
   const dim3 blk(32 * wpc);
   if (stats != nullptr) {  // (bf16 dy only: the dgrad GEMM's output)
     launch_pdl(ln_bwd_kernel<NV, true, true, RB>, dim3(grid), blk, 0, stream, dy, x, stats, gamma, resid, dx, dx_bf16, M, d, eps,
-               win_L, win_row0, win_n);
+               win_L, win_row0, win_n, win_pos);
   } else if (dy_bf16) {
     launch_pdl(ln_bwd_kernel<NV, true, false, RB>, dim3(grid), blk, 0, stream, dy, x, stats, gamma, resid, dx, dx_bf16, M, d, eps,
-               win_L, win_row0, win_n);
+               win_L, win_row0, win_n, win_pos);
   } else {
     launch_pdl(ln_bwd_kernel<NV, false, false, RB>, dim3(grid), blk, 0, stream, dy, x, stats, gamma, resid, dx, dx_bf16, M, d, eps,
-               win_L, win_row0, win_n);
+               win_L, win_row0, win_n, win_pos);
   }
 }
 
 template <bool RB>
 static void dispatch_ln_bwd(const void* dy, bool dy_bf16, const void* x, const float2* stats, const float* gamma, const void* resid,
                             float* dx, bf16* dx_bf16, int M, int d, float eps, int win_L, int win_row0, int win_n,
-                            cudaStream_t stream) {
+                            const int* win_pos, cudaStream_t stream) {
   switch (pick_nv(d)) {
-    case 1: launch_ln_bwd<1, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream); break;
-    case 2: launch_ln_bwd<2, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream); break;
-    case 4: launch_ln_bwd<4, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream); break;
-    case 6: launch_ln_bwd<6, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream); break;
-    default: launch_ln_bwd<8, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream); break;
+    case 1: launch_ln_bwd<1, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream); break;
+    case 2: launch_ln_bwd<2, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream); break;
+    case 4: launch_ln_bwd<4, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream); break;
+    case 6: launch_ln_bwd<6, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream); break;
+    default: launch_ln_bwd<8, RB>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream); break;
   }
 }
 
@@ -366,6 +372,7 @@ struct LnPipeArgs {
   int M, d;
   float eps;
   int win_L, win_row0, win_n;
+  const int* win_pos;   // or null: the window position of a row is row % win_L
   int stages;
   unsigned stage_bytes;
 };
@@ -508,7 +515,8 @@ __global__ void __launch_bounds__(256) ln_bwd_pipe_kernel(const LnPipeArgs a) {
       const float k2 = -(rstd * rstd * rstd * (cc * inv_d));  // -rstd^2 * s2 with s2 = mean(g * xhat) = rstd * mean(g (x - mean))
       const float c0 = -rstd * s1;
       // ---- dx = resid + rstd * (g - s1 - xhat * s2) = (resid - rstd * s1) + rstd * g - (x - mean) * rstd^3 * mean(g (x - mean))
-      const bool write_f32 = a.dx != nullptr && (!windowed || (pos >= a.win_row0 && pos < a.win_row0 + a.win_n));
+      const int wp = a.win_pos != nullptr ? a.win_pos[row] : pos;
+      const bool write_f32 = a.dx != nullptr && (!windowed || (wp >= a.win_row0 && wp < a.win_row0 + a.win_n));
       const size_t off = static_cast<size_t>(row) * d + lane * 8u;
 #pragma unroll
       for (int i = 0; i < NP; ++i) {
@@ -557,6 +565,7 @@ struct LnFwdPipeArgs {
   float eps;
   const float* sp_prompt;  // or null
   int sp_L, sp_row0, sp_n;
+  const int* sp_pos;       // or null: the position of a row is row % sp_L
   int stages;
   unsigned stage_bytes;
 };
@@ -631,10 +640,11 @@ __global__ void __launch_bounds__(256) ln_fwd_pipe_kernel(const LnFwdPipeArgs a)
     if (++s == stages) { s = 0; phase ^= 1u; st = stage0; } else { st += a.stage_bytes; }
     if (row < a.M) {  // (warp-uniform)
       const size_t off = static_cast<size_t>(row) * d + lane * 8u;
-      if (splicing && pos >= a.sp_row0 && pos < a.sp_row0 + a.sp_n) {
+      const int sp = a.sp_pos != nullptr ? a.sp_pos[row] : pos;
+      if (splicing && sp >= a.sp_row0 && sp < a.sp_row0 + a.sp_n) {
         // the deep-prompt splice of the block (clip/model.py:281-297): the row takes the prompt's values, copied verbatim
         // into the residual stream (bit-exact), and is normalised like any other
-        const float* src = a.sp_prompt + static_cast<size_t>(pos - a.sp_row0) * d + lane * 8u;
+        const float* src = a.sp_prompt + static_cast<size_t>(sp - a.sp_row0) * d + lane * 8u;
 #pragma unroll
         for (int i = 0; i < NP; ++i) {
           const float4 u0 = *reinterpret_cast<const float4*>(src + i * 256), u1 = *reinterpret_cast<const float4*>(src + i * 256 + 4);
@@ -806,12 +816,12 @@ static const char* launch_ln_fwd_pipe(LnFwdPipeArgs a, cudaStream_t stream) {
 }
 
 static bool ln_fwd_pipe_try(float* x, const float* gamma, const float* beta, bf16* out, int M, int d, float eps, const float* sp_prompt,
-                            int sp_L, int sp_row0, int sp_n, cudaStream_t stream, const char** err) {
+                            int sp_L, int sp_row0, int sp_n, const int* sp_pos, cudaStream_t stream, const char** err) {
   *err = nullptr;
   if (ln_fwd_pipe_mode() <= 0 || d % 256 != 0 || d > 1024 || M < 64) return false;
   LnFwdPipeArgs a;
   a.x = x; a.x_w = x; a.gamma = gamma; a.beta = beta; a.out = out; a.M = M; a.eps = eps;
-  a.sp_prompt = sp_prompt; a.sp_L = sp_L > 0 ? sp_L : 1; a.sp_row0 = sp_row0; a.sp_n = sp_n; a.stages = 0; a.stage_bytes = 0;
+  a.sp_prompt = sp_prompt; a.sp_L = sp_L > 0 ? sp_L : 1; a.sp_row0 = sp_row0; a.sp_n = sp_n; a.sp_pos = sp_pos; a.stages = 0; a.stage_bytes = 0;
   const char* e = d == 256 ? launch_ln_fwd_pipe<1>(a, stream)
                            : d == 512 ? launch_ln_fwd_pipe<2>(a, stream) : d == 768 ? launch_ln_fwd_pipe<3>(a, stream) : launch_ln_fwd_pipe<4>(a, stream);
   if (e == kLnPipeNoFit) return false;
@@ -824,18 +834,19 @@ static bool ln_fwd_pipe_try(float* x, const float* gamma, const float* beta, bf1
 // win_n >= 0: fp32 rows are written inside the deep-prompt window only (see the kernel).
 const char* layernorm_bwd_stream(const void* dy, bool dy_bf16, const void* x, const float2* stats, const float* gamma,
                                  const void* resid, bool resid_bf16, float* dx, bf16* dx_bf16, int M, int d, float eps,
-                                 int win_L, int win_row0, int win_n, cudaStream_t stream) {
+                                 int win_L, int win_row0, int win_n, cudaStream_t stream, const int* win_pos) {
   if (M <= 0) return nullptr;
   if (d % 4 != 0 || d > LN_MAXV * 128) return "layernorm: width must be a multiple of 4 and <= 1024";
   if (stats != nullptr && (!dy_bf16 || d % 64 != 0)) return "layernorm: the bf16-input form needs bf16 dy and width % 64 == 0";
   if (dx == nullptr && dx_bf16 == nullptr) return "layernorm bwd: no output";
-  if (win_n > 0 && (win_L <= 0 || win_row0 < 0 || win_row0 + win_n > win_L)) return "layernorm bwd: bad window";
+  if (win_pos != nullptr) win_L = 1;  // (positions come from win_pos)
+  if (win_n > 0 && win_pos == nullptr && (win_L <= 0 || win_row0 < 0 || win_row0 + win_n > win_L)) return "layernorm bwd: bad window";
   if (win_n >= 0 && win_L <= 0) win_L = 1;
   // bf16 dy, width a multiple of 256 (one 8-column piece per lane and 256 columns: 512 / 768 / 1024, the widths of the CLIP towers)
   if (ln_bwd_pipe_mode() > 0 && dy_bf16 && d % 256 == 0 && M >= 64) {
     LnPipeArgs a;
     a.dy = reinterpret_cast<const bf16*>(dy); a.x = x; a.stats = stats; a.gamma = gamma; a.resid = resid; a.dx = dx; a.dx_bf16 = dx_bf16;
-    a.M = M; a.d = d; a.eps = eps; a.win_L = win_L; a.win_row0 = win_row0; a.win_n = win_n; a.stages = 0; a.stage_bytes = 0;
+    a.M = M; a.d = d; a.eps = eps; a.win_L = win_L; a.win_row0 = win_row0; a.win_n = win_n; a.win_pos = win_pos; a.stages = 0; a.stage_bytes = 0;
     const int rk = resid == nullptr ? 0 : (resid_bf16 ? 1 : 2);
     const char* e = dispatch_ln_pipe(a, stats != nullptr, rk, stream);
     if (e == nullptr) {
@@ -845,9 +856,9 @@ const char* layernorm_bwd_stream(const void* dy, bool dy_bf16, const void* x, co
     if (e != kLnPipeNoFit) return e;
   }
   if (resid_bf16 && resid != nullptr)
-    dispatch_ln_bwd<true>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream);
+    dispatch_ln_bwd<true>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream);
   else
-    dispatch_ln_bwd<false>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, stream);
+    dispatch_ln_bwd<false>(dy, dy_bf16, x, stats, gamma, resid, dx, dx_bf16, M, d, eps, win_L, win_row0, win_n, win_pos, stream);
   count_launch(1);
   return launch_status("layernorm bwd launch failed");
 }
@@ -877,7 +888,7 @@ const char* splice_fwd(float* x, const float* prompt, int S, int L, int row0, in
   return launch_status("splice fwd launch failed");
 }
 
-// dprompt[r, :] = sum_s dx[s, row0 + r, :]; optionally the rows of dx (fp32 and bf16 copy) are
+// dprompt[r, :] = sum_s dx[s, row0 + r, :] (packed variable-length sequences: row seq_off[s] + row0 + r); optionally the rows of dx (fp32 and bf16 copy) are
 // then zeroed (the overwritten activations receive no gradient, SURVEY.md 3.3).
 // Deterministic two-stage reduction: stage 1 sums a fixed slice of the sequences per block
 // (fixed partition over 8 warps, fixed-order smem reduction) into partial[slice][r][:],
@@ -886,7 +897,8 @@ static constexpr int SPLICE_MAX_SLICES = 64;
 
 __global__ void __launch_bounds__(256) splice_bwd_partial_kernel(float* __restrict__ dx, bf16* __restrict__ dx_bf16,
                                                                  float* __restrict__ partial, int S, int L, int row0,
-                                                                 int n, int d, int per_slice, int zero_rows) {
+                                                                 int n, int d, int per_slice, int zero_rows,
+                                                                 const int* __restrict__ seq_off) {
   __shared__ float4 part[8][32];
   const int r = blockIdx.x, slice = blockIdx.z;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -897,7 +909,7 @@ __global__ void __launch_bounds__(256) splice_bwd_partial_kernel(float* __restri
   pdl_trigger();
   if (c < d) {
     for (int s = slice * per_slice + warp; s < s_end; s += 8) {
-      const size_t off = (static_cast<size_t>(s) * L + row0 + r) * d + c;
+      const size_t off = ((seq_off != nullptr ? static_cast<size_t>(seq_off[s]) : static_cast<size_t>(s) * L) + row0 + r) * d + c;
       const float4 v = *reinterpret_cast<const float4*>(dx + off);
       acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
       if (zero_rows) {
@@ -923,7 +935,7 @@ __global__ void __launch_bounds__(256) splice_bwd_partial_kernel(float* __restri
 __global__ void __launch_bounds__(256) splice_bwd_fused_kernel(float* __restrict__ dx, bf16* __restrict__ dx_bf16,
                                                                float* __restrict__ partial, float* __restrict__ dprompt,
                                                                unsigned* __restrict__ ticket, int S, int L, int row0, int n, int d,
-                                                               int per_slice, int zero_rows) {
+                                                               int per_slice, int zero_rows, const int* __restrict__ seq_off) {
   __shared__ float4 part[8][32];
   __shared__ unsigned s_last;
   const int r = blockIdx.x, slice = blockIdx.z, nslices = gridDim.z;
@@ -935,7 +947,7 @@ __global__ void __launch_bounds__(256) splice_bwd_fused_kernel(float* __restrict
   pdl_trigger();
   if (c < d) {
     for (int s = slice * per_slice + warp; s < s_end; s += 8) {
-      const size_t off = (static_cast<size_t>(s) * L + row0 + r) * d + c;
+      const size_t off = ((seq_off != nullptr ? static_cast<size_t>(seq_off[s]) : static_cast<size_t>(s) * L) + row0 + r) * d + c;
       const float4 v = *reinterpret_cast<const float4*>(dx + off);
       acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
       if (zero_rows) {
@@ -991,9 +1003,9 @@ static size_t splice_ticket_slots(int n, int d) { return static_cast<size_t>(n) 
 size_t splice_bwd_workspace_floats(int n, int d) { return static_cast<size_t>(SPLICE_MAX_SLICES) * n * d + splice_ticket_slots(n, d); }
 
 const char* splice_bwd(float* dx, bf16* dx_bf16, float* dprompt, float* workspace, int S, int L, int row0, int n, int d,
-                       bool zero_rows, cudaStream_t stream) {
+                       bool zero_rows, cudaStream_t stream, const int* seq_off) {
   if (n <= 0) return nullptr;
-  if (d % 4 != 0 || row0 < 0 || row0 + n > L) return "splice: bad geometry";
+  if (d % 4 != 0 || row0 < 0 || (seq_off == nullptr && row0 + n > L)) return "splice: bad geometry";
   int nslices = (S + 15) / 16;  // >= 16 sequences per block
   if (nslices > SPLICE_MAX_SLICES) nslices = SPLICE_MAX_SLICES;
   if (nslices < 1) nslices = 1;
@@ -1001,7 +1013,7 @@ const char* splice_bwd(float* dx, bf16* dx_bf16, float* dprompt, float* workspac
   // the tickets live behind the partials and must be zero before the first launch (the owner of the workspace zeroes it once)
   unsigned* ticket = reinterpret_cast<unsigned*>(workspace + static_cast<size_t>(SPLICE_MAX_SLICES) * n * d);
   launch_pdl(splice_bwd_fused_kernel, dim3(n, (d + 127) / 128, nslices), dim3(256), 0, stream, dx, dx_bf16, workspace, dprompt, ticket,
-             S, L, row0, n, d, per_slice, zero_rows ? 1 : 0);
+             S, L, row0, n, d, per_slice, zero_rows ? 1 : 0, seq_off);
   count_launch(1);
   return launch_status("splice bwd launch failed");
 }
@@ -1245,18 +1257,40 @@ const char* write_cls_rows(float* x, const float* cls, const float* pos, int S, 
 
 // x0[c, l, :] = emb[c, l, :] + pos[l, :] for l < L (L <= Lsrc): text-tower input, built once
 // per class set (trainers/mudpt.py:143); the ctx rows are overwritten by the splice each step.
+// seq_off != null: packed variable-length sequences, row seq_off[c] + l for l < seq_off[c+1] - seq_off[c] (L = the longest).
 __global__ void add_pos_kernel(float* __restrict__ x0, const float* __restrict__ emb, const float* __restrict__ pos,
-                               int L, int Lsrc, int d) {
+                               int L, int Lsrc, int d, const int* __restrict__ seq_off) {
   const int c = blockIdx.x, l = blockIdx.y;
+  if (seq_off != nullptr && l >= seq_off[c + 1] - seq_off[c]) return;
   const float* src = emb + (static_cast<size_t>(c) * Lsrc + l) * d;
-  float* dst = x0 + (static_cast<size_t>(c) * L + l) * d;
+  float* dst = x0 + ((seq_off != nullptr ? static_cast<size_t>(seq_off[c]) : static_cast<size_t>(c) * L) + l) * d;
   for (int i = threadIdx.x; i < d; i += blockDim.x) dst[i] = src[i] + pos[static_cast<size_t>(l) * d + i];
 }
-const char* add_positional(float* x0, const float* emb, const float* pos, int S, int L, int Lsrc, int d, cudaStream_t stream) {
+const char* add_positional(float* x0, const float* emb, const float* pos, int S, int L, int Lsrc, int d, cudaStream_t stream,
+                           const int* seq_off) {
   if (S <= 0) return nullptr;
-  add_pos_kernel<<<dim3(S, L), 128, 0, stream>>>(x0, emb, pos, L, Lsrc, d);
+  add_pos_kernel<<<dim3(S, L), 128, 0, stream>>>(x0, emb, pos, L, Lsrc, d, seq_off);
   count_launch(1);
   return launch_status("add_pos launch failed");
+}
+
+// out[s, l, :] = x[seq_off[s] + l, :] for l < len_s, 0 for len_s <= l < L: packed variable-length rows to the padded
+// [S, L, d] layout (the dense input gradient of a ragged text tower; zero past each length is exact under the causal mask)
+__global__ void unpack_rows_kernel(const float* __restrict__ x, const int* __restrict__ seq_off, int L, int d, float* __restrict__ out) {
+  const int s = blockIdx.x, l = blockIdx.y;
+  pdl_wait();
+  pdl_trigger();
+  const int r0 = seq_off[s], len = seq_off[s + 1] - r0;
+  float4* dst = reinterpret_cast<float4*>(out + (static_cast<size_t>(s) * L + l) * d);
+  const float4* src = reinterpret_cast<const float4*>(x + static_cast<size_t>(r0 + l) * d);
+  for (int c = threadIdx.x; c < d / 4; c += blockDim.x) dst[c] = l < len ? src[c] : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+const char* unpack_rows(const float* x, const int* seq_off, int S, int L, int d, float* out, cudaStream_t stream) {
+  if (S <= 0 || L <= 0) return nullptr;
+  if (d % 4 != 0) return "unpack_rows: width must be a multiple of 4";
+  launch_pdl(unpack_rows_kernel, dim3(S, L), dim3(128), 0, stream, x, seq_off, L, d, out);
+  count_launch(1);
+  return launch_status("unpack_rows launch failed");
 }
 
 __global__ void cast_bf16_kernel(const float* __restrict__ in, bf16* __restrict__ out, size_t n) {

@@ -8,11 +8,34 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, Optional
+from typing import Dict, List, Optional, Tuple
 
 import torch
 
 from . import _lib
+
+
+def text_lengths(eot: torch.Tensor, mode, full_len: int, min_len: int) -> Tuple[int, Optional[List[int]]]:
+    """Token counts the text tower runs for classes whose EOT tokens sit at positions `eot` [C].
+
+    mode True: one length for all classes, max(eot) + 1; False: all `full_len` positions; "per_class": class c runs
+    max(eot_c + 1, min_len) tokens (a ragged tower).  Every length is at least `min_len` (SOT + the n_ctx prompt rows).
+    Dropping the tokens after EOT is exact under the causal mask.  Returns (padded length, per-class lengths or None)."""
+    if mode == "per_class":
+        lengths = [max(int(e) + 1, min_len) for e in eot.tolist()]
+        return max(lengths), lengths
+    if mode is not True and mode is not False:
+        raise ValueError(f"mudpt_b200: text truncation mode must be True, False or 'per_class', not {mode!r}")
+    seq_len = int(eot.max()) + 1 if mode else int(full_len)
+    return max(seq_len, min_len), None
+
+
+def packed_offsets(lengths: List[int]) -> List[int]:
+    """Row offsets [C + 1] of the packed ragged layout: class c occupies rows [off[c], off[c + 1])."""
+    off = [0]
+    for n in lengths:
+        off.append(off[-1] + int(n))
+    return off
 
 
 class Engine:
@@ -102,13 +125,23 @@ class Engine:
                                                   _lib.stream_ptr(self.device)), self.h)
         return dP
 
-    def text_set_classes(self, embeddings: torch.Tensor, eot: torch.Tensor, seq_len: int) -> None:
-        """embeddings [C, src_len, width] fp32; eot [C] int (position of the EOT token)."""
+    def text_set_classes(self, embeddings: torch.Tensor, eot: torch.Tensor, seq_len: int,
+                         lengths: Optional[List[int]] = None) -> None:
+        """embeddings [C, src_len, width] fp32; eot [C] int (position of the EOT token).  With `lengths` [C] the tower is
+        ragged: class c runs its first lengths[c] tokens (packed rows, see text_lengths) and seq_len is ignored."""
         embeddings = embeddings.to(device=self.device, dtype=torch.float32).contiguous()
         Cn, src_len, _ = embeddings.shape
         eot_host = (C.c_int32 * Cn)(*[int(v) for v in eot.tolist()])
-        _lib.check(self.lib.mudpt_text_set_classes(self.h, embeddings.data_ptr(), Cn, src_len, int(seq_len), eot_host,
-                                                   _lib.stream_ptr(self.device)), self.h)
+        if lengths is None:
+            _lib.check(self.lib.mudpt_text_set_classes(self.h, embeddings.data_ptr(), Cn, src_len, int(seq_len), eot_host,
+                                                       _lib.stream_ptr(self.device)), self.h)
+        else:
+            if len(lengths) != Cn:
+                raise ValueError(f"mudpt_b200: {len(lengths)} lengths for {Cn} classes")
+            len_host = (C.c_int32 * Cn)(*[int(v) for v in lengths])
+            _lib.check(self.lib.mudpt_text_set_classes_ragged(self.h, embeddings.data_ptr(), Cn, src_len, len_host, eot_host,
+                                                              _lib.stream_ptr(self.device)), self.h)
+            seq_len = max(int(v) for v in lengths)
         torch.cuda.current_stream(self.device).synchronize()
         self.n_classes, self.text_len = Cn, int(seq_len)
         self.class_key = None
@@ -335,8 +368,11 @@ class TextTowerDenseFn(torch.autograd.Function):
     prompt embeddings [C, L, width] in, dense gradient out."""
 
     @staticmethod
-    def forward(ctx, engine: Engine, prompts_full, eot, deep_prompts, seq_len):
-        engine.text_set_classes(prompts_full.detach(), eot, seq_len)
+    def forward(ctx, engine: Engine, prompts_full, eot, deep_prompts, seq_len, lengths=None):
+        if lengths is None:  # (engine stand-ins without the ragged form take three arguments)
+            engine.text_set_classes(prompts_full.detach(), eot, seq_len)
+        else:
+            engine.text_set_classes(prompts_full.detach(), eot, seq_len, lengths)
         w = engine.arch["transformer_width"]
         P = torch.zeros(engine.depth, engine.n_ctx, w, device=engine.device, dtype=torch.float32)
         if engine.depth > 1:
@@ -354,7 +390,7 @@ class TextTowerDenseFn(torch.autograd.Function):
         dP, dx0 = e.text_backward(d_out, True)
         d_full = torch.zeros(dx0.shape[0], ctx.full_len, dx0.shape[2], device=dx0.device, dtype=dx0.dtype)
         d_full[:, :dx0.shape[1]] = dx0  # positions past seq_len are dead under the causal mask
-        return None, d_full, None, dP[1:], None
+        return None, d_full, None, dP[1:], None, None
 
 
 class LogitsFn(torch.autograd.Function):

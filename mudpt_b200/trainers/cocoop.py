@@ -24,7 +24,7 @@ import torch
 from torch import nn
 
 from .. import clip
-from ..engine import TextTowerDenseFn
+from ..engine import TextTowerDenseFn, text_lengths
 from .mudpt import (TRAINER_REGISTRY, TrainerX, apply_freeze_rule, build_lr_scheduler, build_optimizer, load_pretrained_weights,
                     restore_checkpoints)
 
@@ -55,15 +55,15 @@ class TextEncoder(nn.Module):
             setattr(self, member, getattr(clip_model, member))
         self.dtype = clip_model.dtype
         object.__setattr__(self, "_clip_ref", [clip_model])
-        self.truncate_to_eot = True
+        self.truncate_to_eot = True  # True / False / "per_class" (see engine.text_lengths)
 
     def forward(self, prompts, tokenized_prompts):
         """prompts [N, 77, d] (N = C, or B*C batched), tokenized_prompts [N, 77] -> text features [N, e]."""
         engine = self._clip_ref[0].engine(prompts.device)
         eot = tokenized_prompts.argmax(dim=-1).cpu()
-        seq_len = int(eot.max()) + 1 if self.truncate_to_eot else prompts.shape[1]
+        seq_len, lengths = text_lengths(eot, self.truncate_to_eot, prompts.shape[1], 1 + engine.n_ctx)
         deep = torch.zeros(0, 0, prompts.shape[-1], device=prompts.device)
-        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep, seq_len)
+        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep, seq_len, lengths)
 
 
 class PromptLearner(nn.Module):

@@ -27,7 +27,7 @@ import torch.nn.functional as F
 
 from .. import clip
 from .. import dist as mdist
-from ..engine import prompt_algebra_forward, prompt_algebra_backward, LogitsFn, PromptAlgebraFn, TextTowerDenseFn, TextTowerFn, VisionTowerFn
+from ..engine import prompt_algebra_forward, prompt_algebra_backward, text_lengths, LogitsFn, PromptAlgebraFn, TextTowerDenseFn, TextTowerFn, VisionTowerFn
 
 try:  # the Dassl engine is not in the reference tree nor in this image (SURVEY.md section 2 row 13)
     from dassl.engine import TRAINER_REGISTRY, TrainerX
@@ -246,15 +246,14 @@ class TextEncoder(nn.Module):
         self.dtype = clip_model.dtype
         # strong reference that is NOT a registered submodule (state-dict keys must match the reference)
         object.__setattr__(self, "_clip_ref", [clip_model])
-        self.truncate_to_eot = True
+        self.truncate_to_eot = True  # True / False / "per_class" (see engine.text_lengths)
 
     def forward(self, prompts, tokenized_prompts, deep_prompts):
         """Reference API (trainers/mudpt.py:142-156): prompts [C, 77, d] -> text features [C, e]."""
         engine = self._clip_ref[0].engine(prompts.device)
         eot = tokenized_prompts.argmax(dim=-1).cpu()
-        seq_len = int(eot.max()) + 1 if self.truncate_to_eot else prompts.shape[1]
-        seq_len = max(seq_len, 1 + engine.n_ctx)
-        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep_prompts.float(), seq_len)
+        seq_len, lengths = text_lengths(eot, self.truncate_to_eot, prompts.shape[1], 1 + engine.n_ctx)
+        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep_prompts.float(), seq_len, lengths)
 
 
 class CustomCLIP(nn.Module):
@@ -269,7 +268,8 @@ class CustomCLIP(nn.Module):
         self.deep_prompts_depth = self.mudpt_prompt_learner.deep_prompts_depth
         # strong reference that is NOT a registered submodule (state-dict keys must match the reference)
         object.__setattr__(self, "_clip_ref", [clip_model])
-        # exact under the causal mask (SURVEY.md 8c-i); set False to run all 77 positions
+        # exact under the causal mask (SURVEY.md 8c-i); set False to run all 77 positions, "per_class" to run every class
+        # at its own length (packed rows: no class pays for the longest one; see engine.text_lengths)
         self.truncate_text_to_eot = os.environ.get("MUDPT_TEXT_FULL_LENGTH", "0") != "1"
         self.shard_classes = True           # class-sharded text tower when torch.distributed is initialised
         self._cached_text_features = None   # eval-time cache (parameters frozen under no_grad)
@@ -304,16 +304,20 @@ class CustomCLIP(nn.Module):
             self._replicas_synced = True
         lo, hi = self._class_range()
         eot_all = self.tokenized_prompts.argmax(dim=-1)
-        # one global length so that every rank runs the same shapes
-        seq_len = int(eot_all.max()) + 1 if self.truncate_text_to_eot else self.tokenized_prompts.shape[1]
-        seq_len = max(seq_len, 1 + pl.n_ctx)
+        mode = self.truncate_text_to_eot
+        # padded: one global length so that every rank runs the same shapes; "per_class": each shard packs its own classes
+        seq_len, lengths = text_lengths(eot_all[lo:hi] if mode == "per_class" else eot_all, mode, self.tokenized_prompts.shape[1],
+                                        1 + pl.n_ctx)
         eng = self._engine(device)
-        key = (id(self), lo, hi, seq_len)
+        key = (id(self), lo, hi, seq_len, mode)
         if eng.class_key == key:
             return
         prefix, suffix = pl.token_prefix[lo:hi], pl.token_suffix[lo:hi]
         emb = torch.cat([prefix, torch.zeros(hi - lo, pl.n_ctx, pl.ctx_dim, device=prefix.device, dtype=prefix.dtype), suffix], dim=1)
-        eng.text_set_classes(emb.float(), eot_all[lo:hi], seq_len)
+        if lengths is None:  # (engine stand-ins without the ragged form take three arguments)
+            eng.text_set_classes(emb.float(), eot_all[lo:hi], seq_len)
+        else:
+            eng.text_set_classes(emb.float(), eot_all[lo:hi], seq_len, lengths)
         eng.class_key = key
 
     def _native_prompt_args(self):
