@@ -123,6 +123,25 @@ int mudpt_text_forward(mudpt_handle* h, const float* prompts, int32_t splice_lay
  * [C, max(len_host), width] with zeros at positions >= len_c (exact: those tokens do not reach any output). */
 int mudpt_text_backward(mudpt_handle* h, const float* d_f_txt, float* d_prompts, float* d_x0, void* stream);
 
+/* ---- forward-only towers (evaluation, frozen towers) ---------------------------------------------
+ * The same arguments and results as mudpt_vision_forward / mudpt_text_forward (the text tower runs over the registered
+ * class set), for a result nothing will differentiate:
+ *   - f_img / f_txt are bitwise equal to those of the training forward on the same inputs (same kernel sequence; the
+ *     c_fc GEMMs write QuickGELU(h) only instead of h and QuickGELU(h));
+ *   - the walk runs in an inference workspace of its own (a few buffers every layer shares, about 26 * width bytes per
+ *     token row, DESIGN.md section 3), allocated at the first call; nothing a pending mudpt_*_backward reads is touched,
+ *     so a training forward, an infer call (any batch size, any prompts) and the backward give the gradients of the
+ *     forward alone;
+ *   - stream ordering as for the other tower calls: the training and the inference workspaces are disjoint, so a
+ *     training walk and an infer call may also run on two streams at once;
+ *   - CUDA-graph capturable after the first (allocating) call with the largest shape. */
+int mudpt_vision_infer(mudpt_handle* h, const float* images, int32_t B, const float* prompts, float* f_img, void* stream);
+int mudpt_text_infer(mudpt_handle* h, const float* prompts, int32_t splice_layer0, float* f_txt, void* stream);
+/* Device bytes the handle holds for `tower` (MUDPT_TOWER_*): kind 0 = training workspace (allocated at the first
+ * mudpt_*_forward), 1 = inference workspace (first mudpt_*_infer), 2 = tower input (class set / vision stem output).
+ * Requested sizes: each allocation carries 256 B of slack besides. */
+int mudpt_workspace_bytes(mudpt_handle* h, int32_t tower, int32_t kind, int64_t* bytes);
+
 /* ---- logits + loss head (trainers/mudpt.py:178-182, :250) ---------------------------------------
  * labels int64 [B] or NULL (logits only).  loss (1 float) = sum_b CE_b * inv_global_batch,
  * d_f_img [B,e] / d_f_txt [C,e] = gradients of that loss (NULL to skip). */
@@ -179,6 +198,8 @@ int mudpt_gemm_bf16(const uint16_t* A, const uint16_t* B, int32_t M, int32_t N, 
  *   10 f32 = resid + rstd*(acc - c1 - xhat*c2) (+ bf16 copy): LayerNorm dgrad in the dgrad GEMM's epilogue,
  *      c1 = sum_p dots[row,p].x / ln_width, c2 = sum_p dots[row,p].y / ln_width, xhat from x2 and ln_stats
  *   11 mode 4 + dots_out[row, col/span] = (sum dh*colsum, sum dh*(h - bias')) with sb = interleaved (colsum, bias')
+ *   12 out0 = QuickGELU(acc + bias): out1 of mode 3 alone (bitwise), one output stream   c_fc of a forward-only walk
+ *   13 out0 = QuickGELU(rstd*(acc - mean*colsum) + bias): out1 of mode 8 alone (bitwise)
  * stream_k: 0 = whole tiles only, 1 = cut the tail wave into k-block ranges whenever possible, -1 = cost model. */
 typedef struct mudpt_gemm_epilogue {
   int32_t mode, ldc;

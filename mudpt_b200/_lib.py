@@ -33,6 +33,9 @@ SIGNATURES = {
     "mudpt_text_set_classes_ragged": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mudpt_text_forward": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, C.c_void_p]),
     "mudpt_text_backward": (C.c_int, [C.c_void_p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "mudpt_vision_infer": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, c_f32p, C.c_void_p]),
+    "mudpt_text_infer": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, C.c_void_p]),
+    "mudpt_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "mudpt_logits_head": (C.c_int, [C.c_void_p, c_f32p, c_f32p, C.c_void_p, C.c_int32, C.c_int32, C.c_float,
                                     c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_logits_backward": (C.c_int, [C.c_void_p, c_f32p, c_f32p, c_f32p, C.c_int32, C.c_int32, c_f32p, c_f32p, C.c_void_p]),

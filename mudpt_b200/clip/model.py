@@ -24,7 +24,7 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
-from ..engine import Engine, VisionTowerFn
+from ..engine import Engine, vision_tower
 
 
 def _cfg_get(cfg, key: str):
@@ -135,7 +135,7 @@ class VisionTransformer_MuDPT(nn.Module):
     def forward(self, x: torch.Tensor, shared_prompt, t2v_visual_prompts):
         engine = self._owner().engine(x.device)
         text_prompts = self.visual_ctx_deep_projections(self.visual_ctx_deep_prompts)   # v2t, clip/model.py:539
-        feats = VisionTowerFn.apply(engine, x, self.prompt_stack(shared_prompt, t2v_visual_prompts))
+        feats = vision_tower(engine, x, self.prompt_stack(shared_prompt, t2v_visual_prompts))
         return feats, text_prompts
 
 
@@ -195,7 +195,7 @@ class VisionTransformer_UMuDPT(nn.Module):
 
     def forward(self, x: torch.Tensor, shared_ctx, deeper_prompts):
         engine = self._owner().engine(x.device)
-        return VisionTowerFn.apply(engine, x, _stack_with_ln_pre(self, shared_ctx, deeper_prompts))
+        return vision_tower(engine, x, _stack_with_ln_pre(self, shared_ctx, deeper_prompts))
 
 
 class VisionTransformer_UUMuDPT(nn.Module):
@@ -232,7 +232,7 @@ class VisionTransformer_UUMuDPT(nn.Module):
         engine = self._owner().engine(x.device)
         shared = shared_ctx + self.visual_ctx.unsqueeze(0)
         deeper = deeper_prompts + self.visual_ctx_deep_prompts
-        feats = VisionTowerFn.apply(engine, x, _stack_with_ln_pre(self, shared, deeper))
+        feats = vision_tower(engine, x, _stack_with_ln_pre(self, shared, deeper))
         return feats, self.textual_prompts()
 
 
@@ -259,7 +259,7 @@ class VisionTransformer(nn.Module):
         engine = self._owner().engine(x.device)
         empty = torch.zeros(engine.depth, 0, self.conv1.weight.shape[0], device=x.device, dtype=torch.float32)
         with torch.no_grad():  # the tower is frozen and carries no prompts: nothing to differentiate
-            return engine.vision_forward(x, empty)
+            return vision_tower(engine, x, empty)
 
 
 class CLIP(nn.Module):

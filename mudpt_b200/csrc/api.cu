@@ -48,6 +48,33 @@ struct Layer {
   int have = 0;  // bit per tensor
 };
 
+// Device memory of one kind (tower input, training workspace, inference workspace): allocated together and released
+// together when the tower outgrows it.
+struct AllocGroup {
+  std::vector<void*> ptrs;
+  size_t bytes = 0;  // requested bytes (mudpt_workspace_bytes; each cudaMalloc adds 256 B of slack)
+};
+
+// The buffers one forward walk of a tower writes (tower_forward).  The training view gives every layer its own
+// activations, which the backward reads; the inference view (Tower::inf) aliases the same few buffers in every layer.
+struct FwdView {
+  int S = 0, rows = 0;  // sequences and token rows of the walk (the row layout is the tower's)
+  double attn_sq = 0;   // sum over sequences of length^2
+  std::vector<float*> x_in, x_mid;  // [layers + 1], [layers]
+  std::vector<bf16*> xb_in, xb_mid;  // fused LayerNorm: bf16 copies of x_in / x_mid ...
+  std::vector<float2*> st_in, st_mid;  // ... and their per-64-column partial statistics
+  std::vector<bf16*> qkv, o, h;  // h empty: c_fc writes QuickGELU(h) only (EPI_GELU_ONLY / EPI_LN_GELU_ONLY)
+  std::vector<float*> lse;
+  bf16 *a_buf = nullptr, *g_buf = nullptr;
+  // pruned last block: S gathered rows
+  float *pr_x = nullptr, *pr_xm = nullptr, *pr_xo = nullptr;
+  bf16 *pr_o = nullptr, *pr_xmb = nullptr, *pr_h = nullptr, *pr_g = nullptr, *pr_a = nullptr;
+  float2* pr_stm = nullptr;
+  float* head_ws = nullptr;
+  GemmWorkspace* gws = nullptr;
+  bool fused = false, pruned = false;  // set by the walk: the formulation it ran
+};
+
 struct Tower {
   int d = 0, H = 0, layers = 0, n_ctx = 0, row0 = 0, depth = 0;
   bool causal = false;
@@ -55,16 +82,23 @@ struct Tower {
   int S = 0;        // current sequences
   int rows = 0;     // token rows: S * L, or (ragged) the sum of the sequence lengths
   double attn_sq = 0;  // sum over sequences of length^2 (attention FLOP counts)
+  size_t stem_per_seq = 0;  // vision: bf16 elements of one image's extracted patches (np * Kp); text: 0
   // Ragged text tower (mudpt_text_set_classes_ragged): sequence s occupies the packed rows [seq_off[s], seq_off[s + 1]),
   // tok_pos[row] = the row's position in its sequence; sel_rows / p0_rows hold absolute rows (row stride row_L() = 0).
   // The LayerNorms run stand-alone (the fused GEMM epilogues locate prompt rows with row % L).
   bool ragged = false;
   int *seq_off = nullptr, *tok_pos = nullptr;
-  size_t off_cap = 0, pos_cap = 0;
+  int* eot = nullptr;  // text: absolute EOT row of every class
   int row_L() const { return ragged ? 0 : L; }
   const int* packed_pos() const { return ragged ? tok_pos : nullptr; }  // (the arrays outlive a switch back to padded)
   const int* packed_off() const { return ragged ? seq_off : nullptr; }
-  size_t cap_rows = 0;
+  // tower input (x_in[0], xb_in[0], st_in[0], p0_rows; text: seq_off, tok_pos, eot): mudpt_text_set_classes* or the
+  // vision stem writes it, the training walk reads it (and splices its layer-0 prompt rows into it), so does the backward
+  AllocGroup in_mem;
+  size_t in_rows = 0, in_S = 0;
+  // training workspace (everything else above and below): allocated at the first mudpt_*_forward
+  AllocGroup train_mem;
+  size_t cap_rows = 0, cap_S = 0;
   std::vector<Layer> lw;
   bool fold_dirty = true;  // a tensor that enters the LayerNorm folding changed since the last fold
   // saved activations, per layer
@@ -79,12 +113,10 @@ struct Tower {
   // transients
   bf16 *a_buf = nullptr, *g_buf = nullptr, *dh_buf = nullptr, *do_buf = nullptr, *dqkv_buf = nullptr, *dx_bf16 = nullptr;
   float *dx = nullptr, *dsum = nullptr, *splice_ws = nullptr, *head_ws = nullptr;  // head_ws: feature_head_workspace_floats(S, d, e)
-  size_t head_cap = 0;  // floats in head_ws (sized by the sequence count, which may grow while rows = S * L shrinks)
+  bf16* patches = nullptr;  // vision stem: [S, np, Kp]
   // exact work skipping (SURVEY.md H5): after the last block's attention only one row per sequence is consumed
   // (CLS, clip/model.py:548; EOT, trainers/mudpt.py:154), so its out-proj / MLP run on S gathered rows
   const int* sel_rows = nullptr;  // consumed row per sequence (null: row 0)
-  size_t pr_cap = 0;              // sequences the buffers below hold
-  std::vector<void*> pr_allocs;
   bf16 *pr_o = nullptr, *pr_xmb = nullptr, *pr_h = nullptr, *pr_g = nullptr, *pr_a = nullptr, *pr_dxb = nullptr, *pr_dh = nullptr,
        *pr_do = nullptr;
   float *pr_x = nullptr, *pr_xm = nullptr, *pr_xo = nullptr, *pr_dx = nullptr;
@@ -95,15 +127,21 @@ struct Tower {
   // the S * n_ctx gathered prompt rows
   int* p0_rows = nullptr;  // absolute row of prompt token j of sequence s: s * L + row0 + j
   int p0_S = 0, p0_L = 0;  // shape p0_rows was built for
-  size_t p0_cap = 0;       // rows the buffers below hold
-  std::vector<void*> p0_allocs;
   bf16 *p0_dqkv = nullptr, *p0_a = nullptr, *p0_dxb = nullptr;
   float *p0_x = nullptr, *p0_dx = nullptr;
-  std::vector<void*> ws_allocs;  // everything sized by cap_rows: released when the tower outgrows it
   GemmWorkspace gws;             // stream-K scratch of this tower's stream
   bool fwd_done = false;
   bool fwd_fused = false;  // the saved activations belong to the fused-LayerNorm formulation
   int first_splice = 0;  // 0: layer 0 splices prompts[0]; 1: layer-0 rows kept as given
+  // forward-only walk (mudpt_*_infer): a workspace of its own, so that it touches nothing the backward reads
+  struct Infer {
+    AllocGroup mem;
+    size_t rows = 0, S = 0;
+    bool fused = false;  // holds the bf16 copies + statistics of the fused LayerNorm
+    FwdView v;
+    GemmWorkspace gws;
+    bf16* patches = nullptr;
+  } inf;
 };
 
 }  // namespace
@@ -136,10 +174,6 @@ struct mudpt_handle {
   float *pos_t = nullptr, *ln_final_g = nullptr, *ln_final_b = nullptr, *proj_t = nullptr;
   float logit_scale_exp = 0.f;
   int stem_have = 0;
-  bf16* patches = nullptr;
-  size_t patches_cap = 0;
-  int* eot = nullptr;
-  size_t eot_cap = 0;
   float* head_ws = nullptr;
   size_t head_ws_cap = 0;
   std::vector<void*> allocs;
@@ -147,7 +181,7 @@ struct mudpt_handle {
   // options (mudpt_set_option): LayerNorm folded into the GEMMs (default) or the stand-alone LN kernels -- the
   // fallback for checkpoints whose residual stream has a row mean far above its spread (bf16(x) instead of
   // bf16(LN(x)) as the GEMM operand would lose the signal there)
-  int ln_fused = -1;  // -1 = by tower size (see tower_forward), 0 = never, 1 = always
+  int ln_fused = -1;  // -1 = by tower size (see ln_fused_for), 0 = never, 1 = always
   // LayerNorm dgrad in the dgrad GEMMs' epilogues (EPI_LN_BWD) instead of the stand-alone kernel.  Off by default:
   // measured on B200 the row dots it needs cost more at their producers (GELU' epilogue +66 us, attention backward
   // +82 us per block at the cfg-2 shapes) than the fused epilogue saves (60 us): profiles/r02_ln_fusion_ab.txt
@@ -199,13 +233,26 @@ int fail(mudpt_handle* h, const char* fmt, ...) {
   } while (0)
 
 template <typename T>
-cudaError_t dev_alloc(mudpt_handle* h, T** p, size_t n, std::vector<void*>* group = nullptr) {
+cudaError_t dev_alloc(mudpt_handle* h, T** p, size_t n, AllocGroup* group = nullptr) {
   void* q = nullptr;
   cudaError_t c = cudaMalloc(&q, n * sizeof(T) + 256);
   if (c != cudaSuccess) return c;
-  (group ? *group : h->allocs).push_back(q);
+  if (group) {
+    group->ptrs.push_back(q);
+    group->bytes += n * sizeof(T);
+  } else {
+    h->allocs.push_back(q);
+  }
   *p = reinterpret_cast<T*>(q);
   return cudaSuccess;
+}
+
+// (cudaFree waits for the device, so nothing in flight still uses the released buffers)
+void release(AllocGroup& g) {
+  for (void* p : g.ptrs) cudaFree(p);
+  g.ptrs.clear();
+  g.bytes = 0;
+  gemm_clear_tensor_map_cache();
 }
 
 bool env_flag(const char* name, bool dflt) {
@@ -213,9 +260,20 @@ bool env_flag(const char* name, bool dflt) {
   return e ? atoi(e) != 0 : dflt;
 }
 
-// (re)allocate the activation workspace of a tower for S sequences of L tokens, or (off != null: host row offsets [S+1])
-// for S packed sequences of at most L tokens
-int ensure_tower(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullptr) {
+// Measured on B200 (profiles/r02_ln_fusion_ab.txt): folding the LayerNorm into the GEMMs saves its 4 B/element read
+// but makes the four forward epilogues heavier (+2 B/element bf16 copy, statistics, rank-1 correction).  For the
+// large HBM-bound tower (text, 77,000 rows) that is a gain; for ~6,000-row towers, whose 25-40 us GEMMs are
+// launch / epilogue bound, the stand-alone LayerNorm kernels are faster: choose by row count unless told otherwise.
+// (ragged towers: always the stand-alone kernels, which take the packed positions)
+bool ln_fused_for(const mudpt_handle* h, const Tower& t, int rows) {
+  return !t.ragged && (h->ln_fused == 1 || (h->ln_fused < 0 && rows >= 32768));
+}
+
+// Shape of the tower for S sequences of L tokens, or (off != null: host row offsets [S+1]) for S packed sequences of at
+// most L tokens, and the memory of its input.  The workspaces follow at the first walk that needs them.  Each kind of
+// memory grows to the largest shape seen; the outgrown buffers are released first (a CoCoOp-style caller whose B x C
+// changes would otherwise pile up GBs until mudpt_destroy).
+int ensure_input(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullptr) {
   const size_t rows = off ? static_cast<size_t>(off[S]) : static_cast<size_t>(S) * L;
   t.S = S;
   t.L = L;
@@ -226,55 +284,25 @@ int ensure_tower(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullp
     t.attn_sq = 0;
     for (int q = 0; q < S; ++q) t.attn_sq += static_cast<double>(off[q + 1] - off[q]) * (off[q + 1] - off[q]);
   }
-  const size_t head_need = feature_head_workspace_floats(S, t.d, h->cfg.embed_dim);
-  if (head_need > t.head_cap) {  // gathered CLS / EOT rows of the feature head + split-K partials
-    CUDA_OK(h, dev_alloc(h, &t.head_ws, head_need));
-    t.head_cap = head_need;
-  }
-  if (!t.gws.partials) {
-    CUDA_OK(h, dev_alloc(h, &t.gws.partials, gemm_workspace_partial_bytes() / sizeof(float)));
-    CUDA_OK(h, dev_alloc(h, &t.gws.flags, gemm_workspace_flag_bytes() / sizeof(unsigned)));
-    CUDA_OK(h, cudaMemset(t.gws.flags, 0, gemm_workspace_flag_bytes()));
-  }
-  if (static_cast<size_t>(S) > t.pr_cap) {
-    for (void* p : t.pr_allocs) cudaFree(p);
-    t.pr_allocs.clear();
-    gemm_clear_tensor_map_cache();
-    std::vector<void*>* g = &t.pr_allocs;
-    const size_t Ss = S, d = t.d;
-    const int dots_mlp = (4 * t.d + gemm_dots_span(4 * t.d) - 1) / gemm_dots_span(4 * t.d);
-    CUDA_OK(h, dev_alloc(h, &t.pr_o, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_xmb, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_h, Ss * 4 * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_g, Ss * 4 * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_a, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_dxb, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_dh, Ss * 4 * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_do, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_x, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_xm, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_xo, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_dx, Ss * d, g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_stm, Ss * (d / 64), g));
-    CUDA_OK(h, dev_alloc(h, &t.pr_dots, Ss * dots_mlp, g));
-    t.pr_cap = S;
+  if (rows > t.in_rows || static_cast<size_t>(S) > t.in_S) {
+    release(t.in_mem);
+    t.in_rows = rows > t.in_rows ? rows : t.in_rows;
+    t.in_S = static_cast<size_t>(S) > t.in_S ? S : t.in_S;
+    const size_t R = t.in_rows, Sn = t.in_S, d = t.d;
+    AllocGroup* g = &t.in_mem;
+    CUDA_OK(h, dev_alloc(h, &t.x_in[0], R * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.xb_in[0], R * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.st_in[0], R * (d / 64), g));
+    if (t.n_ctx > 0) CUDA_OK(h, dev_alloc(h, &t.p0_rows, Sn * t.n_ctx, g));
+    if (t.causal) {  // text
+      CUDA_OK(h, dev_alloc(h, &t.seq_off, Sn + 1, g));
+      CUDA_OK(h, dev_alloc(h, &t.tok_pos, R, g));
+      CUDA_OK(h, dev_alloc(h, &t.eot, Sn, g));
+    }
+    t.p0_S = 0;
     t.fwd_done = false;
   }
   const size_t R0 = static_cast<size_t>(S) * t.n_ctx;
-  if (R0 > t.p0_cap) {
-    for (void* p : t.p0_allocs) cudaFree(p);
-    t.p0_allocs.clear();
-    gemm_clear_tensor_map_cache();
-    std::vector<void*>* g = &t.p0_allocs;
-    CUDA_OK(h, dev_alloc(h, &t.p0_rows, R0, g));
-    CUDA_OK(h, dev_alloc(h, &t.p0_dqkv, R0 * 3 * t.d, g));
-    CUDA_OK(h, dev_alloc(h, &t.p0_a, R0 * t.d, g));
-    CUDA_OK(h, dev_alloc(h, &t.p0_dxb, R0 * t.d, g));
-    CUDA_OK(h, dev_alloc(h, &t.p0_x, R0 * t.d, g));
-    CUDA_OK(h, dev_alloc(h, &t.p0_dx, R0 * t.d, g));
-    t.p0_cap = R0;
-    t.p0_S = 0;
-  }
   if (R0 > 0 && (off || t.p0_S != S || t.p0_L != L)) {
     std::vector<int> r(R0);
     for (int q = 0; q < S; ++q)
@@ -283,26 +311,19 @@ int ensure_tower(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullp
     t.p0_S = S;
     t.p0_L = off ? -1 : L;  // (packed rows: rebuilt on the next set-up)
   }
-  if (rows <= t.cap_rows) return 0;
-  // grow: the outgrown buffers are released first (cudaFree waits for the device, so nothing in flight uses them);
-  // a CoCoOp-style caller whose B x C changes would otherwise pile up GBs until mudpt_destroy
-  for (void* p : t.ws_allocs) cudaFree(p);
-  t.ws_allocs.clear();
-  gemm_clear_tensor_map_cache();
-  const size_t d = t.d;
-  const size_t parts = d / 64;
-  std::vector<void*>* g = &t.ws_allocs;
-  t.x_in.assign(t.layers + 1, nullptr);
-  t.x_mid.assign(t.layers, nullptr);
-  t.qkv.assign(t.layers, nullptr);
-  t.o.assign(t.layers, nullptr);
-  t.h.assign(t.layers, nullptr);
-  t.lse.assign(t.layers, nullptr);
-  t.xb_in.assign(t.layers + 1, nullptr);
-  t.xb_mid.assign(t.layers, nullptr);
-  t.st_in.assign(t.layers + 1, nullptr);
-  t.st_mid.assign(t.layers, nullptr);
-  for (int i = 0; i <= t.layers; ++i) {
+  return 0;
+}
+
+// Training workspace for the tower's current shape: the saved activations of every layer (x_in[1..]), the forward and
+// backward transients, the pruned blocks' rows, the feature head's, stream-K and splice scratch, the vision stem's patches
+int ensure_train(mudpt_handle* h, Tower& t, cudaStream_t st) {
+  if (static_cast<size_t>(t.rows) <= t.cap_rows && static_cast<size_t>(t.S) <= t.cap_S) return 0;
+  release(t.train_mem);
+  t.cap_rows = static_cast<size_t>(t.rows) > t.cap_rows ? t.rows : t.cap_rows;
+  t.cap_S = static_cast<size_t>(t.S) > t.cap_S ? t.S : t.cap_S;
+  const size_t rows = t.cap_rows, Ss = t.cap_S, d = t.d, parts = d / 64, R0 = Ss * t.n_ctx;
+  AllocGroup* g = &t.train_mem;
+  for (int i = 1; i <= t.layers; ++i) {
     CUDA_OK(h, dev_alloc(h, &t.x_in[i], rows * d, g));
     CUDA_OK(h, dev_alloc(h, &t.xb_in[i], rows * d, g));
     CUDA_OK(h, dev_alloc(h, &t.st_in[i], rows * parts, g));
@@ -327,14 +348,116 @@ int ensure_tower(mudpt_handle* h, Tower& t, int S, int L, const int* off = nullp
   CUDA_OK(h, dev_alloc(h, &t.dx_bf16, rows * d, g));
   CUDA_OK(h, dev_alloc(h, &t.dx, rows * d, g));
   CUDA_OK(h, dev_alloc(h, &t.dsum, rows * t.H, g));
-  if (!t.splice_ws) {
-    const size_t nws = splice_bwd_workspace_floats(t.n_ctx > 0 ? t.n_ctx : 1, t.d);
-    CUDA_OK(h, dev_alloc(h, &t.splice_ws, nws));
-    CUDA_OK(h, cudaMemset(t.splice_ws, 0, nws * sizeof(float)));  // (the kernel's tickets start at zero and are left at zero)
+  CUDA_OK(h, dev_alloc(h, &t.pr_o, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_xmb, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_h, Ss * 4 * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_g, Ss * 4 * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_a, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_dxb, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_dh, Ss * 4 * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_do, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_x, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_xm, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_xo, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_dx, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_stm, Ss * parts, g));
+  CUDA_OK(h, dev_alloc(h, &t.pr_dots, Ss * dots_mlp, g));
+  if (R0 > 0) {
+    CUDA_OK(h, dev_alloc(h, &t.p0_dqkv, R0 * 3 * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.p0_a, R0 * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.p0_dxb, R0 * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.p0_x, R0 * d, g));
+    CUDA_OK(h, dev_alloc(h, &t.p0_dx, R0 * d, g));
   }
-  t.cap_rows = rows;
+  // gathered CLS / EOT rows of the feature head + split-K partials
+  CUDA_OK(h, dev_alloc(h, &t.head_ws, feature_head_workspace_floats(static_cast<int>(Ss), t.d, h->cfg.embed_dim), g));
+  CUDA_OK(h, dev_alloc(h, &t.gws.partials, gemm_workspace_partial_bytes() / sizeof(float), g));
+  CUDA_OK(h, dev_alloc(h, &t.gws.flags, gemm_workspace_flag_bytes() / sizeof(unsigned), g));
+  CUDA_OK(h, cudaMemset(t.gws.flags, 0, gemm_workspace_flag_bytes()));
+  const size_t nws = splice_bwd_workspace_floats(t.n_ctx > 0 ? t.n_ctx : 1, t.d);
+  CUDA_OK(h, dev_alloc(h, &t.splice_ws, nws, g));
+  CUDA_OK(h, cudaMemset(t.splice_ws, 0, nws * sizeof(float)));  // (the kernel's tickets start at zero and are left at zero)
+  if (t.stem_per_seq) {
+    CUDA_OK(h, dev_alloc(h, &t.patches, Ss * t.stem_per_seq, g));
+    CUDA_OK(h, cudaMemsetAsync(t.patches, 0, Ss * t.stem_per_seq * sizeof(bf16), st));  // (the K padding stays zero)
+  }
   t.fwd_done = false;
   return 0;
+}
+
+// Inference workspace for a walk over S sequences / `rows` token rows (DESIGN.md section 3): two fp32 residual buffers the
+// layers use alternately (x_in, x_mid) with their bf16 copies and statistics when the LayerNorm is fused, one a_buf / qkv /
+// o / g / lse shared by every layer, the pruned block's rows, the feature head's and stream-K scratch, the stem's patches.
+// Nothing in it is read by a backward.
+int ensure_infer(mudpt_handle* h, Tower& t, int S, int rows, bool fused, cudaStream_t st) {
+  Tower::Infer& f = t.inf;
+  if (!f.mem.ptrs.empty() && static_cast<size_t>(rows) <= f.rows && static_cast<size_t>(S) <= f.S && (f.fused || !fused)) return 0;
+  release(f.mem);
+  f.rows = static_cast<size_t>(rows) > f.rows ? rows : f.rows;
+  f.S = static_cast<size_t>(S) > f.S ? S : f.S;
+  f.fused = f.fused || fused;
+  const size_t R = f.rows, Ss = f.S, d = t.d, parts = d / 64;
+  AllocGroup* g = &f.mem;
+  FwdView& v = f.v;
+  float* x[2];
+  bf16* xb[2] = {nullptr, nullptr};
+  float2* xs[2] = {nullptr, nullptr};
+  for (int k = 0; k < 2; ++k) {
+    CUDA_OK(h, dev_alloc(h, &x[k], R * d, g));
+    if (f.fused) {
+      CUDA_OK(h, dev_alloc(h, &xb[k], R * d, g));
+      CUDA_OK(h, dev_alloc(h, &xs[k], R * parts, g));
+    }
+  }
+  bf16 *qkv, *o;
+  float* lse;
+  CUDA_OK(h, dev_alloc(h, &v.a_buf, R * d, g));
+  CUDA_OK(h, dev_alloc(h, &qkv, R * 3 * d, g));
+  CUDA_OK(h, dev_alloc(h, &o, R * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.g_buf, R * 4 * d, g));
+  CUDA_OK(h, dev_alloc(h, &lse, R * t.H, g));
+  v.x_in.assign(t.layers + 1, x[0]);
+  v.x_mid.assign(t.layers, x[1]);
+  v.xb_in.assign(t.layers + 1, xb[0]);
+  v.xb_mid.assign(t.layers, xb[1]);
+  v.st_in.assign(t.layers + 1, xs[0]);
+  v.st_mid.assign(t.layers, xs[1]);
+  v.qkv.assign(t.layers, qkv);
+  v.o.assign(t.layers, o);
+  v.h.clear();
+  v.lse.assign(t.layers, lse);
+  CUDA_OK(h, dev_alloc(h, &v.pr_x, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_o, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_xm, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_xmb, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_stm, Ss * parts, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_g, Ss * 4 * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_a, Ss * d, g));
+  CUDA_OK(h, dev_alloc(h, &v.pr_xo, Ss * d, g));
+  v.pr_h = nullptr;
+  CUDA_OK(h, dev_alloc(h, &v.head_ws, feature_head_workspace_floats(static_cast<int>(Ss), t.d, h->cfg.embed_dim), g));
+  CUDA_OK(h, dev_alloc(h, &f.gws.partials, gemm_workspace_partial_bytes() / sizeof(float), g));
+  CUDA_OK(h, dev_alloc(h, &f.gws.flags, gemm_workspace_flag_bytes() / sizeof(unsigned), g));
+  CUDA_OK(h, cudaMemset(f.gws.flags, 0, gemm_workspace_flag_bytes()));
+  v.gws = &f.gws;
+  if (t.stem_per_seq) {
+    CUDA_OK(h, dev_alloc(h, &f.patches, Ss * t.stem_per_seq, g));
+    CUDA_OK(h, cudaMemsetAsync(f.patches, 0, Ss * t.stem_per_seq * sizeof(bf16), st));
+  }
+  return 0;
+}
+
+// the training walk's view of the tower: every layer its own buffers
+FwdView train_view(Tower& t) {
+  FwdView v;
+  v.S = t.S; v.rows = t.rows; v.attn_sq = t.attn_sq;
+  v.x_in = t.x_in; v.x_mid = t.x_mid; v.xb_in = t.xb_in; v.xb_mid = t.xb_mid; v.st_in = t.st_in; v.st_mid = t.st_mid;
+  v.qkv = t.qkv; v.o = t.o; v.h = t.h; v.lse = t.lse;
+  v.a_buf = t.a_buf; v.g_buf = t.g_buf;
+  v.pr_x = t.pr_x; v.pr_xm = t.pr_xm; v.pr_xo = t.pr_xo; v.pr_o = t.pr_o; v.pr_xmb = t.pr_xmb; v.pr_h = t.pr_h; v.pr_g = t.pr_g;
+  v.pr_a = t.pr_a; v.pr_stm = t.pr_stm;
+  v.head_ws = t.head_ws; v.gws = &t.gws;
+  return v;
 }
 
 // ---------------------------------------------------------------------------- weights
@@ -432,18 +555,17 @@ int ensure_folded(mudpt_handle* h, Tower& t, cudaStream_t st) {
 // (out-proj, c_proj) write the new residual row as fp32 + bf16 + partial statistics (and the NEXT block's spliced
 // prompt rows in place of the computed ones); the QKV / c_fc GEMMs read the bf16 row as their A operand and apply
 // the normalisation in their epilogue (EPI_LN_*: gamma folded into the weight, mean as a rank-1 correction).
-// Precondition of the fused path: x_in[0], xb_in[0], st_in[0] hold the tower input (layer-0 splice excepted).
-int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_splice_layer, cudaStream_t st) {
-  const int M = t.rows, d = t.d;
+// Precondition of the fused path: v.x_in[0], v.xb_in[0], v.st_in[0] hold the tower input (layer-0 splice excepted).
+// The walk writes the buffers of `v` only (and, with a layer-0 splice, the prompt rows of v.x_in[0]); with v.h empty the
+// c_fc GEMMs write QuickGELU(h) alone (no backward will need h): the same values as the training walk, bit for bit.
+int tower_forward(mudpt_handle* h, Tower& t, FwdView& v, const float* prompts, int first_splice_layer, cudaStream_t st) {
+  const int M = v.rows, d = t.d;
   const double Md = static_cast<double>(M), dd = d;
-  const double attn_fl = 4.0 * t.H * t.attn_sq * 64.0;  // QK^T + PV, dense count
-  // Measured on B200 (profiles/r02_ln_fusion_ab.txt): folding the LayerNorm into the GEMMs saves its 4 B/element read
-  // but makes the four forward epilogues heavier (+2 B/element bf16 copy, statistics, rank-1 correction).  For the
-  // large HBM-bound tower (text, 77,000 rows) that is a gain; for ~6,000-row towers, whose 25-40 us GEMMs are
-  // launch / epilogue bound, the stand-alone LayerNorm kernels are faster: choose by row count unless told otherwise.
-  // (ragged towers: always the stand-alone kernels, which take the packed positions)
-  const bool fused = !t.ragged && (h->ln_fused == 1 || (h->ln_fused < 0 && M >= 32768));
+  const double attn_fl = 4.0 * t.H * v.attn_sq * 64.0;  // QK^T + PV, dense count
+  const bool fused = ln_fused_for(h, t, M);
   const bool pruned = h->prune;
+  const bool keep_h = !v.h.empty();
+  const double fc_out = keep_h ? 2.0 : 1.0;  // bf16 outputs of c_fc
   const int parts = d / 64;
   auto spliced = [&](int i) { return i < t.depth && i >= first_splice_layer && t.n_ctx > 0 && i < t.layers; };
   if (fused && ensure_folded(h, t, st)) return -1;
@@ -453,74 +575,80 @@ int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_spl
     // residual epilogue (layer 0: a kernel of its own, with the statistics of the spliced rows)
     if (spliced(i) && fused && i == 0) {
       const float* pr = prompts + static_cast<size_t>(i) * t.n_ctx * d;
-      CKP(h, st, PC_SPLICE, 0, 2.0 * t.S * t.n_ctx * dd * 4, splice_fwd_stats(t.x_in[i], t.xb_in[i], t.st_in[i], pr, t.S, t.L, t.row0, t.n_ctx, d, st));
+      CKP(h, st, PC_SPLICE, 0, 2.0 * v.S * t.n_ctx * dd * 4, splice_fwd_stats(v.x_in[i], v.xb_in[i], v.st_in[i], pr, v.S, t.L, t.row0, t.n_ctx, d, st));
     }
     // x + attn(ln_1(x))   (clip/model.py:299)
     GemmEpilogue e1;
-    e1.out0 = t.qkv[i]; e1.ldc = 3 * d;
+    e1.out0 = v.qkv[i]; e1.ldc = 3 * d;
     if (fused) {
-      e1.mode = EPI_LN_BF16; e1.bias = w.b_in_ln; e1.colsum = w.cs_in; e1.ln_stats = t.st_in[i]; e1.ln_parts = parts; e1.ln_width = d; e1.ln_eps = kLnEps;
+      e1.mode = EPI_LN_BF16; e1.bias = w.b_in_ln; e1.colsum = w.cs_in; e1.ln_stats = v.st_in[i]; e1.ln_parts = parts; e1.ln_width = d; e1.ln_eps = kLnEps;
       CKP(h, st, PC_GEMM_QKV, 2.0 * Md * 3 * dd * dd, 2 * (Md * dd + 3 * dd * dd + Md * 3 * dd),
-          gemm_bf16_tn(t.xb_in[i], d, w.w_in_ln, d, e1, M, 3 * d, d, st, &t.gws));
+          gemm_bf16_tn(v.xb_in[i], d, w.w_in_ln, d, e1, M, 3 * d, d, st, v.gws));
     } else {
       CKP(h, st, PC_LN_FWD, 0, Md * dd * 6,
-          layernorm_fwd_splice(t.x_in[i], spliced(i) ? prompts + static_cast<size_t>(i) * t.n_ctx * d : nullptr, t.L, t.row0,
-                               spliced(i) ? t.n_ctx : 0, w.ln1_g, w.ln1_b, t.a_buf, true, M, d, kLnEps, st, t.packed_pos()));
+          layernorm_fwd_splice(v.x_in[i], spliced(i) ? prompts + static_cast<size_t>(i) * t.n_ctx * d : nullptr, t.L, t.row0,
+                               spliced(i) ? t.n_ctx : 0, w.ln1_g, w.ln1_b, v.a_buf, true, M, d, kLnEps, st, t.packed_pos()));
       e1.mode = EPI_BF16; e1.bias = w.b_in;
       CKP(h, st, PC_GEMM_QKV, 2.0 * Md * 3 * dd * dd, 2 * (Md * dd + 3 * dd * dd + Md * 3 * dd),
-          gemm_bf16_tn(t.a_buf, d, w.w_in, d, e1, M, 3 * d, d, st, &t.gws));
+          gemm_bf16_tn(v.a_buf, d, w.w_in, d, e1, M, 3 * d, d, st, v.gws));
     }
     CKP(h, st, PC_ATTN_FWD, attn_fl, Md * dd * 2 * 4,
-        t.ragged ? attention_varlen_fwd(t.qkv[i], t.o[i], t.lse[i], t.seq_off, t.S, t.L, t.H, d, st)
-                 : attention_fwd(t.qkv[i], t.o[i], t.lse[i], t.S, t.L, t.H, d, t.causal, st));
+        t.ragged ? attention_varlen_fwd(v.qkv[i], v.o[i], v.lse[i], t.seq_off, v.S, t.L, t.H, d, st)
+                 : attention_fwd(v.qkv[i], v.o[i], v.lse[i], v.S, t.L, t.H, d, t.causal, st));
     if (pruned && i == t.layers - 1) {
       // the block's output is consumed on one row per sequence: out-proj and the MLP on S gathered rows
-      const int S = t.S;
+      const int S = v.S;
       const double Sd = S;
-      CKP(h, st, PC_SPLICE, 0, Sd * dd * 12, gather_rows(t.x_in[i], t.o[i], t.sel_rows, S, t.row_L(), t.pr_x, t.pr_o, d, st));
+      CKP(h, st, PC_SPLICE, 0, Sd * dd * 12, gather_rows(v.x_in[i], v.o[i], t.sel_rows, S, t.row_L(), v.pr_x, v.pr_o, d, st));
       GemmEpilogue p2;
-      p2.out0 = t.pr_xm; p2.bias = w.b_out; p2.resid = t.pr_x; p2.ldc = d;
-      if (fused) { p2.mode = EPI_RESID_STATS; p2.out2 = t.pr_xmb; p2.stats_out = t.pr_stm; }
+      p2.out0 = v.pr_xm; p2.bias = w.b_out; p2.resid = v.pr_x; p2.ldc = d;
+      if (fused) { p2.mode = EPI_RESID_STATS; p2.out2 = v.pr_xmb; p2.stats_out = v.pr_stm; }
       else p2.mode = EPI_RESID_F32;
-      CKP(h, st, PC_GEMM, 2.0 * Sd * dd * dd, 2 * (Sd * dd + dd * dd) + 10 * Sd * dd, gemm_bf16_tn(t.pr_o, d, w.w_out, d, p2, S, d, d, st, &t.gws));
+      CKP(h, st, PC_GEMM, 2.0 * Sd * dd * dd, 2 * (Sd * dd + dd * dd) + 10 * Sd * dd, gemm_bf16_tn(v.pr_o, d, w.w_out, d, p2, S, d, d, st, v.gws));
       GemmEpilogue p3;
-      p3.out0 = t.pr_h; p3.out1 = t.pr_g; p3.ldc = 4 * d;
+      p3.ldc = 4 * d;
+      if (keep_h) { p3.out0 = v.pr_h; p3.out1 = v.pr_g; }
+      else p3.out0 = v.pr_g;
       if (fused) {
-        p3.mode = EPI_LN_GELU; p3.bias = w.b_fc_ln; p3.colsum = w.cs_fc; p3.ln_stats = t.pr_stm; p3.ln_parts = parts; p3.ln_width = d; p3.ln_eps = kLnEps;
-        CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * dd + 4 * dd * dd + 2 * Sd * 4 * dd), gemm_bf16_tn(t.pr_xmb, d, w.w_fc_ln, d, p3, S, 4 * d, d, st, &t.gws));
+        p3.mode = keep_h ? EPI_LN_GELU : EPI_LN_GELU_ONLY; p3.bias = w.b_fc_ln; p3.colsum = w.cs_fc; p3.ln_stats = v.pr_stm; p3.ln_parts = parts;
+        p3.ln_width = d; p3.ln_eps = kLnEps;
+        CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * dd + 4 * dd * dd + fc_out * Sd * 4 * dd), gemm_bf16_tn(v.pr_xmb, d, w.w_fc_ln, d, p3, S, 4 * d, d, st, v.gws));
       } else {
-        CKP(h, st, PC_LN_FWD, 0, Sd * dd * 6, layernorm_fwd(t.pr_xm, w.ln2_g, w.ln2_b, t.pr_a, true, S, d, kLnEps, st));
-        p3.mode = EPI_GELU; p3.bias = w.b_fc;
-        CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * dd + 4 * dd * dd + 2 * Sd * 4 * dd), gemm_bf16_tn(t.pr_a, d, w.w_fc, d, p3, S, 4 * d, d, st, &t.gws));
+        CKP(h, st, PC_LN_FWD, 0, Sd * dd * 6, layernorm_fwd(v.pr_xm, w.ln2_g, w.ln2_b, v.pr_a, true, S, d, kLnEps, st));
+        p3.mode = keep_h ? EPI_GELU : EPI_GELU_ONLY; p3.bias = w.b_fc;
+        CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * dd + 4 * dd * dd + fc_out * Sd * 4 * dd), gemm_bf16_tn(v.pr_a, d, w.w_fc, d, p3, S, 4 * d, d, st, v.gws));
       }
       GemmEpilogue p4;
-      p4.mode = EPI_RESID_F32; p4.out0 = t.pr_xo; p4.bias = w.b_pr; p4.resid = t.pr_xm; p4.ldc = d;
-      CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * 4 * dd + 4 * dd * dd) + 8 * Sd * dd, gemm_bf16_tn(t.pr_g, 4 * d, w.w_pr, 4 * d, p4, S, d, 4 * d, st, &t.gws));
+      p4.mode = EPI_RESID_F32; p4.out0 = v.pr_xo; p4.bias = w.b_pr; p4.resid = v.pr_xm; p4.ldc = d;
+      CKP(h, st, PC_GEMM, 2.0 * Sd * 4 * dd * dd, 2 * (Sd * 4 * dd + 4 * dd * dd) + 8 * Sd * dd, gemm_bf16_tn(v.pr_g, 4 * d, w.w_pr, 4 * d, p4, S, d, 4 * d, st, v.gws));
       break;
     }
     GemmEpilogue e2;
-    e2.out0 = t.x_mid[i]; e2.bias = w.b_out; e2.resid = t.x_in[i]; e2.ldc = d;
-    if (fused) { e2.mode = EPI_RESID_STATS; e2.out2 = t.xb_mid[i]; e2.stats_out = t.st_mid[i]; }
+    e2.out0 = v.x_mid[i]; e2.bias = w.b_out; e2.resid = v.x_in[i]; e2.ldc = d;
+    if (fused) { e2.mode = EPI_RESID_STATS; e2.out2 = v.xb_mid[i]; e2.stats_out = v.st_mid[i]; }
     else e2.mode = EPI_RESID_F32;
     CKP(h, st, PC_GEMM_OUT, 2.0 * Md * dd * dd, 2 * (Md * dd + dd * dd) + (fused ? 10 : 8) * Md * dd,
-        gemm_bf16_tn(t.o[i], d, w.w_out, d, e2, M, d, d, st, &t.gws));
+        gemm_bf16_tn(v.o[i], d, w.w_out, d, e2, M, d, d, st, v.gws));
     // x + c_proj(QuickGELU(c_fc(ln_2(x))))   (clip/model.py:300)
     GemmEpilogue e3;
-    e3.out0 = t.h[i]; e3.out1 = t.g_buf; e3.ldc = 4 * d;
+    e3.ldc = 4 * d;
+    if (keep_h) { e3.out0 = v.h[i]; e3.out1 = v.g_buf; }
+    else e3.out0 = v.g_buf;
     if (fused) {
-      e3.mode = EPI_LN_GELU; e3.bias = w.b_fc_ln; e3.colsum = w.cs_fc; e3.ln_stats = t.st_mid[i]; e3.ln_parts = parts; e3.ln_width = d; e3.ln_eps = kLnEps;
-      CKP(h, st, PC_GEMM_FC, 2.0 * Md * 4 * dd * dd, 2 * (Md * dd + 4 * dd * dd + 2 * Md * 4 * dd),
-          gemm_bf16_tn(t.xb_mid[i], d, w.w_fc_ln, d, e3, M, 4 * d, d, st, &t.gws));
+      e3.mode = keep_h ? EPI_LN_GELU : EPI_LN_GELU_ONLY; e3.bias = w.b_fc_ln; e3.colsum = w.cs_fc; e3.ln_stats = v.st_mid[i]; e3.ln_parts = parts;
+      e3.ln_width = d; e3.ln_eps = kLnEps;
+      CKP(h, st, PC_GEMM_FC, 2.0 * Md * 4 * dd * dd, 2 * (Md * dd + 4 * dd * dd + fc_out * Md * 4 * dd),
+          gemm_bf16_tn(v.xb_mid[i], d, w.w_fc_ln, d, e3, M, 4 * d, d, st, v.gws));
     } else {
-      CKP(h, st, PC_LN_FWD, 0, Md * dd * 6, layernorm_fwd(t.x_mid[i], w.ln2_g, w.ln2_b, t.a_buf, true, M, d, kLnEps, st));
-      e3.mode = EPI_GELU; e3.bias = w.b_fc;
-      CKP(h, st, PC_GEMM_FC, 2.0 * Md * 4 * dd * dd, 2 * (Md * dd + 4 * dd * dd + 2 * Md * 4 * dd),
-          gemm_bf16_tn(t.a_buf, d, w.w_fc, d, e3, M, 4 * d, d, st, &t.gws));
+      CKP(h, st, PC_LN_FWD, 0, Md * dd * 6, layernorm_fwd(v.x_mid[i], w.ln2_g, w.ln2_b, v.a_buf, true, M, d, kLnEps, st));
+      e3.mode = keep_h ? EPI_GELU : EPI_GELU_ONLY; e3.bias = w.b_fc;
+      CKP(h, st, PC_GEMM_FC, 2.0 * Md * 4 * dd * dd, 2 * (Md * dd + 4 * dd * dd + fc_out * Md * 4 * dd),
+          gemm_bf16_tn(v.a_buf, d, w.w_fc, d, e3, M, 4 * d, d, st, v.gws));
     }
     GemmEpilogue e4;
-    e4.out0 = t.x_in[i + 1]; e4.bias = w.b_pr; e4.resid = t.x_mid[i]; e4.ldc = d;
+    e4.out0 = v.x_in[i + 1]; e4.bias = w.b_pr; e4.resid = v.x_mid[i]; e4.ldc = d;
     if (fused) {
-      e4.mode = EPI_RESID_STATS; e4.out2 = t.xb_in[i + 1]; e4.stats_out = t.st_in[i + 1];
+      e4.mode = EPI_RESID_STATS; e4.out2 = v.xb_in[i + 1]; e4.stats_out = v.st_in[i + 1];
       if (spliced(i + 1)) {  // the next block's prompt rows replace the computed ones (they get no gradient: splice_bwd)
         e4.splice_prompt = prompts + static_cast<size_t>(i + 1) * t.n_ctx * d;
         e4.splice_row0 = t.row0; e4.splice_n = t.n_ctx; e4.splice_L = t.L;
@@ -529,19 +657,28 @@ int tower_forward(mudpt_handle* h, Tower& t, const float* prompts, int first_spl
       e4.mode = EPI_RESID_F32;
     }
     CKP(h, st, PC_GEMM_PROJ, 2.0 * Md * 4 * dd * dd, 2 * (Md * 4 * dd + 4 * dd * dd) + (fused ? 10 : 8) * Md * dd,
-        gemm_bf16_tn(t.g_buf, 4 * d, w.w_pr, 4 * d, e4, M, d, 4 * d, st, &t.gws));
+        gemm_bf16_tn(v.g_buf, 4 * d, w.w_pr, 4 * d, e4, M, d, 4 * d, st, v.gws));
   }
-  t.fwd_done = true;
-  t.fwd_fused = fused;
-  t.fwd_pruned = pruned;
+  v.fused = fused;
+  v.pruned = pruned;
   return 0;
 }
 
-// x (and the row stride) the feature head reads its one row per sequence from
-const float* tower_head_input(const Tower& t, const int** rows, int* L) {
-  if (t.fwd_pruned) { *rows = nullptr; *L = 1; return t.pr_xo; }
+// x (and the row stride) the feature head reads its one row per sequence from, after a walk over `v`
+const float* tower_head_input(const Tower& t, const FwdView& v, const int** rows, int* L) {
+  if (v.pruned) { *rows = nullptr; *L = 1; return v.pr_xo; }
   *rows = t.sel_rows; *L = t.row_L();
-  return t.x_in[t.layers];
+  return v.x_in[t.layers];
+}
+
+// the training walk: saves the activations for the backward
+int tower_forward_train(mudpt_handle* h, Tower& t, const float* prompts, int first_splice_layer, cudaStream_t st, FwdView& v) {
+  v = train_view(t);
+  if (tower_forward(h, t, v, prompts, first_splice_layer, st)) return -1;
+  t.fwd_done = true;
+  t.fwd_fused = v.fused;
+  t.fwd_pruned = v.pruned;
+  return 0;
 }
 
 // Precondition: t.dx / t.dx_bf16 hold the gradient w.r.t. the tower output x_in[layers].
@@ -739,6 +876,19 @@ int mudpt_create(const mudpt_config* cfg, mudpt_handle** out) {
   t.L = cfg->context_length; t.row0 = 1; t.depth = cfg->prompt_depth; t.causal = true;
   t.lw.resize(t.layers);
   h->Kp = (3 * cfg->vision_patch_size * cfg->vision_patch_size + 7) & ~7;
+  v.stem_per_seq = static_cast<size_t>(np) * h->Kp;
+  for (Tower* w : {&v, &t}) {
+    w->x_in.assign(w->layers + 1, nullptr);
+    w->xb_in.assign(w->layers + 1, nullptr);
+    w->st_in.assign(w->layers + 1, nullptr);
+    w->x_mid.assign(w->layers, nullptr);
+    w->xb_mid.assign(w->layers, nullptr);
+    w->st_mid.assign(w->layers, nullptr);
+    w->qkv.assign(w->layers, nullptr);
+    w->o.assign(w->layers, nullptr);
+    w->h.assign(w->layers, nullptr);
+    w->lse.assign(w->layers, nullptr);
+  }
   h->launches_at_create = g_launch_counter.load();
   h->ln_fused = getenv("MUDPT_LN_FUSED") ? (atoi(getenv("MUDPT_LN_FUSED")) != 0 ? 1 : 0) : -1;
   h->ln_bwd_fused = env_flag("MUDPT_LN_BWD_FUSED", false);
@@ -753,11 +903,9 @@ void mudpt_destroy(mudpt_handle* h) {
   if (!h) return;
   cudaSetDevice(h->cfg.device);
   for (void* p : h->allocs) cudaFree(p);
-  for (Tower* t : {&h->vis, &h->txt}) {
-    for (void* p : t->ws_allocs) cudaFree(p);
-    for (void* p : t->pr_allocs) cudaFree(p);
-    for (void* p : t->p0_allocs) cudaFree(p);
-  }
+  for (Tower* t : {&h->vis, &h->txt})
+    for (AllocGroup* g : {&t->in_mem, &t->train_mem, &t->inf.mem})
+      for (void* p : g->ptrs) cudaFree(p);
   for (ProfRec& r : h->prof.recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
   for (cudaEvent_t e : h->prof.pool) cudaEventDestroy(e);
   gemm_clear_tensor_map_cache();
@@ -829,38 +977,57 @@ int mudpt_weights_complete(mudpt_handle* h) {
   return 0;
 }
 
+// conv1 as a GEMM over extracted patches, scattered to token rows 1..np with +pos (clip/model.py:527-531), the CLS rows,
+// then ln_pre in place (:541) -- the prompt rows are overwritten by the layer-0 splice with prompts[0] = ln_pre(visual_ctx +
+// shared_ctx), which is identical for every image -- and, for the fused LayerNorm, the bf16 copy + statistics of x0
+static int vision_stem(mudpt_handle* h, const float* images, int B, bf16* patches, float* x0, bf16* xb0, float2* st0, cudaStream_t st) {
+  const mudpt_config& c = h->cfg;
+  const Tower& t = h->vis;
+  const int np = t.row0 - 1;
+  CK(h, im2col_bf16(images, patches, B, c.image_resolution, c.vision_patch_size, h->Kp, st));
+  GemmEpilogue ep;
+  ep.mode = EPI_PATCH; ep.out0 = x0; ep.resid = h->pos_v; ep.ldc = t.d; ep.patch_np = np; ep.patch_L = t.L;
+  CK(h, gemm_bf16_tn(patches, h->Kp, h->w_conv, h->Kp, ep, B * np, t.d, h->Kp, st));
+  CK(h, write_cls_rows(x0, h->cls, h->pos_v, B, t.L, t.d, st));
+  CK(h, layernorm_fwd(x0, h->ln_pre_g, h->ln_pre_b, x0, false, B * t.L, t.d, kLnEps, st));
+  if (ln_fused_for(h, t, B * t.L)) CK(h, rowstats(x0, xb0, st0, B * t.L, t.d, st));
+  return 0;
+}
+
 int mudpt_vision_forward(mudpt_handle* h, const float* images, int32_t B, const float* prompts, float* f_img, void* stream) {
   if (!h || !images || !f_img || (!prompts && h->cfg.n_ctx > 0)) return fail(h, "mudpt_vision_forward: null argument");
   if (B <= 0) return fail(h, "mudpt_vision_forward: empty batch");
   if (mudpt_weights_complete(h)) return -1;
   cudaSetDevice(h->cfg.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const mudpt_config& c = h->cfg;
   Tower& t = h->vis;
-  const int np = t.row0 - 1;
-  if (ensure_tower(h, t, B, t.row0 + t.n_ctx)) return -1;
-  const size_t need = static_cast<size_t>(B) * np * h->Kp;
-  if (need > h->patches_cap) {
-    CUDA_OK(h, dev_alloc(h, &h->patches, need));
-    CUDA_OK(h, cudaMemsetAsync(h->patches, 0, need * sizeof(bf16), st));
-    h->patches_cap = need;
-  }
-  // conv1 as a GEMM over extracted patches, scattered to token rows 1..np with +pos (clip/model.py:527-531)
-  CK(h, im2col_bf16(images, h->patches, B, c.image_resolution, c.vision_patch_size, h->Kp, st));
-  GemmEpilogue ep;
-  ep.mode = EPI_PATCH; ep.out0 = t.x_in[0]; ep.resid = h->pos_v; ep.ldc = t.d; ep.patch_np = np; ep.patch_L = t.L;
-  CK(h, gemm_bf16_tn(h->patches, h->Kp, h->w_conv, h->Kp, ep, B * np, t.d, h->Kp, st));
-  CK(h, write_cls_rows(t.x_in[0], h->cls, h->pos_v, B, t.L, t.d, st));
-  // ln_pre in place (:541); the prompt rows are overwritten by the layer-0 splice with
-  // prompts[0] = ln_pre(visual_ctx + shared_ctx), which is identical for every image
-  CK(h, layernorm_fwd(t.x_in[0], h->ln_pre_g, h->ln_pre_b, t.x_in[0], false, B * t.L, t.d, kLnEps, st));
-  if (h->ln_fused == 1 || (h->ln_fused < 0 && B * t.L >= 32768))  // (the rule of tower_forward)
-    CK(h, rowstats(t.x_in[0], t.xb_in[0], t.st_in[0], B * t.L, t.d, st));  // tower input as fp32 + bf16 + statistics
+  if (ensure_input(h, t, B, t.row0 + t.n_ctx) || ensure_train(h, t, st)) return -1;
+  if (vision_stem(h, images, B, t.patches, t.x_in[0], t.xb_in[0], t.st_in[0], st)) return -1;
   t.sel_rows = nullptr;  // CLS row (clip/model.py:548)
-  if (tower_forward(h, t, prompts, 0, st)) return -1;
+  FwdView v;
+  if (tower_forward_train(h, t, prompts, 0, st, v)) return -1;
   const int* rows; int Lh;
-  const float* xh = tower_head_input(t, &rows, &Lh);
-  CK(h, feature_head_fwd(xh, rows, h->ln_post_g, h->ln_post_b, h->proj_v, f_img, t.head_ws, B, Lh, t.d, c.embed_dim, kLnEps, st));
+  const float* xh = tower_head_input(t, v, &rows, &Lh);
+  CK(h, feature_head_fwd(xh, rows, h->ln_post_g, h->ln_post_b, h->proj_v, f_img, v.head_ws, B, Lh, t.d, h->cfg.embed_dim, kLnEps, st));
+  return 0;
+}
+
+int mudpt_vision_infer(mudpt_handle* h, const float* images, int32_t B, const float* prompts, float* f_img, void* stream) {
+  if (!h || !images || !f_img || (!prompts && h->cfg.n_ctx > 0)) return fail(h, "mudpt_vision_infer: null argument");
+  if (B <= 0) return fail(h, "mudpt_vision_infer: empty batch");
+  if (mudpt_weights_complete(h)) return -1;
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  Tower& t = h->vis;
+  const int M = B * t.L;
+  if (ensure_infer(h, t, B, M, ln_fused_for(h, t, M), st)) return -1;
+  FwdView& v = t.inf.v;
+  v.S = B; v.rows = M; v.attn_sq = static_cast<double>(B) * t.L * t.L;
+  if (vision_stem(h, images, B, t.inf.patches, v.x_in[0], v.xb_in[0], v.st_in[0], st)) return -1;
+  if (tower_forward(h, t, v, prompts, 0, st)) return -1;
+  const int* rows; int Lh;
+  const float* xh = tower_head_input(t, v, &rows, &Lh);
+  CK(h, feature_head_fwd(xh, rows, h->ln_post_g, h->ln_post_b, h->proj_v, f_img, v.head_ws, B, Lh, t.d, h->cfg.embed_dim, kLnEps, st));
   return 0;
 }
 
@@ -887,12 +1054,8 @@ int mudpt_text_set_classes(mudpt_handle* h, const float* embeddings, int32_t C, 
   cudaSetDevice(c.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Tower& t = h->txt;
-  if (ensure_tower(h, t, C, seq_len)) return -1;
-  if (static_cast<size_t>(C) > h->eot_cap) {
-    CUDA_OK(h, dev_alloc(h, &h->eot, static_cast<size_t>(C)));
-    h->eot_cap = C;
-  }
-  CUDA_OK(h, cudaMemcpyAsync(h->eot, eot_host, C * sizeof(int), cudaMemcpyHostToDevice, st));
+  if (ensure_input(h, t, C, seq_len)) return -1;
+  CUDA_OK(h, cudaMemcpyAsync(t.eot, eot_host, C * sizeof(int), cudaMemcpyHostToDevice, st));
   CUDA_OK(h, cudaStreamSynchronize(st));  // eot_host may be freed by the caller after return
   CK(h, add_positional(t.x_in[0], embeddings, h->pos_t, C, seq_len, src_len, t.d, st));
   CK(h, rowstats(t.x_in[0], t.xb_in[0], t.st_in[0], C * seq_len, t.d, st));  // (the prompt rows are rewritten every step)
@@ -929,20 +1092,8 @@ int mudpt_text_set_classes_ragged(mudpt_handle* h, const float* embeddings, int3
   std::vector<int> pos(M);
   for (int i = 0; i < C; ++i)
     for (int j = 0; j < len_host[i]; ++j) pos[off[i] + j] = j;
-  if (ensure_tower(h, t, C, max_len, off.data())) return -1;
-  if (static_cast<size_t>(C) > h->eot_cap) {
-    CUDA_OK(h, dev_alloc(h, &h->eot, static_cast<size_t>(C)));
-    h->eot_cap = C;
-  }
-  if (static_cast<size_t>(C) + 1 > t.off_cap) {
-    CUDA_OK(h, dev_alloc(h, &t.seq_off, static_cast<size_t>(C) + 1));
-    t.off_cap = static_cast<size_t>(C) + 1;
-  }
-  if (static_cast<size_t>(M) > t.pos_cap) {
-    CUDA_OK(h, dev_alloc(h, &t.tok_pos, static_cast<size_t>(M)));
-    t.pos_cap = M;
-  }
-  CUDA_OK(h, cudaMemcpyAsync(h->eot, sel.data(), C * sizeof(int), cudaMemcpyHostToDevice, st));
+  if (ensure_input(h, t, C, max_len, off.data())) return -1;
+  CUDA_OK(h, cudaMemcpyAsync(t.eot, sel.data(), C * sizeof(int), cudaMemcpyHostToDevice, st));
   CUDA_OK(h, cudaMemcpyAsync(t.seq_off, off.data(), (C + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
   CUDA_OK(h, cudaMemcpyAsync(t.tok_pos, pos.data(), M * sizeof(int), cudaMemcpyHostToDevice, st));
   CUDA_OK(h, cudaStreamSynchronize(st));  // (the host vectors go out of scope)
@@ -955,15 +1106,63 @@ int mudpt_text_forward(mudpt_handle* h, const float* prompts, int32_t splice_lay
   if (!h || !f_txt || (!prompts && h->cfg.n_ctx > 0)) return fail(h, "mudpt_text_forward: null argument");
   if (mudpt_weights_complete(h)) return -1;
   Tower& t = h->txt;
-  if (t.cap_rows == 0 || t.S <= 0) return fail(h, "mudpt_text_forward: call mudpt_text_set_classes first");
+  if (t.in_rows == 0 || t.S <= 0) return fail(h, "mudpt_text_forward: call mudpt_text_set_classes first");
   cudaSetDevice(h->cfg.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  t.sel_rows = h->eot;  // EOT row (trainers/mudpt.py:154)
-  if (tower_forward(h, t, prompts, splice_layer0 ? 0 : 1, st)) return -1;
+  if (ensure_train(h, t, st)) return -1;
+  t.sel_rows = t.eot;  // EOT row (trainers/mudpt.py:154)
+  FwdView v;
+  if (tower_forward_train(h, t, prompts, splice_layer0 ? 0 : 1, st, v)) return -1;
   const int* rows; int Lh;
-  const float* xh = tower_head_input(t, &rows, &Lh);
-  CK(h, feature_head_fwd(xh, rows, h->ln_final_g, h->ln_final_b, h->proj_t, f_txt, t.head_ws, t.S, Lh, t.d, h->cfg.embed_dim, kLnEps, st));
+  const float* xh = tower_head_input(t, v, &rows, &Lh);
+  CK(h, feature_head_fwd(xh, rows, h->ln_final_g, h->ln_final_b, h->proj_t, f_txt, v.head_ws, t.S, Lh, t.d, h->cfg.embed_dim, kLnEps, st));
   t.first_splice = splice_layer0 ? 0 : 1;  // the backward must mirror the forward's splice set
+  return 0;
+}
+
+int mudpt_text_infer(mudpt_handle* h, const float* prompts, int32_t splice_layer0, float* f_txt, void* stream) {
+  if (!h || !f_txt || (!prompts && h->cfg.n_ctx > 0)) return fail(h, "mudpt_text_infer: null argument");
+  if (mudpt_weights_complete(h)) return -1;
+  Tower& t = h->txt;
+  if (t.in_rows == 0 || t.S <= 0) return fail(h, "mudpt_text_infer: call mudpt_text_set_classes first");
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool fused = ln_fused_for(h, t, t.rows);
+  if (ensure_infer(h, t, t.S, t.rows, fused, st)) return -1;
+  FwdView& v = t.inf.v;
+  v.S = t.S; v.rows = t.rows; v.attn_sq = t.attn_sq;
+  // The walk splices the layer-0 prompt rows into its input in place.  The class set's input belongs to the training walk
+  // (its backward reads those rows again), so with a layer-0 splice this walk starts from a copy in its own residual buffer.
+  if (splice_layer0 && t.n_ctx > 0 && t.layers > 0) {
+    const size_t n = static_cast<size_t>(t.rows) * t.d;
+    v.x_in[0] = v.x_in[t.layers];
+    v.xb_in[0] = v.xb_in[t.layers];
+    v.st_in[0] = v.st_in[t.layers];
+    CUDA_OK(h, cudaMemcpyAsync(v.x_in[0], t.x_in[0], n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (fused) {
+      CUDA_OK(h, cudaMemcpyAsync(v.xb_in[0], t.xb_in[0], n * sizeof(bf16), cudaMemcpyDeviceToDevice, st));
+      CUDA_OK(h, cudaMemcpyAsync(v.st_in[0], t.st_in[0], n / 64 * sizeof(float2), cudaMemcpyDeviceToDevice, st));
+    }
+  } else {  // read only
+    v.x_in[0] = t.x_in[0];
+    v.xb_in[0] = t.xb_in[0];
+    v.st_in[0] = t.st_in[0];
+  }
+  t.sel_rows = t.eot;
+  if (tower_forward(h, t, v, prompts, splice_layer0 ? 0 : 1, st)) return -1;
+  const int* rows; int Lh;
+  const float* xh = tower_head_input(t, v, &rows, &Lh);
+  CK(h, feature_head_fwd(xh, rows, h->ln_final_g, h->ln_final_b, h->proj_t, f_txt, v.head_ws, t.S, Lh, t.d, h->cfg.embed_dim, kLnEps, st));
+  return 0;
+}
+
+int mudpt_workspace_bytes(mudpt_handle* h, int32_t tower, int32_t kind, int64_t* bytes) {
+  if (!h || !bytes) return fail(h, "mudpt_workspace_bytes: null argument");
+  if (tower != MUDPT_TOWER_VISION && tower != MUDPT_TOWER_TEXT) return fail(h, "mudpt_workspace_bytes: bad tower %d", tower);
+  Tower& t = tower == MUDPT_TOWER_VISION ? h->vis : h->txt;
+  const AllocGroup* g = kind == 0 ? &t.train_mem : kind == 1 ? &t.inf.mem : kind == 2 ? &t.in_mem : nullptr;
+  if (!g) return fail(h, "mudpt_workspace_bytes: kind must be 0 (training workspace), 1 (inference workspace) or 2 (tower input)");
+  *bytes = static_cast<int64_t>(g->bytes);
   return 0;
 }
 

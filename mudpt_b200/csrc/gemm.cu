@@ -68,9 +68,12 @@ template <int MODE> struct GemmThreads { static constexpr int value = 64 + 32 * 
 // 64B-swizzled (bf16) or 4 KB 128B-swizzled (fp32) staging boxes.  Only the patch-embedding scatter keeps the
 // transposing epilogue below.
 template <int MODE> struct RowEpi { static constexpr bool value = (MODE != EPI_PATCH); };
-template <int MODE> struct LnFwd { static constexpr bool value = (MODE == EPI_LN_BF16 || MODE == EPI_LN_GELU); };
+template <int MODE> struct LnFwd { static constexpr bool value = (MODE == EPI_LN_BF16 || MODE == EPI_LN_GELU || MODE == EPI_LN_GELU_ONLY); };
+// two bf16 outputs (h and QuickGELU(h))
 template <int MODE> struct GeluFwd { static constexpr bool value = (MODE == EPI_GELU || MODE == EPI_LN_GELU); };
-template <int MODE> struct Bf16Fwd { static constexpr bool value = (MODE == EPI_BF16 || MODE == EPI_LN_BF16); };
+// one bf16 output: the fused value, or its QuickGELU (GeluOnly)
+template <int MODE> struct GeluOnly { static constexpr bool value = (MODE == EPI_GELU_ONLY || MODE == EPI_LN_GELU_ONLY); };
+template <int MODE> struct Bf16Fwd { static constexpr bool value = (MODE == EPI_BF16 || MODE == EPI_LN_BF16 || GeluOnly<MODE>::value); };
 // fp32 output box with an optional second (bf16) box: residual + statistics, LayerNorm backward
 template <int MODE> struct DualEpi { static constexpr bool value = (MODE == EPI_RESID_STATS || MODE == EPI_LN_BWD); };
 template <int MODE> struct F32Epi { static constexpr bool value = (MODE == EPI_F32 || MODE == EPI_RESID_F32 || DualEpi<MODE>::value); };
@@ -462,7 +465,10 @@ __device__ __forceinline__ void epilogue_rows(const EpiMaps mp, const GemmEpilog
         for (int j = 0; j < 4; ++j) {
           uint32_t o[4];
 #pragma unroll
-          for (int q = 0; q < 4; ++q) o[q] = pack_bf16_2(value(8 * j + 2 * q));
+          for (int q = 0; q < 4; ++q) {
+            if constexpr (GeluOnly<MODE>::value) o[q] = pack_bf16_2(quick_gelu2(value(8 * j + 2 * q)));  // (as out1 of the GELU modes)
+            else o[q] = pack_bf16_2(value(8 * j + 2 * q));
+          }
           *reinterpret_cast<uint4*>(u + unit_slot(lane, j)) = make_uint4(o[0], o[1], o[2], o[3]);
         }
         fence_proxy_async_smem();
@@ -1351,12 +1357,20 @@ const char* gemm_bf16_tn(const bf16* A, int lda, const bf16* B, int ldb, const G
       if (ep.resid == nullptr) return "gemm: EPI_RESID_F32 needs a residual";
       return launch_mode<EPI_RESID_F32>(A, lda, B, ldb, ep, M, N, K, stream, ws);
     case EPI_GELU: return launch_mode<EPI_GELU>(A, lda, B, ldb, ep, M, N, K, stream, ws);
+    case EPI_GELU_ONLY:
+      if (ep.out0 == nullptr) return "gemm: EPI_GELU_ONLY needs out0";
+      return launch_mode<EPI_GELU_ONLY>(A, lda, B, ldb, ep, M, N, K, stream, ws);
     case EPI_GELU_BWD: return launch_mode<EPI_GELU_BWD>(A, lda, B, ldb, ep, M, N, K, stream, ws);
     case EPI_PATCH: return launch_mode<EPI_PATCH>(A, lda, B, ldb, ep, M, N, K, stream, ws);
     case EPI_LN_BF16:
     case EPI_LN_GELU:
+    case EPI_LN_GELU_ONLY:
       if (!ep.ln_stats || !ep.colsum || !ep.bias || ep.ln_parts <= 0 || ep.ln_width <= 0)
         return "gemm: fused LayerNorm needs row statistics, column sums and the folded bias";
+      if (ep.mode == EPI_LN_GELU_ONLY) {
+        if (ep.out0 == nullptr) return "gemm: EPI_LN_GELU_ONLY needs out0";
+        return launch_mode<EPI_LN_GELU_ONLY>(A, lda, B, ldb, ep, M, N, K, stream, ws);
+      }
       return ep.mode == EPI_LN_BF16 ? launch_mode<EPI_LN_BF16>(A, lda, B, ldb, ep, M, N, K, stream, ws)
                                     : launch_mode<EPI_LN_GELU>(A, lda, B, ldb, ep, M, N, K, stream, ws);
     case EPI_RESID_STATS:

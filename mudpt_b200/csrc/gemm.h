@@ -28,6 +28,9 @@ enum GemmEpilogueMode {
                         //   c1 = mean_k(g), c2 = mean_k(g*xhat) computed by the PRODUCER of the GEMM's A operand from
                         //   c1 = (1/d) sum_c dout_c colsum_c,  c2 = (1/d) sum_c dout_c (y_c - b'_c)   (y = saved LN-GEMM output)
   EPI_GELU_BWD_DOTS = 11,  // EPI_GELU_BWD + dots_out[row][col/span] = partial (sum dh*colsum, sum dh*(h - b')) for the above
+  // ---- forward-only c_fc (no backward will read the pre-activation h): one bf16 output, bitwise out1 of modes 3 / 8
+  EPI_GELU_ONLY = 12,     // out0(bf16) = QuickGELU(acc + bias)
+  EPI_LN_GELU_ONLY = 13,  // out0(bf16) = QuickGELU(rstd*(acc - mean*colsum) + bias)
 };
 
 struct GemmEpilogue {

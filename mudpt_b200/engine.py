@@ -104,7 +104,7 @@ class Engine:
         if shape is not None and tuple(t.shape) != tuple(shape):
             raise RuntimeError(f"mudpt_b200: expected shape {tuple(shape)}, got {tuple(t.shape)}")
 
-    def vision_forward(self, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
+    def _vision(self, fn, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
         a = self.arch
         R = a["image_resolution"]
         images = images.to(torch.float32).contiguous()
@@ -112,10 +112,19 @@ class Engine:
         prompts = prompts.contiguous()
         self._check_f32(prompts, (self.depth, self.n_ctx, a["vision_width"]))
         out = torch.empty(images.shape[0], a["embed_dim"], device=self.device, dtype=torch.float32)
-        _lib.check(self.lib.mudpt_vision_forward(self.h, images.data_ptr(), images.shape[0], prompts.data_ptr(),
-                                                 out.data_ptr(), _lib.stream_ptr(self.device)), self.h)
+        _lib.check(fn(self.h, images.data_ptr(), images.shape[0], prompts.data_ptr(), out.data_ptr(), _lib.stream_ptr(self.device)),
+                   self.h)
+        return out
+
+    def vision_forward(self, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
+        out = self._vision(self.lib.mudpt_vision_forward, images, prompts)
         self.vision_gen += 1
         return out
+
+    def vision_infer(self, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
+        """vision_forward's result, bitwise, from the forward-only walk: no backward state is kept or touched (a pending
+        vision_backward still differentiates the last vision_forward)."""
+        return self._vision(self.lib.mudpt_vision_infer, images, prompts)
 
     def vision_backward(self, d_f_img: torch.Tensor) -> torch.Tensor:
         d_f_img = d_f_img.contiguous()
@@ -146,17 +155,34 @@ class Engine:
         self.n_classes, self.text_len = Cn, int(seq_len)
         self.class_key = None
 
-    def text_forward(self, prompts: torch.Tensor, splice_layer0: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def _text(self, fn, prompts: torch.Tensor, splice_layer0: bool, out: Optional[torch.Tensor]) -> torch.Tensor:
         prompts = prompts.contiguous()
         self._check_f32(prompts, (self.depth, self.n_ctx, self.arch["transformer_width"]))
         if out is None:
             out = torch.empty(self.n_classes, self.arch["embed_dim"], device=self.device, dtype=torch.float32)
         else:  # caller-owned destination (e.g. a peer-mapped buffer of the head's exchange)
             self._check_f32(out, (self.n_classes, self.arch["embed_dim"]))
-        _lib.check(self.lib.mudpt_text_forward(self.h, prompts.data_ptr(), 1 if splice_layer0 else 0, out.data_ptr(),
-                                               _lib.stream_ptr(self.device)), self.h)
+        _lib.check(fn(self.h, prompts.data_ptr(), 1 if splice_layer0 else 0, out.data_ptr(), _lib.stream_ptr(self.device)), self.h)
+        return out
+
+    def text_forward(self, prompts: torch.Tensor, splice_layer0: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        out = self._text(self.lib.mudpt_text_forward, prompts, splice_layer0, out)
         self.text_gen += 1
         return out
+
+    def text_infer(self, prompts: torch.Tensor, splice_layer0: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """text_forward's result, bitwise, from the forward-only walk (see vision_infer)."""
+        return self._text(self.lib.mudpt_text_infer, prompts, splice_layer0, out)
+
+    WORKSPACE_KINDS = {"train": 0, "infer": 1, "input": 2}
+
+    def workspace_bytes(self, tower: str, kind: str) -> int:
+        """Device bytes the handle holds for tower "vision" / "text": kind "train" (training workspace), "infer" (inference
+        workspace) or "input" (the tower input: class set or stem output)."""
+        b = C.c_int64()
+        t = {"vision": 0, "text": 1}[tower]
+        _lib.check(self.lib.mudpt_workspace_bytes(self.h, t, self.WORKSPACE_KINDS[kind], C.byref(b)), self.h)
+        return int(b.value)
 
     def text_backward(self, d_f_txt: torch.Tensor, want_dx0: bool = False):
         d_f_txt = d_f_txt.contiguous()
@@ -368,7 +394,8 @@ class TextTowerDenseFn(torch.autograd.Function):
     prompt embeddings [C, L, width] in, dense gradient out."""
 
     @staticmethod
-    def forward(ctx, engine: Engine, prompts_full, eot, deep_prompts, seq_len, lengths=None):
+    def setup(engine: Engine, prompts_full, eot, deep_prompts, seq_len, lengths=None) -> torch.Tensor:
+        """Registers the per-class prompt embeddings as the class set; returns the prompt stack of the tower call."""
         if lengths is None:  # (engine stand-ins without the ragged form take three arguments)
             engine.text_set_classes(prompts_full.detach(), eot, seq_len)
         else:
@@ -377,6 +404,11 @@ class TextTowerDenseFn(torch.autograd.Function):
         P = torch.zeros(engine.depth, engine.n_ctx, w, device=engine.device, dtype=torch.float32)
         if engine.depth > 1:
             P[1:] = deep_prompts.detach()
+        return P
+
+    @staticmethod
+    def forward(ctx, engine: Engine, prompts_full, eot, deep_prompts, seq_len, lengths=None):
+        P = TextTowerDenseFn.setup(engine, prompts_full, eot, deep_prompts, seq_len, lengths)
         out = engine.text_forward(P, False)
         ctx.engine, ctx.gen = engine, engine.text_gen
         ctx.full_len = prompts_full.shape[1]
@@ -391,6 +423,32 @@ class TextTowerDenseFn(torch.autograd.Function):
         d_full = torch.zeros(dx0.shape[0], ctx.full_len, dx0.shape[2], device=dx0.device, dtype=dx0.dtype)
         d_full[:, :dx0.shape[1]] = dx0  # positions past seq_len are dead under the causal mask
         return None, d_full, None, dP[1:], None, None
+
+
+# Tower calls of the modules: the training forward (activations kept for a backward) only when the result can be
+# differentiated, else the forward-only walk -- the same values bitwise, no backward workspace, and a pending backward
+# of an earlier training forward stays valid.  (Engine stand-ins without the forward-only entry points take the
+# training forward.)
+def _differentiable(*inputs) -> bool:
+    return torch.is_grad_enabled() and any(x.requires_grad for x in inputs)
+
+
+def vision_tower(engine: Engine, images, prompts) -> torch.Tensor:
+    if _differentiable(prompts) or not hasattr(engine, "vision_infer"):
+        return VisionTowerFn.apply(engine, images, prompts)
+    return engine.vision_infer(images, prompts.detach())
+
+
+def text_tower(engine: Engine, prompts) -> torch.Tensor:
+    if _differentiable(prompts) or not hasattr(engine, "text_infer"):
+        return TextTowerFn.apply(engine, prompts)
+    return engine.text_infer(prompts.detach(), True)
+
+
+def text_tower_dense(engine: Engine, prompts_full, eot, deep_prompts, seq_len, lengths=None) -> torch.Tensor:
+    if _differentiable(prompts_full, deep_prompts) or not hasattr(engine, "text_infer"):
+        return TextTowerDenseFn.apply(engine, prompts_full, eot, deep_prompts, seq_len, lengths)
+    return engine.text_infer(TextTowerDenseFn.setup(engine, prompts_full, eot, deep_prompts, seq_len, lengths), False)
 
 
 class LogitsFn(torch.autograd.Function):

@@ -24,7 +24,7 @@ import torch
 from torch import nn
 
 from .. import clip
-from ..engine import TextTowerDenseFn, text_lengths
+from ..engine import text_lengths, text_tower_dense
 from .mudpt import (TRAINER_REGISTRY, TrainerX, apply_freeze_rule, build_lr_scheduler, build_optimizer, load_pretrained_weights,
                     restore_checkpoints)
 
@@ -63,7 +63,7 @@ class TextEncoder(nn.Module):
         eot = tokenized_prompts.argmax(dim=-1).cpu()
         seq_len, lengths = text_lengths(eot, self.truncate_to_eot, prompts.shape[1], 1 + engine.n_ctx)
         deep = torch.zeros(0, 0, prompts.shape[-1], device=prompts.device)
-        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep, seq_len, lengths)
+        return text_tower_dense(engine, prompts.float(), eot, deep, seq_len, lengths)
 
 
 class PromptLearner(nn.Module):

@@ -27,7 +27,8 @@ import torch.nn.functional as F
 
 from .. import clip
 from .. import dist as mdist
-from ..engine import prompt_algebra_forward, prompt_algebra_backward, text_lengths, LogitsFn, PromptAlgebraFn, TextTowerDenseFn, TextTowerFn, VisionTowerFn
+from ..engine import (prompt_algebra_forward, prompt_algebra_backward, text_lengths, text_tower, text_tower_dense, vision_tower, LogitsFn,
+                      PromptAlgebraFn)
 
 try:  # the Dassl engine is not in the reference tree nor in this image (SURVEY.md section 2 row 13)
     from dassl.engine import TRAINER_REGISTRY, TrainerX
@@ -253,7 +254,7 @@ class TextEncoder(nn.Module):
         engine = self._clip_ref[0].engine(prompts.device)
         eot = tokenized_prompts.argmax(dim=-1).cpu()
         seq_len, lengths = text_lengths(eot, self.truncate_to_eot, prompts.shape[1], 1 + engine.n_ctx)
-        return TextTowerDenseFn.apply(engine, prompts.float(), eot, deep_prompts.float(), seq_len, lengths)
+        return text_tower_dense(engine, prompts.float(), eot, deep_prompts.float(), seq_len, lengths)
 
 
 class CustomCLIP(nn.Module):
@@ -360,8 +361,8 @@ class CustomCLIP(nn.Module):
             self._cached_text_features = None  # an optimizer step may follow: evaluation must recompute the text features
         self._register_classes(device)
         P_v, P_t = self.prompt_stacks()
-        image_features = VisionTowerFn.apply(eng, image.type(self.dtype), P_v)
-        text_features = TextTowerFn.apply(eng, P_t)
+        image_features = vision_tower(eng, image.type(self.dtype), P_v)
+        text_features = text_tower(eng, P_t)
         if self.shard_classes and mdist.world_size() > 1:
             text_features = mdist.AllGatherRows.apply(text_features, self.mudpt_prompt_learner.n_cls)
         return LogitsFn.apply(eng, image_features, text_features)
@@ -512,7 +513,7 @@ class CustomCLIP(nn.Module):
         eng = self._engine(device)
         self._register_classes(device)
         _, P_t = self.prompt_stacks()
-        f = eng.text_forward(P_t, True)
+        f = text_tower(eng, P_t)
         if self.shard_classes and mdist.world_size() > 1:
             f = mdist.all_gather_rows(f, self.mudpt_prompt_learner.n_cls)
         self._cached_text_features = f
@@ -525,7 +526,7 @@ class CustomCLIP(nn.Module):
             self.cache_text_features(image.device)
         eng = self._engine(image.device)
         P_v, _ = self.prompt_stacks()
-        f_img = eng.vision_forward(image.type(self.dtype), P_v)
+        f_img = vision_tower(eng, image.type(self.dtype), P_v)
         logits, _, _, _ = eng.logits_head(f_img, self._cached_text_features, None, 1.0, False)
         return logits
 
