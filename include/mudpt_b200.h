@@ -10,6 +10,8 @@
  *   CustomCLIP.forward (normalise + logits) .. trainers/mudpt.py:170-184
  *   F.cross_entropy + loss.backward() ........ trainers/mudpt.py:249-251 (dgrad only: every
  *                                              CLIP weight is frozen, :205-212)
+ *   d loss / d image ......................... the same backward continued through the stem to the
+ *                                              pixels (mudpt_vision_backward_images)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer unless the name ends in _host; fp32 unless noted;
@@ -97,6 +99,19 @@ int mudpt_vision_forward(mudpt_handle* h, const float* images, int32_t B, const 
 /* d_f_img [B, embed_dim] -> d_prompts [depth, n_ctx, vision_width] (summed over the batch).
  * Must follow mudpt_vision_forward on the same handle (uses its saved activations). */
 int mudpt_vision_backward(mudpt_handle* h, const float* d_f_img, float* d_prompts, void* stream);
+/* Image gradients (adversarial evaluation / training, saliency): d_f_img [B, embed_dim] ->
+ *   d_images  [B, 3, R, R], required: the gradient w.r.t. the images passed to the last mudpt_vision_forward (the
+ *             tensor as given, i.e. after the caller's pixel normalisation);
+ *   d_prompts [depth, n_ctx, vision_width] as mudpt_vision_backward, or NULL (not computed).
+ * The tower backward runs densely down to its input (no work skipping below block 0, fp32 gradient stream), then the stem
+ * backward: the patch rows before ln_pre are recomputed from the kept patches, ln_pre's dgrad, the patch dgrad GEMM against
+ * conv1.weight and the inverse im2col.  With the options prune = 0 and grad_stream_bf16 = 0, d_prompts equals that of
+ * mudpt_vision_backward bit for bit.  Must follow mudpt_vision_forward (not mudpt_vision_infer) with no mudpt_set_option
+ * in between; may be repeated.  The first call may allocate (reported under mudpt_workspace_bytes kind 0; nothing for
+ * callers that never ask for image gradients); CUDA-graph capturable after it.  For sequences over 128 tokens the
+ * attention backward takes rowsum(dO O) from the bf16 O (DESIGN.md section 9): image gradients share that error with
+ * the prompt gradients on rows dominated by an attention sink. */
+int mudpt_vision_backward_images(mudpt_handle* h, const float* d_f_img, float* d_prompts, float* d_images, void* stream);
 
 /* ---- text tower: TextEncoder.forward (trainers/mudpt.py:142-156) -------------------------------
  * Class set-up (once per class list): embeddings [C, src_len, width] are the token embeddings of the
@@ -138,7 +153,8 @@ int mudpt_text_backward(mudpt_handle* h, const float* d_f_txt, float* d_prompts,
 int mudpt_vision_infer(mudpt_handle* h, const float* images, int32_t B, const float* prompts, float* f_img, void* stream);
 int mudpt_text_infer(mudpt_handle* h, const float* prompts, int32_t splice_layer0, float* f_txt, void* stream);
 /* Device bytes the handle holds for `tower` (MUDPT_TOWER_*): kind 0 = training workspace (allocated at the first
- * mudpt_*_forward), 1 = inference workspace (first mudpt_*_infer), 2 = tower input (class set / vision stem output).
+ * mudpt_*_forward; vision: plus what the first mudpt_vision_backward_images adds), 1 = inference workspace (first
+ * mudpt_*_infer), 2 = tower input (class set / vision stem output).
  * Requested sizes: each allocation carries 256 B of slack besides. */
 int mudpt_workspace_bytes(mudpt_handle* h, int32_t tower, int32_t kind, int64_t* bytes);
 
@@ -241,6 +257,9 @@ int mudpt_attention_backward_dots(const uint16_t* qkv, const uint16_t* o, const 
  * 129..256 tokens: the vision tower), 2 = every sequence of up to 256 tokens.  Process-wide (tests, A/B runs). */
 int mudpt_set_attention_tc(int32_t mode);
 int mudpt_im2col(const float* images, uint16_t* patches, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream);
+/* inverse index map of mudpt_im2col, fp32: patches [B * (R/patch)^2, ld] -> images [B, 3, R, R]; every image element is
+ * written exactly once (stride = kernel size: a permutation), columns >= 3 * patch^2 are not read */
+int mudpt_col2im(const float* patches, float* images, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream);
 int mudpt_cast_bf16(const float* in, uint16_t* out, int64_t numel, void* stream);
 
 /* ---- own collectives over NVLink peer memory for the head's exchange (replaces the all_gather / reduce_scatter that

@@ -238,7 +238,7 @@ class VisionTransformer_UUMuDPT(nn.Module):
 
 class VisionTransformer(nn.Module):
     """Plain ViT tower without image prompts (clip/model.py:443-496, cfg=None): same parameter names;
-    forward(x) -> image features through the native tower (no trainable tensor inside: forward only)."""
+    forward(x) -> image features through the native tower (no trainable tensor inside: differentiable w.r.t. x only)."""
 
     def __init__(self, input_resolution: int, patch_size: int, width: int, layers: int, heads: int, output_dim: int, cfg=None):
         super().__init__()
@@ -258,8 +258,8 @@ class VisionTransformer(nn.Module):
     def forward(self, x: torch.Tensor):
         engine = self._owner().engine(x.device)
         empty = torch.zeros(engine.depth, 0, self.conv1.weight.shape[0], device=x.device, dtype=torch.float32)
-        with torch.no_grad():  # the tower is frozen and carries no prompts: nothing to differentiate
-            return vision_tower(engine, x, empty)
+        # the tower is frozen and carries no prompts: the forward-only walk unless x itself requires a gradient
+        return vision_tower(engine, x, empty)
 
 
 class CLIP(nn.Module):

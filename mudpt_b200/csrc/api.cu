@@ -1,5 +1,5 @@
 // C ABI of libmudpt_b200.so (include/mudpt_b200.h): handle, frozen-weight conversion, tower
-// forward / dgrad-only backward orchestration.  All launches go to the caller's stream; no
+// forward / dgrad-only backward orchestration (to the prompts, and through the vision stem to the images).  All launches go to the caller's stream; no
 // device synchronisation happens here (except the one-time read of logit_scale in set_weight).
 #include "../../include/mudpt_b200.h"
 
@@ -130,6 +130,12 @@ struct Tower {
   bf16 *p0_dqkv = nullptr, *p0_a = nullptr, *p0_dxb = nullptr;
   float *p0_x = nullptr, *p0_dx = nullptr;
   GemmWorkspace gws;             // stream-K scratch of this tower's stream
+  // image gradients (mudpt_vision_backward_images): what the stem backward cannot keep in the backward transients that are
+  // free after block 0 -- allocated at the first such call, reported with the training workspace (DESIGN.md section 3)
+  AllocGroup img_mem;
+  size_t img_S = 0;
+  float* img_dpatch = nullptr;   // [S * np, Kp] fp32 patch gradient, where it does not fit in g_buf
+  float* img_dprompt = nullptr;  // [depth, n_ctx, d]: the splice backward's sink when no prompt gradient is asked for
   bool fwd_done = false;
   bool fwd_fused = false;  // the saved activations belong to the fused-LayerNorm formulation
   int first_splice = 0;  // 0: layer 0 splices prompts[0]; 1: layer-0 rows kept as given
@@ -168,6 +174,7 @@ struct mudpt_handle {
   Tower vis, txt;
   // vision stem / heads
   bf16* w_conv = nullptr;  // [dv, Kp] bf16 (Kp = 3*p*p padded to a multiple of 8)
+  bf16* w_conv_t = nullptr;  // [Kp, dv] transposed copy: B operand of the patch dgrad (padding rows zero)
   int Kp = 0;
   float *cls = nullptr, *pos_v = nullptr, *ln_pre_g = nullptr, *ln_pre_b = nullptr, *ln_post_g = nullptr,
         *ln_post_b = nullptr, *proj_v = nullptr;
@@ -904,7 +911,7 @@ void mudpt_destroy(mudpt_handle* h) {
   cudaSetDevice(h->cfg.device);
   for (void* p : h->allocs) cudaFree(p);
   for (Tower* t : {&h->vis, &h->txt})
-    for (AllocGroup* g : {&t->in_mem, &t->train_mem, &t->inf.mem})
+    for (AllocGroup* g : {&t->in_mem, &t->train_mem, &t->inf.mem, &t->img_mem})
       for (void* p : g->ptrs) cudaFree(p);
   for (ProfRec& r : h->prof.recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
   for (cudaEvent_t e : h->prof.pool) cudaEventDestroy(e);
@@ -946,6 +953,11 @@ int mudpt_set_weight(mudpt_handle* h, const char* name, const float* data, int64
     } else {  // padded rows (ViT-L/14: 588 -> 592)
       for (int r = 0; r < dv; ++r) CK(h, cast_to_bf16(data + static_cast<size_t>(r) * k, h->w_conv + static_cast<size_t>(r) * h->Kp, k, st));
     }
+    // [k, dv] transposed + (Kp - k) zero rows
+    if (!h->w_conv_t) CUDA_OK(h, dev_alloc(h, &h->w_conv_t, static_cast<size_t>(h->Kp) * dv));
+    if (h->Kp != k)
+      CUDA_OK(h, cudaMemsetAsync(h->w_conv_t + static_cast<size_t>(k) * dv, 0, static_cast<size_t>(h->Kp - k) * dv * sizeof(bf16), st));
+    CK(h, transpose_cast_bf16(data, h->w_conv_t, dv, k, st));
     h->stem_have |= SB_CONV; rc = 0;
   } else if (!strcmp(name, "visual.class_embedding")) { rc = store_f32(h, &h->cls, data, numel, dv, name, st); h->stem_have |= SB_CLS; }
   else if (!strcmp(name, "visual.positional_embedding")) { rc = store_f32(h, &h->pos_v, data, numel, static_cast<int64_t>(np + 1) * dv, name, st); h->stem_have |= SB_POS_V; }
@@ -1039,6 +1051,65 @@ int mudpt_vision_backward(mudpt_handle* h, const float* d_f_img, float* d_prompt
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (head_backward(h, t, d_f_img, h->ln_post_g, h->proj_v, st)) return -1;
   return tower_backward(h, t, d_prompts, 0, st);
+}
+
+// The fp32 patch gradient [S * np, Kp] goes to g_buf (the forward's QuickGELU transient, which no backward reads) where it
+// fits: per image L * 4d bf16 against np * Kp fp32 -- ViT-B/16 and ViT-L/14 yes, ViT-B/32 (Kp = 4d) no.
+static bool dpatch_in_g_buf(const mudpt_handle* h) {
+  const Tower& t = h->vis;
+  return static_cast<size_t>(t.row0 - 1) * h->Kp * sizeof(float) <= static_cast<size_t>(t.L) * 4 * t.d * sizeof(bf16);
+}
+
+// Image-gradient memory beyond the training workspace (Tower::img_mem), for the tower's current batch
+static int ensure_image_grad(mudpt_handle* h, Tower& t) {
+  if (static_cast<size_t>(t.S) <= t.img_S) return 0;  // (img_S = 0 until the first call)
+  release(t.img_mem);
+  t.img_S = t.S;
+  t.img_dpatch = t.img_dprompt = nullptr;
+  AllocGroup* g = &t.img_mem;
+  if (!dpatch_in_g_buf(h)) CUDA_OK(h, dev_alloc(h, &t.img_dpatch, t.img_S * (t.row0 - 1) * h->Kp, g));
+  if (t.n_ctx > 0) CUDA_OK(h, dev_alloc(h, &t.img_dprompt, static_cast<size_t>(t.depth) * t.n_ctx * t.d, g));
+  return 0;
+}
+
+// Backward of the stem (vision_stem) into the images, on the patch rows b * L + 1 + p: x = conv1(img) + pos, y = ln_pre(x).
+// Precondition: t.dx holds dL/dy for every row in fp32 (tower_backward with need_dx0).  The CLS rows (class_embedding is
+// frozen) and the prompt rows (their ln_pre belongs to the prompt algebra; their gradient went to d_prompts[0]) are dropped.
+//   1. x again from the kept bf16 patches with the forward's own patch GEMM: bitwise the rows ln_pre normalised
+//   2. ln_pre dgrad over the row map b * np + p <- b * L + 1 + p, bf16 compact rows
+//   3. patch dgrad d_patches [S * np, Kp] = dy_ln . W_conv (the transposed bf16 copy), fp32
+//   4. col2im into d_images [S, 3, R, R]
+// Scratch: x in dh_buf, dy_ln in a_buf, d_patches in g_buf or img_dpatch -- transients no one reads after block 0.
+static int stem_backward(mudpt_handle* h, float* d_images, cudaStream_t st) {
+  const mudpt_config& c = h->cfg;
+  Tower& t = h->vis;
+  const int B = t.S, np = t.row0 - 1, d = t.d, Kp = h->Kp, M = B * np;
+  const double Md = M, dd = d, Kd = Kp;
+  float* x = reinterpret_cast<float*>(t.dh_buf);
+  GemmEpilogue ep;
+  ep.mode = EPI_PATCH; ep.out0 = x; ep.resid = h->pos_v; ep.ldc = d; ep.patch_np = np; ep.patch_L = t.L;
+  CKP(h, st, PC_STEM, 2.0 * Md * dd * Kd, 2 * (Md * Kd + dd * Kd) + 8 * Md * dd, gemm_bf16_tn(t.patches, Kp, h->w_conv, Kp, ep, M, d, Kp, st));
+  CKP(h, st, PC_LN_BWD, 0, Md * dd * 10, layernorm_bwd_rows(t.dx, x, h->ln_pre_g, t.a_buf, M, d, kLnEps, np, t.L, 1, st));
+  float* dpatch = dpatch_in_g_buf(h) ? reinterpret_cast<float*>(t.g_buf) : t.img_dpatch;
+  GemmEpilogue e2;
+  e2.mode = EPI_F32; e2.out0 = dpatch; e2.ldc = Kp;
+  CKP(h, st, PC_GEMM, 2.0 * Md * Kd * dd, 2 * (Md * dd + Kd * dd) + 4 * Md * Kd, gemm_bf16_tn(t.a_buf, d, h->w_conv_t, d, e2, M, Kp, d, st, &t.gws));
+  CKP(h, st, PC_STEM, 0, 8.0 * B * 3 * c.image_resolution * c.image_resolution,
+      col2im_f32(dpatch, d_images, B, c.image_resolution, c.vision_patch_size, Kp, st));
+  return 0;
+}
+
+int mudpt_vision_backward_images(mudpt_handle* h, const float* d_f_img, float* d_prompts, float* d_images, void* stream) {
+  if (!h || !d_f_img || !d_images) return fail(h, "mudpt_vision_backward_images: null argument");
+  Tower& t = h->vis;
+  if (!t.fwd_done) return fail(h, "mudpt_vision_backward_images: no forward pass to differentiate");
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (ensure_image_grad(h, t)) return -1;
+  if (head_backward(h, t, d_f_img, h->ln_post_g, h->proj_v, st)) return -1;
+  // without d_prompts the splice backward still runs (layers > 0 zero the rows their prompts overwrote) into a sink
+  if (tower_backward(h, t, d_prompts ? d_prompts : t.img_dprompt, 0, st, /*need_dx0=*/true)) return -1;
+  return stem_backward(h, d_images, st);
 }
 
 int mudpt_text_set_classes(mudpt_handle* h, const float* embeddings, int32_t C, int32_t src_len, int32_t seq_len,
@@ -1162,7 +1233,7 @@ int mudpt_workspace_bytes(mudpt_handle* h, int32_t tower, int32_t kind, int64_t*
   Tower& t = tower == MUDPT_TOWER_VISION ? h->vis : h->txt;
   const AllocGroup* g = kind == 0 ? &t.train_mem : kind == 1 ? &t.inf.mem : kind == 2 ? &t.in_mem : nullptr;
   if (!g) return fail(h, "mudpt_workspace_bytes: kind must be 0 (training workspace), 1 (inference workspace) or 2 (tower input)");
-  *bytes = static_cast<int64_t>(g->bytes);
+  *bytes = static_cast<int64_t>(g->bytes + (kind == 0 ? t.img_mem.bytes : 0));  // (image gradients: with the training workspace)
   return 0;
 }
 
@@ -1341,6 +1412,10 @@ int mudpt_set_attention_tc(int32_t mode) {
 }
 int mudpt_im2col(const float* images, uint16_t* patches, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream) {
   CKG(im2col_bf16(images, reinterpret_cast<bf16*>(patches), B, R, patch, ld, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+int mudpt_col2im(const float* patches, float* images, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream) {
+  CKG(col2im_f32(patches, images, B, R, patch, ld, static_cast<cudaStream_t>(stream)));
   return 0;
 }
 int mudpt_peer_all_gather_rows(const void* peers_dev, int32_t world, int32_t n_total, int32_t width, float* out, void* stream) {

@@ -334,6 +334,98 @@ static void dispatch_ln_bwd(const void* dy, bool dy_bf16, const void* x, const f
   }
 }
 
+// ------------------------------------------------------------------ LayerNorm backward over a row map
+// out[r] = bf16(rstd (g - mean(g) - xhat mean(g xhat))), g = dy[src] * gamma, for the compact rows r < M, where the source
+// row is src = (r / per) * L + row0 + r % per: one block of `per` rows out of every sequence of L rows.  fp32 dy and x,
+// statistics recomputed from x, no residual.  The vision stem's ln_pre backward on the patch rows of every image (the
+// output is the A operand of the patch dgrad GEMM); the same arithmetic as ln_bwd_kernel.
+template <int NV>
+__global__ void __launch_bounds__(256) ln_bwd_rows_kernel(const float* __restrict__ dy, const float* __restrict__ x,
+                                                          const float* __restrict__ gamma, bf16* __restrict__ out, int M, int d,
+                                                          float eps, int per, int L, int row0) {
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  pdl_wait();
+  pdl_trigger();
+  if (row >= M) return;
+  const int seq = row / per;
+  const size_t src = (static_cast<size_t>(seq) * L + row0 + (row - seq * per)) * d;
+  float4 v[NV], g[NV];
+  float sum = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = (i * 32 + lane) * 4;
+    if (c < d) {
+      v[i] = *reinterpret_cast<const float4*>(x + src + c);
+      g[i] = *reinterpret_cast<const float4*>(dy + src + c);
+      sum += (v[i].x + v[i].y) + (v[i].z + v[i].w);
+    }
+  }
+  const float mean = warp_sum(sum) / d;
+  float sq = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = (i * 32 + lane) * 4;
+    if (c < d) {
+      v[i].x -= mean; v[i].y -= mean; v[i].z -= mean; v[i].w -= mean;
+      sq += (v[i].x * v[i].x + v[i].y * v[i].y) + (v[i].z * v[i].z + v[i].w * v[i].w);
+    }
+  }
+  const float rstd = rsqrtf(warp_sum(sq) / d + eps);
+  float s1 = 0.f, s2 = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = (i * 32 + lane) * 4;
+    if (c < d) {
+      const float4 gm = *reinterpret_cast<const float4*>(gamma + c);
+      v[i].x *= rstd; v[i].y *= rstd; v[i].z *= rstd; v[i].w *= rstd;  // xhat
+      g[i].x *= gm.x; g[i].y *= gm.y; g[i].z *= gm.z; g[i].w *= gm.w;
+      s1 += (g[i].x + g[i].y) + (g[i].z + g[i].w);
+      s2 += (g[i].x * v[i].x + g[i].y * v[i].y) + (g[i].z * v[i].z + g[i].w * v[i].w);
+    }
+  }
+  s1 = warp_sum(s1) / d;
+  s2 = warp_sum(s2) / d;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = (i * 32 + lane) * 4;
+    if (c < d) {
+      float4 o;
+      o.x = rstd * (g[i].x - s1 - v[i].x * s2);
+      o.y = rstd * (g[i].y - s1 - v[i].y * s2);
+      o.z = rstd * (g[i].z - s1 - v[i].z * s2);
+      o.w = rstd * (g[i].w - s1 - v[i].w * s2);
+      uint2 u;
+      u.x = pack_bf16(o.x, o.y);
+      u.y = pack_bf16(o.z, o.w);
+      *reinterpret_cast<uint2*>(out + static_cast<size_t>(row) * d + c) = u;
+    }
+  }
+}
+
+template <int NV>
+static void launch_ln_bwd_rows(const float* dy, const float* x, const float* gamma, bf16* out, int M, int d, float eps, int per,
+                               int L, int row0, cudaStream_t stream) {
+  const int wpc = ln_warps();
+  launch_pdl(ln_bwd_rows_kernel<NV>, dim3((M + wpc - 1) / wpc), dim3(32 * wpc), 0, stream, dy, x, gamma, out, M, d, eps, per, L, row0);
+}
+
+const char* layernorm_bwd_rows(const float* dy, const float* x, const float* gamma, bf16* out, int M, int d, float eps, int per,
+                               int L, int row0, cudaStream_t stream) {
+  if (M <= 0) return nullptr;
+  if (d % 4 != 0 || d > LN_MAXV * 128) return "layernorm: width must be a multiple of 4 and <= 1024";
+  if (per <= 0 || row0 < 0 || row0 + per > L) return "layernorm bwd (row map): bad geometry";
+  switch (pick_nv(d)) {
+    case 1: launch_ln_bwd_rows<1>(dy, x, gamma, out, M, d, eps, per, L, row0, stream); break;
+    case 2: launch_ln_bwd_rows<2>(dy, x, gamma, out, M, d, eps, per, L, row0, stream); break;
+    case 4: launch_ln_bwd_rows<4>(dy, x, gamma, out, M, d, eps, per, L, row0, stream); break;
+    case 6: launch_ln_bwd_rows<6>(dy, x, gamma, out, M, d, eps, per, L, row0, stream); break;
+    default: launch_ln_bwd_rows<8>(dy, x, gamma, out, M, d, eps, per, L, row0, stream); break;
+  }
+  count_launch(1);
+  return launch_status("layernorm bwd (row map) launch failed");
+}
+
 // ------------------------------------------------------------------ LayerNorm backward, shared-memory pipeline
 // The register kernel above has one row per warp in flight: measured on the bf16 gradient stream it moves 3.5 TB/s where
 // 6.5 are available (ncu: every warp waits a full DRAM round trip per row, 45 % of the warp slots, no byte in flight while
@@ -1240,6 +1332,38 @@ const char* im2col_bf16(const float* img, bf16* out, int B, int R, int p, int ld
   im2col_kernel<<<static_cast<unsigned>((total2 + 255) / 256), 256, 0, stream>>>(img, out, R, p, ldo, total2);
   count_launch(1);
   return launch_status("im2col launch failed");
+}
+
+// The inverse index map of im2col_kernel, fp32: image[b, c, py*p + iy, px*p + ix] = patches[(b*gh + py)*gw + px, (c*p + iy)*p + ix].
+// Stride equals the kernel size, so this is a permutation: every image element is written exactly once, nothing is
+// accumulated, and the padding columns >= 3*p*p of the rows are never read.  Threads walk the image (coalesced writes),
+// two consecutive ix per thread (p is even, so both lie in one patch).
+__global__ void col2im_kernel(const float* __restrict__ cols, float* __restrict__ img, int R, int p, int ldi, size_t total2) {
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  pdl_wait();
+  pdl_trigger();
+  if (i >= total2) return;
+  const size_t e = i * 2;
+  const int x = static_cast<int>(e % R);
+  const size_t r2 = e / R;
+  const int y = static_cast<int>(r2 % R);
+  const size_t bc = r2 / R;
+  const int c = static_cast<int>(bc % 3);
+  const size_t b = bc / 3;
+  const int gw = R / p;
+  const int px = x / p, ix = x - px * p, py = y / p, iy = y - py * p;
+  const size_t row = (b * gw + py) * gw + px;
+  const int col = (c * p + iy) * p + ix;
+  *reinterpret_cast<float2*>(img + e) = *reinterpret_cast<const float2*>(cols + row * ldi + col);
+}
+
+const char* col2im_f32(const float* cols, float* img, int B, int R, int p, int ldi, cudaStream_t stream) {
+  if (B <= 0) return nullptr;
+  if (R % p != 0 || p % 2 != 0 || ldi < 3 * p * p || ldi % 2 != 0) return "col2im: bad geometry";
+  const size_t total2 = static_cast<size_t>(B) * 3 * R * R / 2;
+  launch_pdl(col2im_kernel, dim3(static_cast<unsigned>((total2 + 255) / 256)), dim3(256), 0, stream, cols, img, R, p, ldi, total2);
+  count_launch(1);
+  return launch_status("col2im launch failed");
 }
 
 // ------------------------------------------------------------------ small helpers

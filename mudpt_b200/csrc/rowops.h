@@ -22,6 +22,10 @@ const char* layernorm_bwd(const void* dy, bool dy_bf16, const void* x, const flo
 const char* layernorm_bwd_stream(const void* dy, bool dy_bf16, const void* x, const float2* stats, const float* gamma,
                                  const void* resid, bool resid_bf16, float* dx, __nv_bfloat16* dx_bf16, int M, int d, float eps,
                                  int win_L, int win_row0, int win_n, cudaStream_t stream, const int* win_pos = nullptr);
+// LayerNorm dgrad of `per` rows out of every sequence of L rows, compacted: out[r] (bf16) from dy / x (fp32) at row
+// (r / per) * L + row0 + r % per, r < M; no residual (the vision stem's ln_pre on the patch rows)
+const char* layernorm_bwd_rows(const float* dy, const float* x, const float* gamma, __nv_bfloat16* out, int M, int d, float eps,
+                               int per, int L, int row0, cudaStream_t stream);
 const char* splice_fwd(float* x, const float* prompt, int S, int L, int row0, int n, int d, cudaStream_t stream);
 size_t splice_bwd_workspace_floats(int n, int d);  // must be zero-initialised once (it ends with the kernel's tickets)
 // seq_off != null: packed variable-length sequences ([S+1] device int32), sequence s's prompt rows start at seq_off[s] + row0
@@ -40,6 +44,8 @@ const char* scatter_rows_bf16(const __nv_bfloat16* src, const int* rows, int S, 
 const char* gather_rows(const float* src_f, const __nv_bfloat16* src_b, const int* rows, int S, int L, float* dst_f,
                         __nv_bfloat16* dst_b, int d, cudaStream_t stream);
 const char* im2col_bf16(const float* img, __nv_bfloat16* out, int B, int R, int p, int ldo, cudaStream_t stream);
+// inverse of im2col_bf16's index map, fp32 (patch rows of row stride ldi >= 3*p*p -> [B, 3, R, R], every element written once)
+const char* col2im_f32(const float* cols, float* img, int B, int R, int p, int ldi, cudaStream_t stream);
 const char* write_cls_rows(float* x, const float* cls, const float* pos, int S, int L, int d, cudaStream_t stream);
 // seq_off != null: packed variable-length output rows (L = the longest sequence)
 const char* add_positional(float* x0, const float* emb, const float* pos, int S, int L, int Lsrc, int d, cudaStream_t stream,

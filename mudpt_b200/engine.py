@@ -59,6 +59,7 @@ class Engine:
         _lib.check(self.lib.mudpt_create(C.byref(cfg), C.byref(h)))
         self.h = h
         self.vision_gen = 0  # generation counters: a backward must match the latest forward
+        self.vision_batch = 0  # images of the latest vision_forward
         self.text_gen = 0
         self.n_classes = 0
         self.text_len = 0
@@ -119,6 +120,7 @@ class Engine:
     def vision_forward(self, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
         out = self._vision(self.lib.mudpt_vision_forward, images, prompts)
         self.vision_gen += 1
+        self.vision_batch = out.shape[0]
         return out
 
     def vision_infer(self, images: torch.Tensor, prompts: torch.Tensor) -> torch.Tensor:
@@ -133,6 +135,20 @@ class Engine:
         _lib.check(self.lib.mudpt_vision_backward(self.h, d_f_img.data_ptr(), dP.data_ptr(),
                                                   _lib.stream_ptr(self.device)), self.h)
         return dP
+
+    def vision_backward_images(self, d_f_img: torch.Tensor, want_prompts: bool = True):
+        """(d_prompts or None, d_images [B, 3, R, R]) of the last vision_forward: the gradient w.r.t. the images as they
+        were passed in, and (want_prompts) w.r.t. the prompt stack, as vision_backward."""
+        d_f_img = d_f_img.contiguous()
+        B, R = self.vision_batch, self.arch["image_resolution"]
+        self._check_f32(d_f_img, (B, self.arch["embed_dim"]))
+        d_img = torch.empty(B, 3, R, R, device=self.device, dtype=torch.float32)
+        dP = None
+        if want_prompts:
+            dP = torch.empty(self.depth, self.n_ctx, self.arch["vision_width"], device=self.device, dtype=torch.float32)
+        _lib.check(self.lib.mudpt_vision_backward_images(self.h, d_f_img.data_ptr(), dP.data_ptr() if dP is not None else None,
+                                                         d_img.data_ptr(), _lib.stream_ptr(self.device)), self.h)
+        return dP, d_img
 
     def text_set_classes(self, embeddings: torch.Tensor, eot: torch.Tensor, seq_len: int,
                          lengths: Optional[List[int]] = None) -> None:
@@ -198,14 +214,16 @@ class Engine:
         return dP, dx0
 
     def logits_head(self, f_img, f_txt, labels: Optional[torch.Tensor], inv_global_batch: float, want_grads: bool,
-                    d_t_out: Optional[torch.Tensor] = None):
+                    d_t_out: Optional[torch.Tensor] = None, text_grad: bool = True):
+        """(logits, loss, d_f_img, d_f_txt); with want_grads and text_grad=False the text-feature gradient is not computed
+        (None)."""
         f_img, f_txt = f_img.contiguous(), f_txt.contiguous()
         B, Cn = f_img.shape[0], f_txt.shape[0]
         logits = torch.empty(B, Cn, device=self.device, dtype=torch.float32)
         loss = torch.zeros((), device=self.device, dtype=torch.float32)
         d_i = torch.empty_like(f_img) if want_grads else None
         d_t = None
-        if want_grads:
+        if want_grads and text_grad:
             if d_t_out is not None:  # caller-owned destination (peer-mapped buffer)
                 self._check_f32(d_t_out, tuple(f_txt.shape))
                 d_t = d_t_out
@@ -354,8 +372,8 @@ class PromptAlgebraFn(torch.autograd.Function):
 
 
 class VisionTowerFn(torch.autograd.Function):
-    """f_img = vision_tower(images; prompts).  Gradient flows to `prompts` only: the image and
-    every CLIP weight are frozen (trainers/mudpt.py:205-212)."""
+    """f_img = vision_tower(images; prompts).  Gradient flows to `prompts` and, when they require it, to `images` (the
+    tensor as passed in); every CLIP weight is frozen (trainers/mudpt.py:205-212)."""
 
     @staticmethod
     def forward(ctx, engine: Engine, images, prompts):
@@ -368,7 +386,13 @@ class VisionTowerFn(torch.autograd.Function):
         e = ctx.engine
         if ctx.gen != e.vision_gen:
             raise RuntimeError("mudpt_b200: vision backward does not match the latest forward (activations were overwritten)")
-        return None, None, e.vision_backward(d_out)
+        if not ctx.needs_input_grad[1]:  # prompts only
+            return None, None, e.vision_backward(d_out)
+        if not hasattr(e, "vision_backward_images"):
+            raise RuntimeError(f"mudpt_b200: the engine ({type(e).__name__}) has no vision_backward_images: it cannot "
+                               "differentiate the vision tower w.r.t. the images")
+        dP, d_img = e.vision_backward_images(d_out, want_prompts=ctx.needs_input_grad[2])
+        return None, d_img, dP
 
 
 class TextTowerFn(torch.autograd.Function):
@@ -434,7 +458,7 @@ def _differentiable(*inputs) -> bool:
 
 
 def vision_tower(engine: Engine, images, prompts) -> torch.Tensor:
-    if _differentiable(prompts) or not hasattr(engine, "vision_infer"):
+    if _differentiable(images, prompts) or not hasattr(engine, "vision_infer"):
         return VisionTowerFn.apply(engine, images, prompts)
     return engine.vision_infer(images, prompts.detach())
 

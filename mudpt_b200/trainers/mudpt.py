@@ -530,6 +530,29 @@ class CustomCLIP(nn.Module):
         logits, _, _, _ = eng.logits_head(f_img, self._cached_text_features, None, 1.0, False)
         return logits
 
+    @torch.no_grad()
+    def image_gradient(self, image, label):
+        """Fused attack step (PGD, AutoAttack, adversarial prompt tuning): (loss, logits, d_image) of the mean
+        cross-entropy over this batch w.r.t. `image` [B, 3, H, W] (the tensor as given, after pixel normalisation).
+
+        The text features are the cached ones (computed like inference() does if there are none), so no text tower and no
+        collective runs: under torchrun every rank attacks its own images.  One training vision forward with the prompts
+        detached, the logits head with `label` (the text-feature gradient is not computed) and the vision backward into
+        the images, without autograd.  `logits` are bitwise those of inference(image).
+
+        The vision forward here replaces the tower's saved activations (it moves the engine's vision generation): a
+        vision backward still pending from an earlier forward raises instead of returning wrong gradients."""
+        if self._cached_text_features is None:
+            self.cache_text_features(image.device)
+        eng = self._engine(image.device)
+        P_v, _ = self.prompt_stacks()
+        image = image.type(self.dtype)
+        f_img = eng.vision_forward(image, P_v.detach())
+        logits, loss, d_i, _ = eng.logits_head(f_img, self._cached_text_features, label, 1.0 / image.shape[0], True,
+                                               text_grad=False)
+        _, d_image = eng.vision_backward_images(d_i, want_prompts=False)
+        return loss, logits, d_image
+
 
 @TRAINER_REGISTRY.register()
 def apply_freeze_rule(model, keep):
