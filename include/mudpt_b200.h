@@ -112,6 +112,21 @@ int mudpt_vision_backward(mudpt_handle* h, const float* d_f_img, float* d_prompt
  * attention backward takes rowsum(dO O) from the bf16 O (DESIGN.md section 9): image gradients share that error with
  * the prompt gradients on rows dominated by an attention sink. */
 int mudpt_vision_backward_images(mudpt_handle* h, const float* d_f_img, float* d_prompts, float* d_images, void* stream);
+/* One l-inf PGD step (adversarial evaluation / training) on the images of the last mudpt_vision_forward, which were
+ * x_norm = (x_adv - mean) / std.  d_f_img [B, embed_dim] -> the image gradient g = dL/dx_norm as in
+ * mudpt_vision_backward_images (no prompt gradient), never written as an image, then per element, channel c:
+ *   s      = sign(g / std[c])                                  (0 for a zero quotient)
+ *   x'     = min(max(x_adv + alpha * s, x_clean - eps), x_clean + eps)
+ *   x'     = min(max(x', 0), 1)
+ *   x_adv  <- x'                                               (in place)
+ *   x_norm <- (x' - mean[c]) / std[c]
+ * x_adv, x_clean, x_norm [B, 3, R, R] (pixel space for the first two), 8-byte aligned.  Every operation is IEEE fp32
+ * without flushing subnormals: bitwise the PyTorch loop x = (x + alpha * (g / std).sign()).clamp(x_clean - eps,
+ * x_clean + eps).clamp(0, 1), whose g / std is the autograd of the normalisation.  x_norm may be the tensor the forward
+ * read.  eps finite >= 0, alpha finite > 0, std finite > 0.  Memory and CUDA-graph capture as
+ * mudpt_vision_backward_images; must follow mudpt_vision_forward; may be repeated (each call reads the same forward). */
+int mudpt_vision_pgd_step(mudpt_handle* h, const float* d_f_img, float* x_adv, const float* x_clean, float* x_norm,
+                          const float* mean_host, const float* std_host, float eps, float alpha, void* stream);
 
 /* ---- text tower: TextEncoder.forward (trainers/mudpt.py:142-156) -------------------------------
  * Class set-up (once per class list): embeddings [C, src_len, width] are the token embeddings of the
@@ -260,6 +275,11 @@ int mudpt_im2col(const float* images, uint16_t* patches, int32_t B, int32_t R, i
 /* inverse index map of mudpt_im2col, fp32: patches [B * (R/patch)^2, ld] -> images [B, 3, R, R]; every image element is
  * written exactly once (stride = kernel size: a permutation), columns >= 3 * patch^2 are not read */
 int mudpt_col2im(const float* patches, float* images, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream);
+/* the update of mudpt_vision_pgd_step alone: dpatch [B * (R/patch)^2, ld] in mudpt_col2im's layout (columns >= 3 * patch^2
+ * not read) is g = dL/dx_norm; x_adv updated in place, x_norm written, both [B, 3, R, R] */
+int mudpt_pgd_linf_update(const float* dpatch, int32_t ld, float* x_adv, const float* x_clean, float* x_norm, int32_t B,
+                          int32_t R, int32_t patch, const float* mean_host, const float* std_host, float eps, float alpha,
+                          void* stream);
 int mudpt_cast_bf16(const float* in, uint16_t* out, int64_t numel, void* stream);
 
 /* ---- own collectives over NVLink peer memory for the head's exchange (replaces the all_gather / reduce_scatter that

@@ -30,6 +30,8 @@ SIGNATURES = {
     "mudpt_vision_forward": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_vision_backward": (C.c_int, [C.c_void_p, c_f32p, c_f32p, C.c_void_p]),
     "mudpt_vision_backward_images": (C.c_int, [C.c_void_p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "mudpt_vision_pgd_step": (C.c_int, [C.c_void_p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p, C.c_void_p, C.c_float,
+                                         C.c_float, C.c_void_p]),
     "mudpt_text_set_classes": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "mudpt_text_set_classes_ragged": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mudpt_text_forward": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, c_f32p, C.c_void_p]),
@@ -67,6 +69,8 @@ SIGNATURES = {
     "mudpt_set_attention_tc": (C.c_int, [C.c_int32]),
     "mudpt_im2col": (C.c_int, [c_f32p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "mudpt_col2im": (C.c_int, [c_f32p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "mudpt_pgd_linf_update": (C.c_int, [c_f32p, C.c_int32, c_f32p, c_f32p, c_f32p, C.c_int32, C.c_int32, C.c_int32,
+                                         C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p]),
     "mudpt_cast_bf16": (C.c_int, [c_f32p, C.c_void_p, C.c_int64, C.c_void_p]),
     "mudpt_prompt_forward": (C.c_int, [C.c_void_p, C.c_void_p]),
     "mudpt_prompt_backward": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -1077,11 +1077,10 @@ static int ensure_image_grad(mudpt_handle* h, Tower& t) {
 // frozen) and the prompt rows (their ln_pre belongs to the prompt algebra; their gradient went to d_prompts[0]) are dropped.
 //   1. x again from the kept bf16 patches with the forward's own patch GEMM: bitwise the rows ln_pre normalised
 //   2. ln_pre dgrad over the row map b * np + p <- b * L + 1 + p, bf16 compact rows
-//   3. patch dgrad d_patches [S * np, Kp] = dy_ln . W_conv (the transposed bf16 copy), fp32
-//   4. col2im into d_images [S, 3, R, R]
+//   3. patch dgrad d_patches [S * np, Kp] = dy_ln . W_conv (the transposed bf16 copy), fp32, returned in *dpatch
+// The output stage (col2im for the image gradient, or the PGD update) reads *dpatch.
 // Scratch: x in dh_buf, dy_ln in a_buf, d_patches in g_buf or img_dpatch -- transients no one reads after block 0.
-static int stem_backward(mudpt_handle* h, float* d_images, cudaStream_t st) {
-  const mudpt_config& c = h->cfg;
+static int stem_backward(mudpt_handle* h, cudaStream_t st, const float** dpatch_out) {
   Tower& t = h->vis;
   const int B = t.S, np = t.row0 - 1, d = t.d, Kp = h->Kp, M = B * np;
   const double Md = M, dd = d, Kd = Kp;
@@ -1094,9 +1093,18 @@ static int stem_backward(mudpt_handle* h, float* d_images, cudaStream_t st) {
   GemmEpilogue e2;
   e2.mode = EPI_F32; e2.out0 = dpatch; e2.ldc = Kp;
   CKP(h, st, PC_GEMM, 2.0 * Md * Kd * dd, 2 * (Md * dd + Kd * dd) + 4 * Md * Kd, gemm_bf16_tn(t.a_buf, d, h->w_conv_t, d, e2, M, Kp, d, st, &t.gws));
-  CKP(h, st, PC_STEM, 0, 8.0 * B * 3 * c.image_resolution * c.image_resolution,
-      col2im_f32(dpatch, d_images, B, c.image_resolution, c.vision_patch_size, Kp, st));
+  *dpatch_out = dpatch;
   return 0;
+}
+
+// The vision backward of the last forward down to the patch gradient: head, dense tower backward, stem backward
+static int image_backward(mudpt_handle* h, const float* d_f_img, float* d_prompts, cudaStream_t st, const float** dpatch) {
+  Tower& t = h->vis;
+  if (ensure_image_grad(h, t)) return -1;
+  if (head_backward(h, t, d_f_img, h->ln_post_g, h->proj_v, st)) return -1;
+  // without d_prompts the splice backward still runs (layers > 0 zero the rows their prompts overwrote) into a sink
+  if (tower_backward(h, t, d_prompts ? d_prompts : t.img_dprompt, 0, st, /*need_dx0=*/true)) return -1;
+  return stem_backward(h, st, dpatch);
 }
 
 int mudpt_vision_backward_images(mudpt_handle* h, const float* d_f_img, float* d_prompts, float* d_images, void* stream) {
@@ -1105,11 +1113,37 @@ int mudpt_vision_backward_images(mudpt_handle* h, const float* d_f_img, float* d
   if (!t.fwd_done) return fail(h, "mudpt_vision_backward_images: no forward pass to differentiate");
   cudaSetDevice(h->cfg.device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (ensure_image_grad(h, t)) return -1;
-  if (head_backward(h, t, d_f_img, h->ln_post_g, h->proj_v, st)) return -1;
-  // without d_prompts the splice backward still runs (layers > 0 zero the rows their prompts overwrote) into a sink
-  if (tower_backward(h, t, d_prompts ? d_prompts : t.img_dprompt, 0, st, /*need_dx0=*/true)) return -1;
-  return stem_backward(h, d_images, st);
+  const mudpt_config& c = h->cfg;
+  const float* dpatch;
+  if (image_backward(h, d_f_img, d_prompts, st, &dpatch)) return -1;
+  CKP(h, st, PC_STEM, 0, 8.0 * t.S * 3 * c.image_resolution * c.image_resolution,
+      col2im_f32(dpatch, d_images, t.S, c.image_resolution, c.vision_patch_size, h->Kp, st));
+  return 0;
+}
+
+static PgdParams pgd_params(const float* mean_host, const float* std_host, float eps, float alpha) {
+  PgdParams p;
+  for (int c = 0; c < 3; ++c) { p.mean[c] = mean_host[c]; p.std[c] = std_host[c]; }
+  p.eps = eps; p.alpha = alpha;
+  return p;
+}
+
+int mudpt_vision_pgd_step(mudpt_handle* h, const float* d_f_img, float* x_adv, const float* x_clean, float* x_norm,
+                          const float* mean_host, const float* std_host, float eps, float alpha, void* stream) {
+  if (!h || !d_f_img || !x_adv || !x_clean || !x_norm || !mean_host || !std_host)
+    return fail(h, "mudpt_vision_pgd_step: null argument");
+  Tower& t = h->vis;
+  if (!t.fwd_done) return fail(h, "mudpt_vision_pgd_step: no forward pass to differentiate");
+  const PgdParams prm = pgd_params(mean_host, std_host, eps, alpha);
+  if (const char* e = pgd_linf_check(prm)) return fail(h, "mudpt_vision_pgd_step: %s", e);
+  cudaSetDevice(h->cfg.device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const mudpt_config& c = h->cfg;
+  const float* dpatch;
+  if (image_backward(h, d_f_img, nullptr, st, &dpatch)) return -1;
+  CKP(h, st, PC_STEM, 0, 20.0 * t.S * 3 * c.image_resolution * c.image_resolution,
+      pgd_linf_f32(dpatch, x_adv, x_clean, x_norm, t.S, c.image_resolution, c.vision_patch_size, h->Kp, prm, st));
+  return 0;
 }
 
 int mudpt_text_set_classes(mudpt_handle* h, const float* embeddings, int32_t C, int32_t src_len, int32_t seq_len,
@@ -1416,6 +1450,14 @@ int mudpt_im2col(const float* images, uint16_t* patches, int32_t B, int32_t R, i
 }
 int mudpt_col2im(const float* patches, float* images, int32_t B, int32_t R, int32_t patch, int32_t ld, void* stream) {
   CKG(col2im_f32(patches, images, B, R, patch, ld, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+int mudpt_pgd_linf_update(const float* dpatch, int32_t ld, float* x_adv, const float* x_clean, float* x_norm, int32_t B,
+                          int32_t R, int32_t patch, const float* mean_host, const float* std_host, float eps, float alpha,
+                          void* stream) {
+  if (!dpatch || !x_adv || !x_clean || !x_norm || !mean_host || !std_host) return fail(nullptr, "mudpt_pgd_linf_update: null argument");
+  CKG(pgd_linf_f32(dpatch, x_adv, x_clean, x_norm, B, R, patch, ld, pgd_params(mean_host, std_host, eps, alpha),
+                   static_cast<cudaStream_t>(stream)));
   return 0;
 }
 int mudpt_peer_all_gather_rows(const void* peers_dev, int32_t world, int32_t n_total, int32_t width, float* out, void* stream) {

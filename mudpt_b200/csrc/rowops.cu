@@ -7,6 +7,8 @@
 //   patch extraction .. clip/model.py:527-529 (conv1 with stride == kernel == patch)
 #include "rowops.h"
 
+#include <cmath>
+#include <cstdint>
 #include <cstdlib>
 
 #include "common.cuh"
@@ -1364,6 +1366,85 @@ const char* col2im_f32(const float* cols, float* img, int B, int R, int p, int l
   launch_pdl(col2im_kernel, dim3(static_cast<unsigned>((total2 + 255) / 256)), dim3(256), 0, stream, cols, img, R, p, ldi, total2);
   count_launch(1);
   return launch_status("col2im launch failed");
+}
+
+// ------------------------------------------------------------------ l-inf PGD update
+// IEEE fp32 arithmetic in inline PTX: the library builds with --use_fast_math, under which __fdiv_rn / __fadd_rn /
+// __fsub_rn and fminf / fmaxf compile to their .ftz forms and would flush subnormal gradients and pixels to zero.
+// PyTorch's element-wise kernels do not flush, and the update must be bitwise theirs.
+__device__ __forceinline__ float add_ieee(float a, float b) { float r; asm("add.rn.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float sub_ieee(float a, float b) { float r; asm("sub.rn.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float div_ieee(float a, float b) { float r; asm("div.rn.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float max_ieee(float a, float b) { float r; asm("max.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ float min_ieee(float a, float b) { float r; asm("min.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
+
+// One pixel, op for op the PyTorch loop x = (x + alpha * (g / std).sign()).clamp(x0 - eps, x0 + eps).clamp(0, 1),
+// xn = (x - mean) / std, where g / std is the autograd of the normalisation.  The sign is read from the bits of the
+// quotient (torch.sign: 0 for +-0 and NaN); alpha * sign is exact, so the step is +0 or alpha with the quotient's sign bit.
+__device__ __forceinline__ float pgd_pixel(float g, float x, float x0, float mean, float std, float eps, float alpha, float* xn) {
+  const uint32_t q = __float_as_uint(div_ieee(g, std));
+  const uint32_t mag = q & 0x7fffffffu;
+  const float step = (mag == 0u || mag > 0x7f800000u) ? 0.f : __uint_as_float(__float_as_uint(alpha) | (q & 0x80000000u));
+  float v = add_ieee(x, step);
+  v = min_ieee(max_ieee(v, sub_ieee(x0, eps)), add_ieee(x0, eps));
+  v = min_ieee(max_ieee(v, 0.f), 1.f);
+  *xn = div_ieee(sub_ieee(v, mean), std);
+  return v;
+}
+
+// The patch gradient is read through col2im_kernel's index map (never written as an image; padding columns not read);
+// x_adv is updated in place and x_norm rewritten, two consecutive pixels per thread.
+__global__ void pgd_linf_kernel(const float* __restrict__ cols, float* __restrict__ x_adv, const float* __restrict__ x_clean,
+                                float* __restrict__ x_norm, int R, int p, int ldi, size_t total2, PgdParams prm) {
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  pdl_wait();
+  pdl_trigger();
+  if (i >= total2) return;
+  const size_t e = i * 2;
+  const int x = static_cast<int>(e % R);
+  const size_t r2 = e / R;
+  const int y = static_cast<int>(r2 % R);
+  const size_t bc = r2 / R;
+  const int c = static_cast<int>(bc % 3);
+  const size_t b = bc / 3;
+  const int gw = R / p;
+  const int px = x / p, ix = x - px * p, py = y / p, iy = y - py * p;
+  const size_t row = (b * gw + py) * gw + px;
+  const int col = (c * p + iy) * p + ix;
+  const float2 g = *reinterpret_cast<const float2*>(cols + row * ldi + col);
+  const float2 xa = *reinterpret_cast<const float2*>(x_adv + e);
+  const float2 x0 = *reinterpret_cast<const float2*>(x_clean + e);
+  const float m = prm.mean[c], s = prm.std[c];
+  float2 o, n;
+  o.x = pgd_pixel(g.x, xa.x, x0.x, m, s, prm.eps, prm.alpha, &n.x);
+  o.y = pgd_pixel(g.y, xa.y, x0.y, m, s, prm.eps, prm.alpha, &n.y);
+  *reinterpret_cast<float2*>(x_adv + e) = o;
+  *reinterpret_cast<float2*>(x_norm + e) = n;
+}
+
+const char* pgd_linf_check(const PgdParams& prm) {
+  if (!(std::isfinite(prm.eps) && prm.eps >= 0.f)) return "pgd: eps must be finite and >= 0";
+  if (!(std::isfinite(prm.alpha) && prm.alpha > 0.f)) return "pgd: alpha must be finite and > 0";
+  for (int c = 0; c < 3; ++c) {
+    if (!(std::isfinite(prm.std[c]) && prm.std[c] > 0.f)) return "pgd: std must be finite and > 0";
+    if (!std::isfinite(prm.mean[c])) return "pgd: mean must be finite";
+  }
+  return nullptr;
+}
+
+const char* pgd_linf_f32(const float* cols, float* x_adv, const float* x_clean, float* x_norm, int B, int R, int p, int ldi,
+                         const PgdParams& prm, cudaStream_t stream) {
+  if (const char* e = pgd_linf_check(prm)) return e;
+  if (B <= 0) return nullptr;
+  if (R % p != 0 || p % 2 != 0 || ldi < 3 * p * p || ldi % 2 != 0) return "pgd: bad geometry";
+  for (const void* q : {static_cast<const void*>(cols), static_cast<const void*>(x_adv), static_cast<const void*>(x_clean),
+                        static_cast<const void*>(x_norm)})
+    if (reinterpret_cast<uintptr_t>(q) % 8 != 0) return "pgd: pointers must be 8-byte aligned";
+  const size_t total2 = static_cast<size_t>(B) * 3 * R * R / 2;
+  launch_pdl(pgd_linf_kernel, dim3(static_cast<unsigned>((total2 + 255) / 256)), dim3(256), 0, stream, cols, x_adv, x_clean,
+             x_norm, R, p, ldi, total2, prm);
+  count_launch(1);
+  return launch_status("pgd launch failed");
 }
 
 // ------------------------------------------------------------------ small helpers

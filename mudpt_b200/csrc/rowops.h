@@ -46,6 +46,12 @@ const char* gather_rows(const float* src_f, const __nv_bfloat16* src_b, const in
 const char* im2col_bf16(const float* img, __nv_bfloat16* out, int B, int R, int p, int ldo, cudaStream_t stream);
 // inverse of im2col_bf16's index map, fp32 (patch rows of row stride ldi >= 3*p*p -> [B, 3, R, R], every element written once)
 const char* col2im_f32(const float* cols, float* img, int B, int R, int p, int ldi, cudaStream_t stream);
+// One l-inf PGD step in pixel space (include/mudpt_b200.h, mudpt_pgd_linf_update): the patch gradient cols (col2im_f32's
+// layout, dL/d x_norm) -> x_adv [B, 3, R, R] in place and x_norm = (x_adv - mean) / std, IEEE fp32
+struct PgdParams { float mean[3], std[3], eps, alpha; };
+const char* pgd_linf_check(const PgdParams& prm);  // nullptr, or why the parameters are rejected
+const char* pgd_linf_f32(const float* cols, float* x_adv, const float* x_clean, float* x_norm, int B, int R, int p, int ldi,
+                         const PgdParams& prm, cudaStream_t stream);
 const char* write_cls_rows(float* x, const float* cls, const float* pos, int S, int L, int d, cudaStream_t stream);
 // seq_off != null: packed variable-length output rows (L = the longest sequence)
 const char* add_positional(float* x0, const float* emb, const float* pos, int S, int L, int Lsrc, int d, cudaStream_t stream,

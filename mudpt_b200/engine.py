@@ -150,6 +150,22 @@ class Engine:
                                                          d_img.data_ptr(), _lib.stream_ptr(self.device)), self.h)
         return dP, d_img
 
+    def vision_pgd_step(self, d_f_img: torch.Tensor, x_adv: torch.Tensor, x_clean: torch.Tensor, x_norm: torch.Tensor,
+                        mean, std, eps: float, alpha: float) -> None:
+        """One l-inf PGD step on the images of the last vision_forward, which were x_norm = (x_adv - mean) / std:
+        x_adv <- clamp(clamp(x_adv + alpha * sign(dL/d x_adv), x_clean - eps, x_clean + eps), 0, 1) in place, and x_norm
+        <- (x_adv - mean) / std, bitwise that PyTorch loop (include/mudpt_b200.h, mudpt_vision_pgd_step).  x_adv, x_clean,
+        x_norm [B, 3, R, R] fp32 (x_norm may be the tensor the forward read); mean, std: 3 per-channel values."""
+        d_f_img = d_f_img.contiguous()
+        B, R = self.vision_batch, self.arch["image_resolution"]
+        self._check_f32(d_f_img, (B, self.arch["embed_dim"]))
+        for x in (x_adv, x_clean, x_norm):
+            self._check_f32(x, (B, 3, R, R))
+        mean_h, std_h = (_channels(v) for v in (mean, std))
+        _lib.check(self.lib.mudpt_vision_pgd_step(self.h, d_f_img.data_ptr(), x_adv.data_ptr(), x_clean.data_ptr(),
+                                                  x_norm.data_ptr(), mean_h, std_h, float(eps), float(alpha),
+                                                  _lib.stream_ptr(self.device)), self.h)
+
     def text_set_classes(self, embeddings: torch.Tensor, eot: torch.Tensor, seq_len: int,
                          lengths: Optional[List[int]] = None) -> None:
         """embeddings [C, src_len, width] fp32; eot [C] int (position of the EOT token).  With `lengths` [C] the tower is
@@ -277,6 +293,14 @@ class Engine:
         src = _from_ptr(p.value, n.value, dtype, self.device)
         out.copy_(src)
         return out
+
+
+def _channels(v):
+    """3 per-channel values (a sequence or a tensor of 3 elements) as a host fp32 array"""
+    vals = torch.as_tensor(v, dtype=torch.float32).detach().cpu().flatten().tolist()
+    if len(vals) != 3:
+        raise ValueError(f"mudpt_b200: expected 3 per-channel values, got {len(vals)}")
+    return (C.c_float * 3)(*vals)
 
 
 def _from_ptr(ptr: int, numel: int, dtype: torch.dtype, device: torch.device) -> torch.Tensor:

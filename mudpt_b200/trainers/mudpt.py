@@ -29,6 +29,7 @@ from .. import clip
 from .. import dist as mdist
 from ..engine import (prompt_algebra_forward, prompt_algebra_backward, text_lengths, text_tower, text_tower_dense, vision_tower, LogitsFn,
                       PromptAlgebraFn)
+from ..input_pipeline import CLIP_MEAN, CLIP_STD
 
 try:  # the Dassl engine is not in the reference tree nor in this image (SURVEY.md section 2 row 13)
     from dassl.engine import TRAINER_REGISTRY, TrainerX
@@ -257,6 +258,72 @@ class TextEncoder(nn.Module):
         return text_tower_dense(engine, prompts.float(), eot, deep_prompts.float(), seq_len, lengths)
 
 
+class LinfPGD:
+    """l-inf PGD in pixel space against fixed text features, with the model doing the normalisation (TeCoA / APT-style
+    adversarial prompt tuning and evaluation).  x_adv starts at the clean pixels (or, with random_start, at
+    clamp(pixels + U(-eps, eps), 0, 1) drawn from `generator`); each step is one training vision forward on
+    x_norm = (x_adv - mean) / std, the logits head (mean cross-entropy over the batch, no text-feature gradient) and
+    Engine.vision_pgd_step, which updates x_adv and x_norm in place.  The start and its normalisation are PyTorch ops,
+    the steps native; together they are bitwise the PyTorch loop of INTEGRATION.md."""
+
+    def __init__(self, eng, eps, alpha, steps, random_start=False, generator=None, mean=CLIP_MEAN, std=CLIP_STD):
+        if not hasattr(eng, "vision_pgd_step"):
+            raise RuntimeError(f"mudpt_b200: the engine ({type(eng).__name__}) has no vision_pgd_step: it cannot run the "
+                               "fused PGD attack")
+        if int(steps) != steps or steps < 0:
+            raise ValueError(f"mudpt_b200: PGD steps must be an integer >= 0, not {steps!r}")
+        if not (math.isfinite(eps) and eps >= 0):
+            raise ValueError(f"mudpt_b200: PGD eps must be finite and >= 0, not {eps!r}")
+        if not (math.isfinite(alpha) and alpha > 0):
+            raise ValueError(f"mudpt_b200: PGD alpha must be finite and > 0, not {alpha!r}")
+        # per-channel constants as fp32 values, read once (a CUDA tensor is synchronised here, not at every step)
+        self.mean, self.std = (tuple(torch.as_tensor(v, dtype=torch.float32).detach().cpu().flatten().tolist())
+                               for v in (mean, std))
+        if len(self.mean) != 3 or len(self.std) != 3 or not all(math.isfinite(v) and v > 0 for v in self.std):
+            raise ValueError("mudpt_b200: PGD mean / std must hold 3 values each, std finite and > 0")
+        self.eng, self.eps, self.alpha, self.steps = eng, float(eps), float(alpha), int(steps)
+        self.random_start, self.generator = random_start, generator
+        self.x_clean = self.x_adv = self.x_norm = self.label = None
+
+    def start(self, pixels, label):
+        """x_adv at the start, and x_norm = (x_adv - mean) / std (returned): PyTorch ops on the current stream"""
+        self.x_clean, self.label = pixels, label.to(device=pixels.device)
+        if self.random_start:
+            noise = torch.empty_like(pixels).uniform_(-self.eps, self.eps, generator=self.generator)
+            self.x_adv = (pixels + noise).clamp(0, 1)
+        else:
+            self.x_adv = pixels.clone()
+        mean, std = _channel_view(self.mean, pixels.device), _channel_view(self.std, pixels.device)
+        self.x_norm = (self.x_adv - mean) / std
+        return self.x_norm
+
+    def run(self, P_v, f_txt, f_img=None, forward_last=False):
+        """The steps against f_txt.  f_img: the training forward of the current x_norm if already run.  With forward_last
+        the result is the training forward of the final x_norm (its activations stay for a backward), else None."""
+        eng, B = self.eng, self.x_adv.shape[0]
+        for _ in range(self.steps):
+            if f_img is None:
+                f_img = eng.vision_forward(self.x_norm, P_v)
+            _, _, d_i, _ = eng.logits_head(f_img, f_txt, self.label, 1.0 / B, True, text_grad=False)
+            eng.vision_pgd_step(d_i, self.x_adv, self.x_clean, self.x_norm, self.mean, self.std, self.eps, self.alpha)
+            f_img = None
+        if forward_last and f_img is None:
+            f_img = eng.vision_forward(self.x_norm, P_v)
+        return f_img if forward_last else None
+
+
+_CHANNEL_VIEWS = {}
+
+
+def _channel_view(vals, device):
+    """[1, 3, 1, 1] fp32 tensor of 3 per-channel values on `device`, cached: the host-to-device copy happens once"""
+    key = (vals, str(device))
+    t = _CHANNEL_VIEWS.get(key)
+    if t is None:
+        t = _CHANNEL_VIEWS[key] = torch.tensor(vals, dtype=torch.float32, device=device).view(1, 3, 1, 1)
+    return t
+
+
 class CustomCLIP(nn.Module):
     def __init__(self, cfg, classnames, clip_model, tokenizer=None):
         super().__init__()
@@ -372,6 +439,26 @@ class CustomCLIP(nn.Module):
         """Fused train step: forward, mean cross-entropy over the GLOBAL batch (F.cross_entropy of
         trainers/mudpt.py:250 under nn.DataParallel semantics) and backward into the .grad of the 10
         trainable tensors.  Returns (loss, logits).  Gradients are all-reduced across ranks."""
+        return self._fused_step(image, label, None)
+
+    def forward_backward_adversarial(self, pixels, label, eps, alpha, steps, random_start=False, generator=None,
+                                     mean=CLIP_MEAN, std=CLIP_STD):
+        """Fused adversarial train step (PGD-AT / TeCoA-style adversarial prompt tuning) on pixel-space images
+        `pixels` [B, 3, H, W] in [0, 1]; the model normalises with `mean` / `std`.  Returns (loss, logits, x_adv).
+
+        One text training forward (and its all-gather across ranks), then `steps` l-inf PGD steps of size `alpha` in the
+        eps-ball of `pixels` against those text features (see LinfPGD; each rank attacks its own images against all
+        classes), then forward_backward's step on (x_adv - mean) / std.  Bitwise cache_text_features() + pgd_attack() +
+        forward_backward(x_adv_norm), with one text forward instead of two.  The attack touches neither the text
+        tower's saved activations nor any collective; with overlap_towers it runs on the vision stream."""
+        device = self.logit_scale.device if pixels.device.type == "cpu" and self.logit_scale.device.type == "cuda" else pixels.device
+        attack = LinfPGD(self._engine(device), eps, alpha, steps, random_start, generator, mean, std)
+        loss, logits = self._fused_step(pixels, label, attack)
+        return loss, logits, attack.x_adv
+
+    def _fused_step(self, image, label, attack):
+        """forward_backward, and with `attack` (a LinfPGD) forward_backward_adversarial: `image` holds the pixels, the
+        vision tower's first forward is the attack's, and the attack runs between the text features and the head."""
         host_batch = image.device.type == "cpu" and self.logit_scale.device.type == "cuda"
         device = self.logit_scale.device if host_batch else image.device
         eng = self._engine(device)
@@ -396,10 +483,19 @@ class CustomCLIP(nn.Module):
             host_batch = False
         if not host_batch:
             image = image.type(self.dtype)
+
+        def vision_first(image, label):
+            """the training vision forward that can start before the text features exist"""
+            if attack is not None:
+                image = attack.start(image, label)
+            return eng.vision_forward(image, P_v.detach())
+
         if not self.overlap_towers or device.type != "cuda":  # (CPU: only the gloo tests' stand-in engine)
-            f_img = eng.vision_forward(image, P_v.detach())
+            f_img = vision_first(image, label)
             f_txt_loc = eng.text_forward(P_t.detach(), True)
             f_txt = mdist.all_gather_rows(f_txt_loc, n_cls) if world > 1 else f_txt_loc
+            if attack is not None:
+                f_img = attack.run(P_v.detach(), f_txt, f_img, forward_last=True)
             logits, loss, d_i, d_t = eng.logits_head(f_img, f_txt, label, 1.0 / (image.shape[0] * world), True)
             loss = self._publish_loss(loss, world)
             d_t_loc = mdist.reduce_scatter_rows(d_t, n_cls) if world > 1 else d_t
@@ -429,7 +525,7 @@ class CustomCLIP(nn.Module):
                     # not need the images -- starts at once and hides the PCIe copy (19 MB, ~0.8 ms)
                     image = image.to(device, non_blocking=True).type(self.dtype)
                     label = label.to(device, non_blocking=True)
-                f_img = eng.vision_forward(image, P_v.detach())
+                f_img = vision_first(image, label)
             mark("vision_fwd_end", side)
             # the head's exchange: over NVLink peer memory with the library's own kernels where the ranks share a node,
             # else NCCL collectives
@@ -442,8 +538,17 @@ class CustomCLIP(nn.Module):
                 f_txt_loc = eng.text_forward(P_t.detach(), True)
                 f_txt = mdist.all_gather_rows(f_txt_loc, n_cls) if world > 1 else f_txt_loc
             mark("text_fwd_end", main)
+            if attack is not None:
+                # the attack's heads need the text features; every head of the step stays stream-ordered (one head
+                # workspace per handle): the attack's on the vision stream, then the step's on the main stream
+                side.wait_stream(main)
+                with torch.cuda.stream(side):
+                    f_img = attack.run(P_v.detach(), f_txt, f_img, forward_last=True)
+                mark("attack_end", side)
             main.wait_stream(side)
             f_img.record_stream(main)
+            if attack is not None:
+                attack.x_adv.record_stream(main)
             if host_batch:
                 label.record_stream(main)
             logits, loss, d_i, d_t = eng.logits_head(f_img, f_txt, label, 1.0 / (image.shape[0] * world), True,
@@ -552,6 +657,25 @@ class CustomCLIP(nn.Module):
                                                text_grad=False)
         _, d_image = eng.vision_backward_images(d_i, want_prompts=False)
         return loss, logits, d_image
+
+    @torch.no_grad()
+    def pgd_attack(self, pixels, label, eps, alpha, steps, random_start=False, generator=None, mean=CLIP_MEAN, std=CLIP_STD):
+        """l-inf PGD on the cached text features (adversarial evaluation): `steps` steps of size `alpha` in the eps-ball of
+        `pixels` [B, 3, H, W] in [0, 1], starting there or (random_start) at clamp(pixels + U(-eps, eps), 0, 1) drawn from
+        `generator`.  The model normalises with `mean` / `std`.  Returns (x_adv, x_adv_norm = (x_adv - mean) / std).
+
+        Each step is one training vision forward, the logits head (mean cross-entropy over this batch) and one native
+        PGD step (Engine.vision_pgd_step): no autograd, no text tower, no collective (under torchrun every rank attacks
+        its own images).  Bitwise the PyTorch loop of INTEGRATION.md on image_gradient.  As image_gradient, the vision
+        forwards replace the tower's saved activations: a vision backward still pending from an earlier forward raises."""
+        if self._cached_text_features is None:
+            self.cache_text_features(pixels.device)
+        eng = self._engine(pixels.device)
+        attack = LinfPGD(eng, eps, alpha, steps, random_start, generator, mean, std)
+        P_v, _ = self.prompt_stacks()
+        attack.start(pixels.type(self.dtype), label)
+        attack.run(P_v.detach(), self._cached_text_features)
+        return attack.x_adv, attack.x_norm
 
 
 @TRAINER_REGISTRY.register()
