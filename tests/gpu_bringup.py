@@ -123,7 +123,7 @@ def group_gemm(res):
         big = torch.full((rows + GUARD, N), float("nan"), device=dev, dtype=dtype)
         return big, big[:rows]
 
-    def run(M, N, K, mode):
+    def run(M, N, K, mode, np_=4, L=7):
         A = (torch.randn(M, K, device=dev) * 0.5).bfloat16()
         B = (torch.randn(N, K, device=dev) * 0.5).bfloat16()
         bias = torch.randn(N, device=dev)
@@ -147,7 +147,6 @@ def group_gemm(res):
             hf = aux.double(); s = torch.sigmoid(1.702 * hf)
             exp = (ref + bias.double()) * (s * (1 + 1.702 * hf * (1 - s)))
         elif mode == 5:
-            np_, L = 4, 7
             assert M % np_ == 0
             pos = torch.randn(np_ + 1, N, device=dev); kw["resid"] = pos; kw["np_"] = np_; kw["L"] = L
             big, out = guarded(M // np_ * L, N, f32)
@@ -197,6 +196,13 @@ def group_gemm(res):
             print(key, res[key], flush=True)
     res["gemm_patch_m5"] = run(4 * 6, 128, 768, 5)
     print("gemm_patch_m5", res["gemm_patch_m5"], flush=True)
+    # the stems of the towers (B images x np patches, L = 1 + np + 2 prompt rows): ViT-B/16 at B = 32 (pair tiles) and
+    # B = 165, ViT-B/32 (K = 3072), ViT-L/14 at B = 8 (Kp = 592: a K tail of 16)
+    for (M, N, K, np_, L) in [(6272, 768, 768, 196, 199), (32340, 768, 768, 196, 199), (1568, 768, 3072, 49, 52),
+                              (2048, 1024, 592, 256, 259)]:
+        key = f"gemm_patch_{M}x{N}x{K}_m5"
+        res[key] = run(M, N, K, 5, np_, L)
+        print(key, res[key], flush=True)
     # error pattern of the smallest case for debugging, if wrong
     m = res["gemm_128x128x64_m0"]
     res["gemm_ok"] = all(v.get("rel", 1) < 2e-2 for k, v in res.items() if k.startswith("gemm_") and isinstance(v, dict))
@@ -937,18 +943,21 @@ def group_head(res):
                       r["loss"], r["repeat_bitwise"], r.get("shard_bitwise"), flush=True)
         del eng
     _feature_heads(res, dev)
+    _feature_heads(res, dev, "ViT-L/14")
 
 
-def _feature_heads(res, dev):
-    """Feature heads (gather_ln_kernel + split-K sgemm, csrc/head.cu) at ViT-B/16 widths (vision 768 -> 512, text
-    512 -> 512) on a one-layer-per-tower handle without pruning, so that x_in[layers] holds every row of the tower output:
-    f_img = LN_post(x[:, 0]) @ proj and f_txt = ln_final(x[c, eot_c]) @ text_projection against fp64, per sequence."""
+def _feature_heads(res, dev, arch_name="ViT-B/16"):
+    """Feature heads (gather_ln_kernel + split-K sgemm, csrc/head.cu) at the widths of `arch_name` (ViT-B/16: vision
+    768 -> 512, text 512 -> 512; ViT-L/14: vision 1024 -> 768, text 768 -> 768) on a one-layer-per-tower handle without
+    pruning, so that x_in[layers] holds every row of the tower output: f_img = LN_post(x[:, 0]) @ proj and
+    f_txt = ln_final(x[c, eot_c]) @ text_projection against fp64, per sequence."""
     import dataclasses
     import torch
     import torch.nn.functional as F
     from mudpt_b200 import _lib, synthetic as syn
     from mudpt_b200.engine import Engine
-    arch = dataclasses.replace(syn.ARCHS["ViT-B/16"], vision_layers=1, transformer_layers=1)
+    arch = dataclasses.replace(syn.ARCHS[arch_name], vision_layers=1, transformer_layers=1)
+    tag = "" if arch_name == "ViT-B/16" else "_" + arch_name.replace("/", "").replace("-", "").lower()
     sd = syn.synthetic_clip_state_dict(arch, 0)
     ad = dict(zip(["embed_dim", "image_resolution", "vision_layers", "vision_width", "vision_patch_size", "context_length",
                    "vocab_size", "transformer_width", "transformer_heads", "transformer_layers"], arch.astuple()))
@@ -966,7 +975,7 @@ def _feature_heads(res, dev):
     x = eng.debug_buffer(0, "x_in", 1, torch.float32).view(B, -1, dv)
     ref = F.layer_norm(x[:, 0].double(), (dv,), sd["visual.ln_post.weight"].double().to(dev),
                        sd["visual.ln_post.bias"].double().to(dev), eps) @ sd["visual.proj"].double().to(dev)
-    res["feature_head_image"] = _metrics(f_img, ref, grid=(B,))
+    res["feature_head_image" + tag] = _metrics(f_img, ref, grid=(B,))
     # text: the EOT row of each class, at different positions (and one at the last of the truncated length)
     eot = torch.tensor([3, 9, 4, 20, 7, 12, 5, 20, 16], dtype=torch.int64)
     Cn, seq_len = eot.numel(), int(eot.max()) + 1
@@ -978,8 +987,8 @@ def _feature_heads(res, dev):
     xe = x[torch.arange(Cn, device=dev), eot.to(dev)]
     ref = F.layer_norm(xe.double(), (dt,), sd["ln_final.weight"].double().to(dev), sd["ln_final.bias"].double().to(dev),
                        eps) @ sd["text_projection"].double().to(dev)
-    res["feature_head_text"] = _metrics(f_txt, ref, grid=(Cn,))
-    print("feature heads", res["feature_head_image"], res["feature_head_text"], flush=True)
+    res["feature_head_text" + tag] = _metrics(f_txt, ref, grid=(Cn,))
+    print("feature heads", arch_name, res["feature_head_image" + tag], res["feature_head_text" + tag], flush=True)
     del eng
 
 
